@@ -12,14 +12,20 @@
                                  native reader / writer of libnpore_b200.so (include/npore_bamio.h: multi-threaded BGZF
                                  inflate, record decode into flat arrays, batch SAM formatting) and never builds
                                  per-read Python objects; the pure-Python functions above remain as the tuple API.
+                                 One batch pipeline (_realign_segments) serves both forms: the streamed windows of one
+                                 device, and with devices=[...] one region shard per device (_realign_sharded).
 The GPU path is entered through npore_b200.engine (realign_bam) or npore_b200.bam.realign_reads (tuples).
 """
+import contextlib
 import ctypes as C
 import gzip
 import io
 import os
+import queue
 import struct
 import sys
+import threading
+import time
 import zlib
 
 import numpy as np
@@ -29,6 +35,9 @@ from . import cfg
 _SEQ16 = "=ACMGRSVTWYHKDBN"
 _OPS = "MIDNSHP=XB"
 _SEQ_PAIR = np.frombuffer("".join(a + b for a in _SEQ16 for b in _SEQ16).encode(), dtype=np.uint8).reshape(256, 2)
+_PIPES = {}                     # _pipeline's cache
+_PIPE_LOCK = threading.Lock()   # contexts of different devices are created one after the other
+_MALLOC_TUNED = False           # _keep_freed_buffers_mapped has run
 
 
 def read_fasta(path):
@@ -301,9 +310,6 @@ def select_reads(bam, regions=None, max_reads=0):
             yield ctg, sel
 
 
-_PIPES = {}
-
-
 def _pipeline(sub, npt, n_inflight, device=None):
     """Cached PipelinedRealigner per (tables, cfg, device) (same idea as aln._engine)."""
     from .engine import PipelinedRealigner
@@ -317,68 +323,96 @@ def _pipeline(sub, npt, n_inflight, device=None):
     return p
 
 
+def _record_ops(bam, sel):
+    """D/I ops of each selected record (reference span + aligned read length), from the record columns alone."""
+    return (bam.end[sel] - bam.pos[sel]).astype(np.int64) + bam.aln_len[sel]
+
+
 def _read_loads(bam, sel, max_b_rows=20000, r=30):
-    """Cell updates per selected record (SURVEY.md 8(d)): (Lref + Lseq + n_chunks) * (2r+1), from the record columns alone."""
-    ops = (bam.end[sel] - bam.pos[sel]).astype(np.int64) + bam.aln_len[sel]
+    """Cell updates per selected record (SURVEY.md 8(d)): (Lref + Lseq + n_chunks) * (2r+1)."""
+    ops = _record_ops(bam, sel)
     return (ops + -(-ops // (max_b_rows - 1))) * (2 * r + 1)
 
 
-def _realign_segments(bam, segments, fa, pipe, fd, tm, n_threads, max_batch_ops, n_inflight):
-    """The three-stage pipeline over an explicit list of (contig, record indices) segments: gather batch k+1 while batch k is
-    on the GPU and batch k-1 is formatted and appended to the file descriptor `fd` (not in append mode) -- records in segment
-    order.  Returns the records written."""
-    import queue
-    import threading
-    import time
+def _realign_segments(bam, segments, fa, pipe, open_out, tm, n_threads, nt_text, max_batch_ops, n_inflight, mark, t0):
+    """The three-stage pipeline over (contig, record indices) segments, which may be produced lazily: gather batch k+1 while
+    batch k is on the GPU and a writer thread formats batch k-1 and appends it to the file descriptor that open_out() returns.
+    The writer calls open_out() before its first batch and writes from the descriptor's current size on.  The descriptor must
+    not be in append mode: Linux ignores the offset of a pwrite on an append-mode descriptor, and the formatter threads place
+    their slices by offset.  Records are written in segment order and counted into cfg.counter batch by batch.  n_threads:
+    threads of the nibble / CIGAR gathers and of formatting; nt_text: threads of the SAM-text gather that runs beside the
+    GPU.  tm receives seconds per phase, mark(event) a trace event per step (GPU times in them count from perf_counter() = t0).
+    Returns the records written."""
     from .aln import _report
     from .cig import bases_to_int
     from .engine import NPORE_OUT_NO_EXPANDED, NPORE_OUT_RLE, NPORE_OUT_STANDARDIZE, PackedBatch
     flags = NPORE_OUT_STANDARDIZE | NPORE_OUT_RLE | NPORE_OUT_NO_EXPANDED
     pending = queue.Queue(maxsize=n_inflight + 1)
-    state = {"written": 0, "error": None, "end": os.fstat(fd).st_size}
+    state = {"written": 0, "error": None}
 
     def retire_loop():
+        fd = -1
+        try:
+            fd = open_out()
+            end = os.fstat(fd).st_size
+        except Exception as e:                        # noqa: BLE001
+            state["error"] = e
         while True:
             item = pending.get()
             if item is None:
-                return
+                break
             if state["error"] is not None:
-                continue
+                continue                              # keep draining so that the producer never blocks
             try:
                 fut, cols, g, n = item
                 t1 = time.perf_counter()
-                res, _ = fut.result()
+                res, st_ = fut.result()
                 t2 = time.perf_counter()
+                mark(f"gpu done n={n} kernels_ms={st_['ms_kernels_total']:.1f} h2d_ms={st_['ms_h2d']:.1f} plan_ms={st_['ms_plan']:.1f} d2h_ms={st_['ms_d2h']:.1f} "
+                     f"warps/SM={st_['fwd_warps_per_sm']} context from {1e3 * (st_['wall'][0] - t0):.1f} ms, buffers {1e3 * (st_['wall'][1] - t0):.1f}, "
+                     f"to {1e3 * (st_['wall'][2] - t0):.1f} ms")
                 _report(res.status[:n], "realign_read")
-                state["end"] += len(format_sam(bam, None, g, res.rle, res.rle_off[:n + 1], n_threads, cols=cols, fd=fd, offset=state["end"]))
+                end += len(format_sam(bam, None, g, res.rle, res.rle_off[:n + 1], n_threads, cols=cols, fd=fd, offset=end))
                 t3 = time.perf_counter()
+                mark("formatted + written")
                 tm["gpu_wait"] += t2 - t1; tm["format"] += t3 - t2; tm["write"] += time.perf_counter() - t3
                 state["written"] += n
+                with cfg.counter.get_lock():
+                    cfg.counter.value += n
             except Exception as e:                    # noqa: BLE001
                 state["error"] = e
+        if fd >= 0:
+            os.close(fd)
 
     retire = threading.Thread(target=retire_loop, daemon=True)
     retire.start()
     try:
         for ctg, sel in segments:
             contig = fa[ctg]
-            ops = np.cumsum((bam.end[sel] - bam.pos[sel]).astype(np.int64) + bam.aln_len[sel])
+            ops = np.cumsum(_record_ops(bam, sel))
             cut = 0
             while cut < len(sel) and state["error"] is None:
                 stop = max(cut + 1, int(np.searchsorted(ops, (ops[cut - 1] if cut else 0) + max_batch_ops, "right")))
                 part = sel[cut:stop]
                 t1 = time.perf_counter()
-                nib, nib_start = bam.gather_nib(part, n_threads)              # the upload: BAM's own 4-bit bases + CIGAR words
+                nib, nib_start = bam.gather_nib(part, n_threads)          # the upload: BAM's own 4-bit bases + CIGAR words
+                mark("nib gathered")
                 cig_words, cig_off = bam.gather_cigar(part, n_threads)
+                mark("cigar gathered")
                 lo, hi = int(bam.pos[part].min()), int(bam.end[part].max())
+                # base codes of the batch's reference span only (not the contig: 250 Mb of chr1 for a window that covers 1 Mb)
                 packed = PackedBatch.from_flat_shared_nib(bases_to_int(contig[lo:hi].upper()), bam.pos[part].astype(np.int64) - lo, bam.end[part] - bam.pos[part],
                                                           nib, nib_start, bam.aln_len[part], cig_words, cig_off)
-                fut = pipe.submit(packed, flags)                              # the GPU starts; the SAM-text gather runs beside it
-                g = bam.gather(part, n_threads, want_codes=False, want_cigar=False)      # ASCII bases / qualities / names
+                fut = pipe.submit(packed, flags)                          # the GPU starts; the SAM-text gather runs beside it
+                mark(f"submitted n={len(part)}")
+                g = bam.gather(part, nt_text, want_codes=False, want_cigar=False)    # ASCII bases / qualities / names
+                mark("text gathered")
                 item = (fut, take_columns(bam, part), g, len(part))
                 tm["gather"] += time.perf_counter() - t1
-                pending.put(item)
+                pending.put(item)                                        # blocks while n_inflight + 1 batches are unfinished
                 cut = stop
+            if state["error"] is not None:
+                break
     finally:
         pending.put(None)
         retire.join()
@@ -387,33 +421,17 @@ def _realign_segments(bam, segments, fa, pipe, fd, tm, n_threads, max_batch_ops,
     return state["written"]
 
 
-def realign_bam_sharded(bam_fn, fasta, devices, out_prefix=None, regions=None, max_reads=0, argv=None, max_batch_ops=64_000_000,
-                        n_threads=0, timings=None, n_inflight=2):
+def _realign_sharded(bam, fa, pipes, devices, open_out, regions, max_reads, max_batch_ops, n_threads, n_inflight, tm, mark, t0):
     """realign.py:75-115 on several GPUs of one host (SURVEY.md 8(e)): the coordinate-sorted reads are cut into len(devices)
     contiguous genomic regions of equal cell-update load (the reference's own unit of distribution is the region,
     util.py:44-93 / bam.pyx:27-28); every region is an independent ingest -> GPU -> SAM-text pipeline on its own device (no
-    data-path collective); the host gathers the per-region SAM bodies in region order into ONE file, byte-identical to the
-    single-GPU output.  `devices` may name a device more than once (several pipelines on one GPU).  timings: per phase, summed
-    over the shards, plus 'shards': [{device, reads, cell_updates, seconds}] and 'concat' seconds."""
-    import threading
-    import time
-    from .bam import _tables
+    data-path collective) and host threads; the host gathers the per-region SAM bodies in region order into ONE file,
+    byte-identical to the single-GPU output.  Region 0 writes into the output itself (open_out), the others into part files,
+    which are removed whether the call succeeds or fails.  tm: per phase, summed over the shards, plus
+    'shards': [{device, reads, cell_updates, seconds}] and 'concat' seconds."""
     from .scheduler import cut_balanced
-    tm = timings if timings is not None else {}
-    for k in ("open", "gather", "gpu_wait", "format", "write", "concat"):
-        tm.setdefault(k, 0.0)
-    _keep_freed_buffers_mapped()
-    t0 = time.perf_counter()
-    if out_prefix is not None:
-        cfg.args.out_prefix = out_prefix
-    if not os.path.exists(bam_fn):
-        print(f"\nERROR: BAM file '{bam_fn}' not found.")
-        sys.exit(1)
-    fa = read_fasta(fasta) if isinstance(fasta, str) else fasta
-    bam = NativeBam(bam_fn, n_threads, window_bytes=0)             # region cuts need every record's span
-    out = f"{cfg.args.out_prefix}.sam"
-    create_header(out, bam.refs, argv)
-    sub, npt = _tables()
+    tm.setdefault("concat", 0.0)
+    t1 = time.perf_counter()
     G = len(devices)
     segs = list(select_reads(bam, regions, max_reads))
     loads = [_read_loads(bam, sel) for _, sel in segs]
@@ -429,77 +447,64 @@ def realign_bam_sharded(bam_fn, fasta, devices, out_prefix=None, regions=None, m
             shard_segs[int(gidx)].append((ctg, sel[m]))
             shard_load[int(gidx)] += int(ld[m].sum())
         done += float(ld.sum())
-    tm["open"] += time.perf_counter() - t0
-    parts = [out if g == 0 else f"{cfg.args.out_prefix}.part{g}.sam" for g in range(G)]
+    tm["open"] += time.perf_counter() - t1
+    out = f"{cfg.args.out_prefix}.sam"
+    parts = [f"{cfg.args.out_prefix}.part{g}.sam" for g in range(G)]
+    opens = [open_out] + [lambda p=p: os.open(p, os.O_WRONLY | os.O_CREAT | os.O_TRUNC, 0o644) for p in parts[1:]]
+    nt = max(1, (n_threads or os.cpu_count() or 1) // G)
     results = [None] * G
-    thread_tm = [{k: 0.0 for k in ("gather", "gpu_wait", "format", "write")} for _ in range(G)]
+    shard_tm = [{k: 0.0 for k in ("gather", "gpu_wait", "format", "write")} for _ in range(G)]
 
     def shard_main(g):
-        t1 = time.perf_counter()
+        t2 = time.perf_counter()
         try:
-            pipe = _pipeline(sub, npt, n_inflight, devices[g])
-            # (no O_APPEND: Linux ignores the offset of a pwrite on an append-mode descriptor, and the formatter threads place
-            # their slices by offset)
-            fd = os.open(parts[g], os.O_WRONLY | (0 if g == 0 else os.O_CREAT | os.O_TRUNC), 0o644)
-            try:
-                n = _realign_segments(bam, shard_segs[g], fa, pipe, fd, thread_tm[g], max(1, (n_threads or os.cpu_count() or 1) // G),
-                                      max_batch_ops, n_inflight)
-            finally:
-                os.close(fd)
-            results[g] = (n, time.perf_counter() - t1, None)
+            n = _realign_segments(bam, shard_segs[g], fa, pipes[g], opens[g], shard_tm[g], nt, nt, max_batch_ops, n_inflight, mark, t0)
+            results[g] = (n, time.perf_counter() - t2, None)
         except Exception as e:      # noqa: BLE001
-            results[g] = (0, time.perf_counter() - t1, e)
+            results[g] = (0, time.perf_counter() - t2, e)
 
-    with _PIPE_LOCK:                # contexts of different devices are created one after the other
-        for g in range(G):
-            _pipeline(sub, npt, n_inflight, devices[g])
     threads = [threading.Thread(target=shard_main, args=(g,)) for g in range(G)]
     for t in threads:
         t.start()
     for t in threads:
         t.join()
-    for n, _, err in results:
-        if err is not None:
-            raise err
-    t2 = time.perf_counter()
-    dst = os.open(out, os.O_WRONLY)                                 # host gather: region order = coordinate order
     try:
-        end = os.fstat(dst).st_size
-        for g in range(1, G):
-            with open(parts[g], "rb") as src:
-                left = os.fstat(src.fileno()).st_size
-                try:                                                # in-kernel copy (no bounce through user space)
-                    while left > 0:
-                        n = os.copy_file_range(src.fileno(), dst, left, None, end)
-                        if n <= 0:
-                            break
-                        left -= n; end += n
-                except (AttributeError, OSError):
-                    pass
-                while left > 0:                                     # not supported here (or stopped early): plain copy of the rest
-                    buf = os.pread(src.fileno(), min(left, 16 << 20), os.fstat(src.fileno()).st_size - left)
-                    if not buf:
-                        raise OSError(f"short read while gathering {parts[g]}")
-                    os.pwrite(dst, buf, end)
-                    left -= len(buf); end += len(buf)
-            os.remove(parts[g])
+        for _, _, err in results:
+            if err is not None:
+                raise err
+        t2 = time.perf_counter()
+        dst = os.open(out, os.O_WRONLY)                             # host gather: region order = coordinate order
+        try:
+            end = os.fstat(dst).st_size
+            for part in parts[1:]:
+                with open(part, "rb") as src:
+                    left = os.fstat(src.fileno()).st_size
+                    try:                                            # in-kernel copy (no bounce through user space)
+                        while left > 0:
+                            n = os.copy_file_range(src.fileno(), dst, left, None, end)
+                            if n <= 0:
+                                break
+                            left -= n; end += n
+                    except (AttributeError, OSError):
+                        pass
+                    while left > 0:                                 # not supported here (or stopped early): plain copy of the rest
+                        buf = os.pread(src.fileno(), min(left, 16 << 20), os.fstat(src.fileno()).st_size - left)
+                        if not buf:
+                            raise OSError(f"short read while gathering {part}")
+                        os.pwrite(dst, buf, end)
+                        left -= len(buf); end += len(buf)
+        finally:
+            os.close(dst)
+        tm["concat"] += time.perf_counter() - t2
     finally:
-        os.close(dst)
-    tm["concat"] += time.perf_counter() - t2
+        for part in parts[1:]:
+            with contextlib.suppress(FileNotFoundError):
+                os.remove(part)
     for k in ("gather", "gpu_wait", "format", "write"):
-        tm[k] += sum(x[k] for x in thread_tm)
+        tm[k] += sum(x[k] for x in shard_tm)
     tm["shards"] = [{"device": int(devices[g]), "reads": int(results[g][0]), "cell_updates": int(shard_load[g]), "seconds": round(results[g][1], 4)}
                     for g in range(G)]
-    written = sum(n for n, _, _ in results)
-    with cfg.counter.get_lock():
-        cfg.counter.value += written
-    bam.close()
-    return written
-
-
-import threading as _threading  # noqa: E402
-_PIPE_LOCK = _threading.Lock()
-_MALLOC_TUNED = False
+    return sum(n for n, _, _ in results)
 
 
 def _keep_freed_buffers_mapped():
@@ -531,17 +536,9 @@ def realign_bam(bam_fn, fasta, out_prefix=None, regions=None, max_reads=0, argv=
     formats (native) and writes batch k-1.  One shared reference slice is uploaded per batch.
     timings: optional dict that receives host seconds per phase (open, gather, gpu_wait, format = formatting + the append to the
     file, write = 0 since the formatter threads write themselves); timings["trace"] = [] collects (seconds, event) of every step.
-    devices: CUDA device indices; more than one -> realign_bam_sharded (one region-shard pipeline per device, ordered gather)."""
-    if devices is not None and len(devices) > 1:
-        return realign_bam_sharded(bam_fn, fasta, list(devices), out_prefix=out_prefix, regions=regions, max_reads=max_reads, argv=argv,
-                                   max_batch_ops=max_batch_ops, n_threads=n_threads, timings=timings, n_inflight=n_inflight)
-    import queue
-    import threading
-    import time
+    devices: CUDA device indices; more than one: one region-shard pipeline per device, gathered in order into one file
+    (_realign_sharded; the whole file is loaded, no streaming)."""
     from .bam import _tables
-    from .aln import _report
-    from .cig import bases_to_int
-    from .engine import NPORE_OUT_NO_EXPANDED, NPORE_OUT_RLE, NPORE_OUT_STANDARDIZE, PackedBatch
     tm = timings if timings is not None else {}
     for k in ("open", "gather", "gpu_wait", "format", "write"):
         tm.setdefault(k, 0.0)
@@ -555,117 +552,53 @@ def realign_bam(bam_fn, fasta, out_prefix=None, regions=None, max_reads=0, argv=
         print(f"\nERROR: BAM file '{bam_fn}' not found.")
         sys.exit(1)
     fa = read_fasta(fasta) if isinstance(fasta, str) else fasta
-    # several regions are served region by region (bam.pyx:27-28), which needs the whole file at hand
-    bam = NativeBam(bam_fn, n_threads, window_bytes=window_bytes if not (regions and len(regions) > 1) else 0)
+    devices = list(devices or [None])
+    # several regions are served region by region (bam.pyx:27-28), and region shards are cut from every record's span: both
+    # need the whole file at hand
+    streaming = len(devices) == 1 and not (regions and len(regions) > 1)
+    bam = NativeBam(bam_fn, n_threads, window_bytes=window_bytes if streaming else 0)
     mark("bam open")
-    streaming = bam.window_bytes > 0
-    # the header (and the truncation of a previous output: ~2 ms for a 60 MB file) is written beside the first window's inflate;
-    # the writer thread waits for it before it opens the file
-    header_err = []
+    out = f"{cfg.args.out_prefix}.sam"
 
-    def write_header():
-        try:
-            create_header(f"{cfg.args.out_prefix}.sam", bam.refs, argv)
-            mark("header written")
-        except Exception as e:      # noqa: BLE001
-            header_err.append(e)
+    def open_out():
+        # called by the writer thread: the header (and the truncation of a previous output: ~2 ms for a 60 MB file) is written
+        # beside the first window's inflate
+        create_header(out, bam.refs, argv)
+        mark("header written")
+        return os.open(out, os.O_WRONLY)
 
-    header = threading.Thread(target=write_header, daemon=True)
-    header.start()
-    sub, npt = _tables()
-    pipe = _pipeline(sub, npt, n_inflight, devices[0] if devices else None)
-    flags = NPORE_OUT_STANDARDIZE | NPORE_OUT_RLE | NPORE_OUT_NO_EXPANDED
-    tm["open"] += time.perf_counter() - t0
-    mark("opened")
-    # stage 3 (own thread): wait for batch k, format its records, append them to the SAM -- in submit order
-    pending = queue.Queue(maxsize=n_inflight + 1)
-    state = {"written": 0, "error": None}
-
-    def retire_loop():
-        path = f"{cfg.args.out_prefix}.sam"
-        header.join()
-        if header_err:
-            state["error"] = header_err[0]
-        fd = os.open(path, os.O_WRONLY) if not header_err else -1
-        end = os.path.getsize(path) if fd >= 0 else 0     # the header is there already
-        while True:
-            item = pending.get()
-            if item is None:
-                if fd >= 0:
-                    os.close(fd)
-                return
-            if state["error"] is not None:
-                continue                              # keep draining so that the producer never blocks
-            try:
-                fut, cols, g, n = item
-                t1 = time.perf_counter()
-                res, st_ = fut.result()
-                t2 = time.perf_counter()
-                mark(f"gpu done n={n} kernels_ms={st_['ms_kernels_total']:.1f} h2d_ms={st_['ms_h2d']:.1f} plan_ms={st_['ms_plan']:.1f} d2h_ms={st_['ms_d2h']:.1f} "
-                     f"warps/SM={st_['fwd_warps_per_sm']} context from {1e3 * (st_['wall'][0] - t0):.1f} ms, buffers {1e3 * (st_['wall'][1] - t0):.1f}, "
-                     f"to {1e3 * (st_['wall'][2] - t0):.1f} ms")
-                _report(res.status[:n], "realign_read")
-                end += len(format_sam(bam, None, g, res.rle, res.rle_off[:n + 1], n_threads, cols=cols, fd=fd, offset=end))
-                t3 = time.perf_counter()
-                mark("formatted + written")
-                tm["gpu_wait"] += t2 - t1; tm["format"] += t3 - t2; tm["write"] += time.perf_counter() - t3
-                state["written"] += n
-                with cfg.counter.get_lock():
-                    cfg.counter.value += n
-            except Exception as e:                    # noqa: BLE001
-                state["error"] = e
-
-    retire = threading.Thread(target=retire_loop, daemon=True)
-    retire.start()
-    # the text gather runs right after a submit: leave cores to the GPU worker thread that has just been woken (on 16 cores a
-    # 16-thread gather delayed the start of the upload by 2 ms) and to the writer
-    nt_text = max(1, (n_threads or os.cpu_count() or 1) - int(os.environ.get("NPORE_SPARE_CORES", "3")))
     try:
-        kept = 0
-        while True:
-            if streaming:
-                t1 = time.perf_counter()
-                more = bam.advance()
-                tm["open"] += time.perf_counter() - t1
-                mark(f"window of {more} records")
-                if not more:
-                    break
-            for ctg, sel in select_reads(bam, regions, (max_reads - kept) if max_reads else 0):
-                kept += len(sel)
-                contig = fa[ctg]
-                ops = np.cumsum((bam.end[sel] - bam.pos[sel]).astype(np.int64) + bam.aln_len[sel])
-                cut = 0
-                while cut < len(sel) and state["error"] is None:
-                    stop = max(cut + 1, int(np.searchsorted(ops, (ops[cut - 1] if cut else 0) + max_batch_ops, "right")))
-                    part = sel[cut:stop]
-                    t1 = time.perf_counter()
-                    nib, nib_start = bam.gather_nib(part, n_threads)          # the upload: BAM's own 4-bit bases + CIGAR words
-                    mark("nib gathered")
-                    cig_words, cig_off = bam.gather_cigar(part, n_threads)
-                    mark("cigar gathered")
-                    lo, hi = int(bam.pos[part].min()), int(bam.end[part].max())
-                    # base codes of the batch's reference span only (not the contig: 250 Mb of chr1 for a window that covers 1 Mb)
-                    packed = PackedBatch.from_flat_shared_nib(bases_to_int(contig[lo:hi].upper()), bam.pos[part].astype(np.int64) - lo, bam.end[part] - bam.pos[part],
-                                                              nib, nib_start, bam.aln_len[part], cig_words, cig_off)
-                    fut = pipe.submit(packed, flags)                          # the GPU starts; the SAM-text gather runs beside it
-                    mark(f"submitted n={len(part)}")
-                    g = bam.gather(part, nt_text, want_codes=False, want_cigar=False)    # ASCII bases / qualities / names
-                    mark("text gathered")
-                    item = (fut, take_columns(bam, part), g, len(part))
-                    tm["gather"] += time.perf_counter() - t1
-                    pending.put(item)                                        # blocks while n_inflight + 1 batches are unfinished
-                    cut = stop
-                if max_reads and kept >= max_reads:
-                    break
-            if not streaming or (max_reads and kept >= max_reads) or state["error"] is not None:
-                break
+        sub, npt = _tables()
+        with _PIPE_LOCK:
+            pipes = [_pipeline(sub, npt, n_inflight, d) for d in devices]
+        tm["open"] += time.perf_counter() - t0
+        mark("opened")
+        if len(devices) > 1:
+            written = _realign_sharded(bam, fa, pipes, devices, open_out, regions, max_reads, max_batch_ops, n_threads, n_inflight,
+                                       tm, mark, t0)
+        else:
+            def segments():
+                kept = 0
+                while True:
+                    if bam.window_bytes:
+                        t1 = time.perf_counter()
+                        more = bam.advance()
+                        tm["open"] += time.perf_counter() - t1
+                        mark(f"window of {more} records")
+                        if not more:
+                            return
+                    for ctg, sel in select_reads(bam, regions, (max_reads - kept) if max_reads else 0):
+                        kept += len(sel)
+                        yield ctg, sel
+                    if not bam.window_bytes or (max_reads and kept >= max_reads):
+                        return
+
+            # the text gather runs right after a submit: leave cores to the GPU worker thread that has just been woken (on 16
+            # cores a 16-thread gather delayed the start of the upload by 2 ms) and to the writer
+            nt_text = max(1, (n_threads or os.cpu_count() or 1) - int(os.environ.get("NPORE_SPARE_CORES", "3")))
+            written = _realign_segments(bam, segments(), fa, pipes[0], open_out, tm, n_threads, nt_text, max_batch_ops, n_inflight, mark, t0)
     finally:
-        pending.put(None)
-        retire.join()
-    if state["error"] is not None:
-        raise state["error"]
-    written = state["written"]
-    bam.close()
+        bam.close()
     mark("closed")
     return written
 

@@ -7,7 +7,7 @@
                    one per GPU (SURVEY.md 8(e)); no collective: every shard is realigned independently and the
                    host concatenates the per-GPU outputs in region order.
   cut_balanced     the same cut for items that are ALREADY in (contig, start) order: owner shard of every item, contiguous
-                   and non-decreasing, by the item's load midpoint (bamio.realign_bam_sharded).
+                   and non-decreasing, by the item's load midpoint (bamio.realign_bam with devices=[...]).
 """
 import numpy as np
 
