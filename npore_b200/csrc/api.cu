@@ -30,8 +30,10 @@
 
 namespace {
 
-struct DevBuf {
+struct DevBuf {       // device memory owned by its context: freed when the context is deleted
     void *p = nullptr; size_t cap = 0;
+    DevBuf &operator=(DevBuf &&) = delete;     // and with it both copies: a block has one owner
+    ~DevBuf() { release(); }
     // grow-only; contents are NOT preserved.  The new block is allocated before the old one is released, so a failed growth
     // leaves the buffer usable at its old size; only if both do not fit is the old block given up first.
     cudaError_t ensure(size_t bytes) {
@@ -56,6 +58,8 @@ struct DevBuf {
 
 struct HostBuf {      // pinned staging owned by the library (download path)
     void *p = nullptr; size_t cap = 0;
+    HostBuf &operator=(HostBuf &&) = delete;   // and with it both copies
+    ~HostBuf() { if (p) cudaFreeHost(p); }
     cudaError_t ensure(size_t bytes) {
         if (bytes <= cap) return cudaSuccess;
         if (p) cudaFreeHost(p);
@@ -64,10 +68,19 @@ struct HostBuf {      // pinned staging owned by the library (download path)
         if (e == cudaSuccess) cap = bytes + bytes / 8 + 256;
         return e;
     }
-    void release() { if (p) cudaFreeHost(p); p = nullptr; cap = 0; }
+};
+
+// pinned block npore_run fills for npore_download: per-item lengths, status, run-length counts; chunk results; counters at the end
+struct SmallBlock {
+    static size_t bytes(int n, int64_t n_chunks) { return (size_t)n * 12 + (size_t)n_chunks * sizeof(ChunkOut) + 64; }
+    int32_t *len, *status, *rle_len; ChunkOut *chunk_out; int *counters;
+    SmallBlock(void *base, int n, int64_t n_chunks)
+        : len(static_cast<int32_t *>(base)), status(len + n), rle_len(status + n), chunk_out(reinterpret_cast<ChunkOut *>(rle_len + n + (n & 1))),
+          counters(reinterpret_cast<int *>(static_cast<char *>(base) + bytes(n, n_chunks) - 16)) {}
 };
 
 struct SubBatch { int first, count; };
+enum { EV_COPY_BEGIN, EV_COPY_END, EV_PLAN_BEGIN, EV_PLAN_END, EV_FINISH_BEGIN, EV_FINISH_END, N_EVENTS };   // ctx->ev
 
 std::atomic<long long> g_par_inflight[64];  // effective parallelism (forward_team) of the forward launches in flight per device, all contexts
 std::atomic<int> g_ctx_on_device[64];      // live contexts per device: they share the scratch budget (PipelinedRealigner)
@@ -76,10 +89,12 @@ std::atomic<int> g_ctx_on_device[64];      // live contexts per device: they sha
 
 struct npore_ctx {
     int device = 0, sm_count = 0;
+    std::atomic<int> *on_device = nullptr;           // the device's entries in g_ctx_on_device and g_par_inflight, set
+    std::atomic<long long> *par_inflight = nullptr;  // once the context is counted (devices 0-63)
     cudaStream_t stream = nullptr;
     bool own_stream = true;
     AlignParams P{};
-    int cpl = 2, tbs = 2, np_n = 0;
+    int cpl = 2, tbs = 2;
     size_t scratch_budget = 0;
     DevBuf d_sub, d_np;
     // batch-resident
@@ -90,19 +105,23 @@ struct npore_ctx {
     DevBuf d_colrec, d_relaid, d_rowrec, d_raw_ref, d_raw_seq, d_tb, d_rr_q, d_rr_ctl, d_rr_state;
     int rr_slice = 512;
     DevBuf d_chunk_dst, d_part_cnt;
-    DevBuf d_cm[22];                     // npore_confusion_batch staging (kept between calls)
+    // npore_confusion_batch staging (kept between calls); npore_get_np_info_batch shares ref_codes, ref_off, raw, ebits and out
+    struct {
+        DevBuf range_start, range_end, ref_ascii, ref_off, ref_codes, raw, ebits;
+        DevBuf read_pos, seq, qual, seq_off, rle, cig_off, g_roff, g_qoff, read_end;
+        DevBuf range_reads, range_reads_off, list_maxend, line_of, pos_off;
+        DevBuf out;                    // zeroed: the counts, the error flag, the coverage difference array
+    } pileup;
     HostBuf h_small;
-    int64_t pack_ops_total = 0, pack_rle_total = 0;
     std::vector<ItemDesc> items;
-    std::vector<int32_t> order;
-    std::vector<int32_t> chunk_bmax;
+    std::vector<int32_t> order, chunk_bmax;
     std::vector<ChunkSlot> slots;
     std::vector<SubBatch> subs;
-    int64_t n_chunks = 0, total_ops = 0, total_rle = 0, total_words = 0;
-    bool uploaded = false, ran = false, counted = false, budget_fixed = false;
+    int64_t n_chunks = 0, total_ops = 0, total_rle = 0;
+    bool uploaded = false, ran = false, budget_fixed = false;
     uint32_t run_flags = 0;
     npore_stats stats{};
-    cudaEvent_t ev[8]{};
+    cudaEvent_t ev[N_EVENTS]{};
     std::vector<cudaEvent_t> sub_ev;     // 4 per sub-batch
     std::string err;
 };
@@ -197,7 +216,7 @@ inline int forward_team(const npore_ctx *ctx, int nc32, int n_chunks, double par
     if (nc32 == 8) return 4;
     if (nc32 == 4) return 2;
     const double slots = ctx->sm_count * 16.0;          // resident one-warp chunks of <2,1>
-    const bool siblings = ctx->device < 64 && g_ctx_on_device[ctx->device].load() > 1;      // a pipeline: the next batch is on its way
+    const bool siblings = ctx->on_device && ctx->on_device->load() > 1;      // a pipeline: the next batch is on its way
     if (others > 0.0 || siblings) return 4.0 * (par + others) <= slots ? 2 : 1;
     // us per anti-diagonal of one chunk (r = 30, 10 kb reads) against the share of the warp slots the launch occupies
     static const double S1[][2] = {{0.04, 0.536}, {0.10, 0.559}, {0.21, 0.582}, {0.32, 0.635}, {0.42, 0.652}, {0.63, 0.750}, {0.84, 0.897}, {1.0, 0.93}};
@@ -211,8 +230,8 @@ inline int forward_team(const npore_ctx *ctx, int nc32, int n_chunks, double par
 __global__ void unpack_nib_kernel(const ItemDesc *items, const uint8_t *nib, const int64_t *nib_start, uint8_t *codes, int parts)
 {
     const ItemDesc &I = items[blockIdx.x];
-    const int per = (I.seq_len + parts - 1) / parts;
-    const int lo = min(I.seq_len, (int)blockIdx.y * per), hi = min(I.seq_len, lo + per);
+    int lo, hi;
+    np_slice(I.seq_len, parts, blockIdx.y, lo, hi);
     const int64_t ns = nib_start[blockIdx.x];
     uint8_t *out = codes + I.seq_start;
     for (int t = lo + threadIdx.x; t < hi; t += blockDim.x) {
@@ -221,6 +240,277 @@ __global__ void unpack_nib_kernel(const ItemDesc *items, const uint8_t *nib, con
         const uint32_t v = (k & 1) ? (b & 15u) : (b >> 4);
         out[t] = v == 1u ? 1 : v == 2u ? 2 : v == 4u ? 3 : v == 8u ? 4 : 0;      // "=ACMGRSVTWYHKDBN": A=1 C=2 G=4 T=8
     }
+}
+
+struct InFlight {    // this pass's entry in par_inflight: set per sub-batch, withdrawn when the pass has synchronised (or failed)
+    std::atomic<long long> *g; long long mine = 0;
+    long long set(long long par) { const long long before = g ? g->fetch_add(par - mine) : mine; const long long o = before - mine; mine = par; return o > 0 ? o : 0; }
+    ~InFlight() { if (g && mine) g->fetch_sub(mine); }
+};
+
+// Sub-batches: greedy over `order` under the scratch budget (sizes from the host-side upper bounds).  The budget is this
+// context's share of the device (contexts on one device run side by side: PipelinedRealigner); if the scratch still does not
+// fit (other tenants of the device), the batch is re-cut with half the budget instead of failing.  *rr_cap: run-queue capacity.
+int cut_sub_batches(npore_ctx *ctx, int *rr_cap)
+{
+    const int64_t nchunks = ctx->n_chunks;
+    size_t budget = ctx->scratch_budget;
+    if (!ctx->budget_fixed && ctx->on_device) budget /= (size_t)std::max(1, ctx->on_device->load());
+    for (int attempt = 0;; attempt++) {
+        ctx->slots.assign(nchunks, ChunkSlot{});
+        ctx->subs.clear();
+        size_t max_col = 0, max_row = 0, max_tb = 0;
+        const size_t per_entry = 32 + 8 + 8 + 4 + 8;   // colrec, relaid, raw_ref, rowrec, raw_seq
+        size_t col = 0, row = 0, tb = 0; int first = 0;
+        for (int64_t k = 0; k < nchunks; k++) {
+            const int bm = ctx->chunk_bmax[ctx->order[k]];
+            const size_t ent = (size_t)((bm + 32 * ctx->cpl + 128 + 31) & ~31);
+            const size_t need = (col + ent) * per_entry + (tb + bm) * (size_t)(64 * ctx->tbs);
+            if (k > first && need > budget) {
+                ctx->subs.push_back({first, (int)(k - first)});
+                max_col = std::max(max_col, col); max_row = std::max(max_row, row); max_tb = std::max(max_tb, tb);
+                col = row = tb = 0; first = (int)k;
+            }
+            ChunkSlot &sl = ctx->slots[k];
+            sl.col_off = (int64_t)col; sl.row_off = (int64_t)row; sl.tb_off = (int64_t)tb;
+            sl.col_cap = sl.row_cap = (int32_t)ent;
+            col += ent; row += ent; tb += bm;
+        }
+        if (nchunks > first) {
+            ctx->subs.push_back({first, (int)(nchunks - first)});
+            max_col = std::max(max_col, col); max_row = std::max(max_row, row); max_tb = std::max(max_tb, tb);
+        }
+        cudaError_t e = ctx->d_colrec.ensure(max_col * 32 + 64);
+        if (e == cudaSuccess) e = ctx->d_relaid.ensure(max_col * 8 + 64);
+        if (e == cudaSuccess) e = ctx->d_raw_ref.ensure(max_col * 8 + 64);
+        if (e == cudaSuccess) e = ctx->d_rowrec.ensure(max_row * 4 + 64);
+        if (e == cudaSuccess) e = ctx->d_raw_seq.ensure(max_row * 8 + 64);
+        if (e == cudaSuccess) e = ctx->d_tb.ensure(max_tb * (size_t)(64 * ctx->tbs) + 256);
+        if (e == cudaSuccess) break;
+        cudaGetLastError();
+        if (e != cudaErrorMemoryAllocation || attempt >= 4 || ctx->subs.size() >= (size_t)std::max<int64_t>(nchunks, 1))
+            return fail(ctx, e == cudaErrorMemoryAllocation ? NPORE_ERR_OOM : NPORE_ERR_CUDA, "scratch allocation", e);
+        ctx->d_tb.release(); ctx->d_colrec.release();          // give back what the failed attempt may have grabbed
+        budget /= 2;
+    }
+    int max_sub = 1;
+    for (const SubBatch &sb : ctx->subs) max_sub = std::max(max_sub, sb.count);
+    *rr_cap = 1;
+    while (*rr_cap < 2 * max_sub + 16384) *rr_cap <<= 1;
+    CU(ctx->d_rr_q.ensure(sizeof(int) * (size_t)*rr_cap));
+    CU(ctx->d_rr_ctl.ensure(64));
+    CU(ctx->d_rr_state.ensure(sizeof(uint32_t) * fwd_rr_state_words(ctx->cpl) * (size_t)max_sub));
+    while (ctx->sub_ev.size() < 4 * ctx->subs.size()) {
+        cudaEvent_t e; CU(cudaEventCreate(&e)); ctx->sub_ev.push_back(e);
+    }
+    if (nchunks) CU(cudaMemcpyAsync(ctx->d_slots.p, ctx->slots.data(), sizeof(ChunkSlot) * (size_t)nchunks, cudaMemcpyHostToDevice, ctx->stream));
+    return NPORE_OK;
+}
+
+int launch_forward_for(npore_ctx *ctx, int team, bool wide, const ForwardArgs &fa, int n)
+{
+    switch (ctx->cpl * 100 + team * 10 + (wide ? 1 : 0)) {      // digits: cpl, team, WIDE (the second pass: forward.cuh)
+    case 110: return launch_forward<1, 1, false>(ctx, fa, n);
+    case 210: return launch_forward<2, 1, false>(ctx, fa, n);
+    case 220: return launch_forward<1, 2, false>(ctx, fa, n);
+    case 410: return launch_forward<4, 1, false>(ctx, fa, n);
+    case 420: return launch_forward<2, 2, false>(ctx, fa, n);
+    case 810: return launch_forward<8, 1, false>(ctx, fa, n);
+    case 820: return launch_forward<4, 2, false>(ctx, fa, n);
+    case 840: return launch_forward<2, 4, false>(ctx, fa, n);
+    case 111: return launch_forward<1, 1, true>(ctx, fa, n);
+    case 211: return launch_forward<2, 1, true>(ctx, fa, n);
+    case 221: return launch_forward<1, 2, true>(ctx, fa, n);
+    case 411: return launch_forward<4, 1, true>(ctx, fa, n);
+    case 421: return launch_forward<2, 2, true>(ctx, fa, n);
+    case 821: return launch_forward<4, 2, true>(ctx, fa, n);
+    case 811:                                      // <8, 1, true> is not instantiated: W > 128 runs as teams of four
+    case 841:                                      // forward_team yields no other pair: the last case takes the rest
+    default: return launch_forward<2, 4, true>(ctx, fa, n);
+    }
+}
+
+int run_sub_batch(npore_ctx *ctx, size_t si, bool wide, int rr_cap, InFlight &inflight)
+{
+    const SubBatch &sb = ctx->subs[si];
+    cudaEvent_t *ev = &ctx->sub_ev[4 * si];          // annotate, forward and traceback each run between two of them
+    AnnotateArgs aa{};
+    aa.chunks = ctx->d_chunks.as<ChunkDesc>(); aa.slots = ctx->d_slots.as<ChunkSlot>() + sb.first;
+    aa.order = ctx->d_order.as<int32_t>() + sb.first; aa.n = sb.count; aa.items = ctx->d_items.as<ItemDesc>();
+    aa.ref_codes = ctx->d_ref.as<uint8_t>(); aa.seq_codes = ctx->d_seq.as<uint8_t>();
+    aa.raw_ref = ctx->d_raw_ref.as<uint8_t>(); aa.raw_seq = ctx->d_raw_seq.as<uint8_t>();
+    aa.colrec = ctx->d_colrec.as<uint4>(); aa.relaid = ctx->d_relaid.as<uint2>(); aa.rowrec = ctx->d_rowrec.as<uint32_t>();
+    aa.max_n = ctx->P.max_n; aa.max_l = ctx->P.max_l; aa.nc = 32 * ctx->cpl; aa.inf_row = ctx->P.np_rows;
+    int bm = 1;
+    double bsum = 0.0;
+    for (int k = 0; k < sb.count; k++) { const int b = ctx->chunk_bmax[ctx->order[sb.first + k]]; bm = std::max(bm, b); bsum += b; }
+    const long long par = (long long)(bsum / bm) + 1;
+    const long long others = inflight.set(par);                  // the other contexts' launches on this device
+    const int team = forward_team(ctx, ctx->cpl, sb.count, (double)par, (double)others);      // warps per chunk of this sub-batch's forward launch
+    aa.cpl = ctx->cpl / team;
+    CU(cudaEventRecord(ev[0], ctx->stream));
+    {   // equality words of all periods in dynamic shared memory: 6 planes of (longest slice / 32 + 2) words
+        aa.e6_stride = (bm + 1 + 31) / 32 + 2;
+        const size_t dyn = (size_t)NP_MAXN * aa.e6_stride * sizeof(uint32_t);
+        if (dyn > 48 * 1024) CU(cudaFuncSetAttribute(annotate_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn));
+        annotate_kernel<<<2 * sb.count, ANN_THREADS, dyn, ctx->stream>>>(aa);
+    }
+    CU(cudaGetLastError()); ctx->stats.launches++;
+    CU(cudaEventRecord(ev[1], ctx->stream));
+
+    ForwardArgs fa{};
+    fa.chunks = aa.chunks; fa.slots = aa.slots; fa.order = aa.order; fa.n = sb.count;
+    fa.items = aa.items; fa.bits = ctx->d_bits.as<uint32_t>(); fa.err = ctx->d_counter.as<int>();
+    fa.ovf = wide ? ctx->d_ovf.as<uint4>() : nullptr; fa.ovf_cap = 65536; fa.ovf_cnt = ctx->d_counter.as<int>() + 1;
+    fa.ref_codes = aa.ref_codes; fa.seq_codes = aa.seq_codes; fa.colrec = aa.colrec; fa.relaid = aa.relaid; fa.rowrec = aa.rowrec;
+    fa.tb = ctx->d_tb.as<uint16_t>(); fa.tab = ctx->d_np.as<float>(); fa.sub_tab = ctx->d_sub.as<float>();
+    fa.out = ctx->d_chunk_out.as<ChunkOut>();
+    fa.P = ctx->P;
+    fa.rr_q = ctx->d_rr_q.as<int>(); fa.rr_mask = rr_cap - 1; fa.rr_ctl = ctx->d_rr_ctl.as<int>();
+    fa.rr_state = ctx->d_rr_state.as<uint32_t>(); fa.rr_slice = ctx->rr_slice;
+    CU(cudaMemsetAsync(ctx->d_rr_state.p, 0, sizeof(uint32_t) * fwd_rr_state_words(ctx->cpl) * (size_t)sb.count, ctx->stream));
+    rr_init_kernel<<<64, 256, 0, ctx->stream>>>(fa.rr_q, rr_cap, sb.count, fa.rr_ctl);
+    CU(cudaGetLastError()); ctx->stats.launches++;
+    if (int rc = launch_forward_for(ctx, team, wide, fa, sb.count); rc != NPORE_OK) return rc;
+    ctx->stats.launches++;
+    CU(cudaEventRecord(ev[2], ctx->stream));
+
+    TracebackArgs ta{};
+    ta.chunks = aa.chunks; ta.slots = aa.slots; ta.order = aa.order; ta.n = sb.count; ta.items = aa.items;
+    ta.bits = fa.bits; ta.cum = ctx->d_cum.as<uint32_t>(); ta.ref_codes = aa.ref_codes; ta.seq_codes = aa.seq_codes;
+    ta.tb = fa.tb; ta.ops = ctx->d_scratch_ops.as<uint8_t>(); ta.out = fa.out;
+    ta.r = ctx->P.r; ta.W = ctx->P.W; ta.cpl = ctx->cpl; ta.tbs = ctx->tbs;
+    ta.ovf = fa.ovf; ta.ovf_cnt = fa.ovf_cnt; ta.ovf_cap = fa.ovf_cap; ta.n_sat = ctx->d_counter.as<int>() + 2;
+    traceback_kernel<<<(sb.count + TB_THREADS / 32 - 1) / (TB_THREADS / 32), TB_THREADS, 0, ctx->stream>>>(ta);
+    CU(cudaGetLastError()); ctx->stats.launches++;
+    CU(cudaEventRecord(ev[3], ctx->stream));
+    for (int k = 0; k < sb.count; k++) ctx->stats.tb_bytes += (int64_t)ctx->chunk_bmax[ctx->order[sb.first + k]] * 64 * ctx->tbs;
+    return NPORE_OK;
+}
+
+// the finish kernels; per-item sizes / status / chunk results and the counters travel with the run (npore_download knows exact sizes)
+int launch_finish(npore_ctx *ctx, uint32_t flags, int parts, int max_ops)
+{
+    const int n = (int)ctx->items.size();
+    npore_stats &S = ctx->stats;
+    const bool want_ops = !(flags & NPORE_OUT_NO_EXPANDED), want_rle = (flags & NPORE_OUT_RLE) != 0;
+    CU(cudaEventRecord(ctx->ev[EV_FINISH_BEGIN], ctx->stream));
+    CU(ctx->h_small.ensure(SmallBlock::bytes(n, ctx->n_chunks)));
+    const SmallBlock hs(ctx->h_small.p, n, ctx->n_chunks);
+    if (n) {
+        FinishArgs fa{};
+        fa.items = ctx->d_items.as<ItemDesc>(); fa.n_items = n; fa.chunk_out = ctx->d_chunk_out.as<ChunkOut>();
+        fa.scratch = ctx->d_scratch_ops.as<uint8_t>(); fa.ops = ctx->d_ops.as<uint8_t>();
+        fa.item_len = ctx->d_item_len.as<int32_t>(); fa.item_status = ctx->d_item_status.as<int32_t>();
+        fa.ref_codes = ctx->d_ref.as<uint8_t>(); fa.seq_codes = ctx->d_seq.as<uint8_t>();
+        fa.rleA = ctx->d_rleA.as<uint32_t>(); fa.rleB = ctx->d_rleB.as<uint32_t>();
+        fa.rle_len = ctx->d_rle_len.as<int32_t>(); fa.rle_which = ctx->d_rle_which.as<int32_t>();
+        fa.to_m = (flags & NPORE_OUT_STANDARDIZE) ? 1 : 0;
+        fa.ops_off = ctx->d_ops_off.as<int64_t>(); fa.rle_off = ctx->d_rle_off.as<int64_t>();
+        fa.pack_ops = ctx->d_pack_ops.as<uint8_t>(); fa.pack_rle = ctx->d_pack_rle.as<uint32_t>();
+        CU(ctx->d_chunk_dst.ensure(sizeof(int32_t) * (size_t)std::max<int64_t>(ctx->n_chunks, 1)));
+        fa.chunks = ctx->d_chunks.as<ChunkDesc>(); fa.n_chunks = (int)ctx->n_chunks;
+        fa.chunk_dst = ctx->d_chunk_dst.as<int32_t>(); fa.parts = parts; fa.part_cnt = ctx->d_part_cnt.as<int32_t>();
+        const dim3 grid_np(n, parts);
+        item_len_kernel<<<n, FIN_THREADS, 0, ctx->stream>>>(fa);
+        CU(cudaGetLastError()); S.launches++;
+        if (ctx->n_chunks) {
+            gather_kernel<<<(unsigned)ctx->n_chunks, FIN_THREADS, 0, ctx->stream>>>(fa);
+            CU(cudaGetLastError()); S.launches++;
+        }
+        if (flags & (NPORE_OUT_RLE | NPORE_OUT_STANDARDIZE)) {
+            if (parts > 1) { rle_count_kernel<<<grid_np, FIN_WIDE, 0, ctx->stream>>>(fa); S.launches++; }
+            rle_start_kernel<<<grid_np, FIN_WIDE, 0, ctx->stream>>>(fa);
+            rle_word_kernel<<<grid_np, FIN_WIDE, 0, ctx->stream>>>(fa);
+            CU(cudaGetLastError()); S.launches += 2;
+        } else CU(cudaMemsetAsync(ctx->d_rle_len.p, 0, sizeof(int32_t) * (size_t)n, ctx->stream));
+        if (flags & NPORE_OUT_STANDARDIZE) {
+            // items with many run-length groups (haplotypes) get a whole CTA each; NPORE_STD_LONG_MIN overrides the split (tests)
+            int long_min = 4096;
+            if (const char *e = getenv("NPORE_STD_LONG_MIN")) long_min = std::max(1, atoi(e));
+            const bool any_long = max_ops >= long_min;              // an item cannot have more groups than ops
+            // the long-item kernel goes first and marks its items (rle_which = 1); the per-warp kernel takes what is left.
+            // (Both look at the group count BEFORE standardisation: the sweeps change it.)
+            if (any_long) {
+                standardize_long_kernel<<<n, FIN_WIDE, 0, ctx->stream>>>(fa, long_min);
+                CU(cudaGetLastError()); S.launches++;
+            }
+            standardize_kernel<<<(n + FIN_THREADS / 32 - 1) / (FIN_THREADS / 32), FIN_THREADS, 0, ctx->stream>>>(fa);
+            CU(cudaGetLastError()); S.launches++;
+            if (want_ops) {
+                if (parts > 1) { expand_count_kernel<<<grid_np, FIN_WIDE, 0, ctx->stream>>>(fa); S.launches++; }
+                expand_fill_kernel<<<grid_np, FIN_WIDE, 0, ctx->stream>>>(fa);
+                CU(cudaGetLastError()); S.launches++;
+            }
+        }
+        scan_kernel<<<1, 1024, 0, ctx->stream>>>(fa);
+        CU(cudaGetLastError()); S.launches++;
+        if (want_ops || want_rle) {
+            pack_kernel<<<grid_np, FIN_WIDE, 0, ctx->stream>>>(fa, want_ops ? 1 : 0, want_rle ? 1 : 0);
+            CU(cudaGetLastError()); S.launches++;
+        }
+        CU(cudaMemcpyAsync(hs.len, ctx->d_item_len.p, 4 * (size_t)n, cudaMemcpyDeviceToHost, ctx->stream));
+        CU(cudaMemcpyAsync(hs.status, ctx->d_item_status.p, 4 * (size_t)n, cudaMemcpyDeviceToHost, ctx->stream));
+        CU(cudaMemcpyAsync(hs.rle_len, ctx->d_rle_len.p, 4 * (size_t)n, cudaMemcpyDeviceToHost, ctx->stream));
+        if (ctx->n_chunks) CU(cudaMemcpyAsync(hs.chunk_out, ctx->d_chunk_out.p, sizeof(ChunkOut) * (size_t)ctx->n_chunks, cudaMemcpyDeviceToHost, ctx->stream));
+    }
+    CU(cudaMemcpyAsync(hs.counters, ctx->d_counter.p, 12, cudaMemcpyDeviceToHost, ctx->stream));
+    CU(cudaEventRecord(ctx->ev[EV_FINISH_END], ctx->stream));
+    return NPORE_OK;
+}
+
+int run_pass(npore_ctx *ctx, uint32_t flags, bool wide, int *n_sat)
+{
+    CU(cudaSetDevice(ctx->device));
+    ctx->ran = false;
+    InFlight inflight{ctx->par_inflight};
+    const int n = (int)ctx->items.size();
+    npore_stats &S = ctx->stats;
+    S.launches = 0; S.tb_bytes = 0;
+    ctx->run_flags = flags;
+    if (flags & (NPORE_OUT_RLE | NPORE_OUT_STANDARDIZE))
+        for (DevBuf *d : {&ctx->d_rleA, &ctx->d_rleB}) CU(d->ensure(sizeof(uint32_t) * (size_t)(ctx->total_ops + 64)));
+    if (!(flags & NPORE_OUT_NO_EXPANDED)) CU(ctx->d_pack_ops.ensure((size_t)ctx->total_ops + 64));
+    if (flags & NPORE_OUT_RLE) CU(ctx->d_pack_rle.ensure(sizeof(uint32_t) * (size_t)(ctx->total_ops + 64)));
+    int rr_cap = 1, rc = cut_sub_batches(ctx, &rr_cap);
+    if (rc != NPORE_OK) return rc;
+    CU(cudaMemsetAsync(ctx->d_counter.p, 0, 16, ctx->stream));     // [0] forward-kernel error flag  [1] overflow records  [2] saturated chunks
+    if (wide) CU(ctx->d_ovf.ensure(sizeof(uint4) * 65536));
+    CU(cudaEventRecord(ctx->ev[EV_PLAN_BEGIN], ctx->stream));
+    int max_ops = 1;
+    for (const ItemDesc &I : ctx->items) max_ops = std::max(max_ops, I.total_ops);
+    const int parts = std::min(FIN_MAX_PARTS, (max_ops + 32767) / 32768);     // slices per item for the per-item kernels
+    if (n) {
+        CU(ctx->d_part_cnt.ensure(sizeof(int32_t) * (size_t)n * parts));
+        PlanArgs pa{};
+        pa.items = ctx->d_items.as<ItemDesc>(); pa.n_items = n; pa.rle = ctx->d_rle.as<uint32_t>(); pa.grp_off = ctx->d_grp.as<int32_t>();
+        pa.bits = ctx->d_bits.as<uint32_t>(); pa.cum = ctx->d_cum.as<uint32_t>(); pa.chunks = ctx->d_chunks.as<ChunkDesc>();
+        pa.max_b_rows = ctx->P.max_b_rows; pa.parts = parts; pa.part_cnt = ctx->d_part_cnt.as<int32_t>();
+        const dim3 grid_np(n, parts);
+        plan_groups_kernel<<<n, PLAN_THREADS, 0, ctx->stream>>>(pa);
+        plan_bits_kernel<<<grid_np, PLAN_THREADS, 0, ctx->stream>>>(pa);
+        plan_cum_kernel<<<grid_np, PLAN_THREADS, 0, ctx->stream>>>(pa);
+        plan_chunks_kernel<<<grid_np, PLAN_THREADS, 0, ctx->stream>>>(pa);
+        CU(cudaGetLastError()); S.launches += 4;
+    }
+    CU(cudaEventRecord(ctx->ev[EV_PLAN_END], ctx->stream));
+    for (size_t si = 0; si < ctx->subs.size(); si++)
+        if ((rc = run_sub_batch(ctx, si, wide, rr_cap, inflight)) != NPORE_OK) return rc;
+    if ((rc = launch_finish(ctx, flags, parts, max_ops)) != NPORE_OK) return rc;
+    CU(cudaStreamSynchronize(ctx->stream));
+    const int *counters = SmallBlock(ctx->h_small.p, n, ctx->n_chunks).counters;
+    if (counters[0]) return fail(ctx, NPORE_ERR_CUDA, "forward kernel: shared-memory window smaller than the history rings");
+    *n_sat = counters[2];
+    float ms[3] = {0, 0, 0}, t;                       // annotate, forward, traceback
+    for (size_t si = 0; si < ctx->subs.size(); si++)
+        for (int k = 0; k < 3; k++) { cudaEventElapsedTime(&t, ctx->sub_ev[4 * si + k], ctx->sub_ev[4 * si + k + 1]); ms[k] += t; }
+    cudaEventElapsedTime(&S.ms_plan, ctx->ev[EV_PLAN_BEGIN], ctx->ev[EV_PLAN_END]);
+    cudaEventElapsedTime(&S.ms_finish, ctx->ev[EV_FINISH_BEGIN], ctx->ev[EV_FINISH_END]);
+    cudaEventElapsedTime(&S.ms_kernels_total, ctx->ev[EV_PLAN_BEGIN], ctx->ev[EV_FINISH_END]);
+    S.ms_annotate = ms[0]; S.ms_forward = ms[1]; S.ms_traceback = ms[2];
+    S.n_sub_batches = (int)ctx->subs.size();
+    ctx->ran = true;
+    return NPORE_OK;
 }
 
 }  // namespace
@@ -270,7 +560,6 @@ int npore_ctx_create(npore_ctx **out, int device, const float *sub_scores, const
     ctx->P.r = r; ctx->P.W = 2 * r + 1; ctx->P.max_n = max_n; ctx->P.max_l = max_l; ctx->P.max_b_rows = max_b_rows;
     ctx->P.np_dim = np_dim; ctx->P.np_clamp = max_l - 1; ctx->P.np_rows = max_n * (max_l + 1);
     ctx->P.gap_open = indel_start; ctx->P.gap_ext = indel_extend;
-    ctx->np_n = np_n;
     const int W = 2 * r + 1;
     ctx->cpl = W <= 32 ? 1 : W <= 64 ? 2 : W <= 128 ? 4 : 8;
     ctx->tbs = np_tbs(ctx->cpl);
@@ -301,8 +590,8 @@ int npore_ctx_create(npore_ctx **out, int device, const float *sub_scores, const
     cudaMemGetInfo(&fr, &tot);
     if (cudaGetLastError() != cudaSuccess) return bail(NPORE_ERR_CUDA);
     ctx->scratch_budget = (size_t)((double)fr * 0.55);          // divided by the device's live contexts at run time
-    if (device < 64) g_ctx_on_device[device]++;
-    ctx->counted = true;
+    if (device < 64) { ctx->on_device = &g_ctx_on_device[device]; ctx->par_inflight = &g_par_inflight[device]; }
+    if (ctx->on_device) (*ctx->on_device)++;
     if (const char *s = getenv("NPORE_SCRATCH_MB")) { ctx->scratch_budget = (size_t)atoll(s) << 20; ctx->budget_fixed = true; }
     if (const char *s = getenv("NPORE_RR_SLICE")) ctx->rr_slice = std::max(8, atoi(s));
     *out = ctx;
@@ -313,19 +602,11 @@ void npore_ctx_destroy(npore_ctx *ctx)
 {
     if (!ctx) return;
     cudaSetDevice(ctx->device);
-    if (ctx->counted && ctx->device < 64) g_ctx_on_device[ctx->device]--;
-    DevBuf *bufs[] = {&ctx->d_sub, &ctx->d_np, &ctx->d_items, &ctx->d_ref, &ctx->d_seq, &ctx->d_rle, &ctx->d_grp, &ctx->d_bits,
-                      &ctx->d_cum, &ctx->d_chunks, &ctx->d_chunk_out, &ctx->d_scratch_ops, &ctx->d_ops, &ctx->d_item_len,
-                      &ctx->d_item_status, &ctx->d_rleA, &ctx->d_rleB, &ctx->d_rle_len, &ctx->d_rle_which, &ctx->d_ops_off, &ctx->d_rle_off, &ctx->d_pack_ops, &ctx->d_pack_rle, &ctx->d_order, &ctx->d_slots, &ctx->d_counter,
-                      &ctx->d_nib, &ctx->d_nib_start, &ctx->d_ovf, &ctx->d_colrec, &ctx->d_relaid, &ctx->d_rowrec, &ctx->d_raw_ref, &ctx->d_raw_seq, &ctx->d_tb, &ctx->d_rr_q, &ctx->d_rr_ctl, &ctx->d_rr_state};
-    for (auto *b : bufs) b->release();
-    for (auto &b : ctx->d_cm) b.release();
-    ctx->d_chunk_dst.release(); ctx->d_part_cnt.release();
-    ctx->h_small.release();
+    if (ctx->on_device) (*ctx->on_device)--;
     for (auto &e : ctx->ev) if (e) cudaEventDestroy(e);
     for (auto &e : ctx->sub_ev) cudaEventDestroy(e);
     if (ctx->stream && ctx->own_stream) cudaStreamDestroy(ctx->stream);
-    delete ctx;
+    delete ctx;                          // frees the buffers, on the device set above
 }
 
 int npore_set_stream(npore_ctx *ctx, void *cuda_stream)
@@ -382,7 +663,7 @@ int npore_upload(npore_ctx *ctx, const npore_batch *b)
         n_cu += ((int64_t)I.total_ops + I.n_chunks) * ctx->P.W;
         I.status = 0;
     }
-    ctx->n_chunks = nchunks; ctx->total_ops = out_off; ctx->total_words = words;
+    ctx->n_chunks = nchunks; ctx->total_ops = out_off;
     ctx->total_rle = n ? b->cigar_off[n] - b->cigar_off[0] : 0;
 
     // chunk size upper bounds (exact B needs the break shift computed on device) and processing order
@@ -416,23 +697,17 @@ int npore_upload(npore_ctx *ctx, const npore_batch *b)
     }
     CU(ctx->d_rle.ensure(sizeof(uint32_t) * (size_t)(ctx->total_rle + 1)));
     CU(ctx->d_grp.ensure(sizeof(int32_t) * (size_t)(ctx->total_rle + n + 1)));
-    CU(ctx->d_bits.ensure(sizeof(uint32_t) * (size_t)(words + 128)));
-    CU(ctx->d_cum.ensure(sizeof(uint32_t) * (size_t)(words + 128)));
+    for (DevBuf *d : {&ctx->d_bits, &ctx->d_cum}) CU(d->ensure(sizeof(uint32_t) * (size_t)(words + 128)));
     CU(ctx->d_chunks.ensure(sizeof(ChunkDesc) * (size_t)std::max<int64_t>(nchunks, 1)));
     CU(ctx->d_chunk_out.ensure(sizeof(ChunkOut) * (size_t)std::max<int64_t>(nchunks, 1)));
     CU(ctx->d_order.ensure(sizeof(int32_t) * (size_t)std::max<int64_t>(nchunks, 1)));
     CU(ctx->d_slots.ensure(sizeof(ChunkSlot) * (size_t)std::max<int64_t>(nchunks, 1)));
-    CU(ctx->d_scratch_ops.ensure((size_t)out_off + 64));
-    CU(ctx->d_ops.ensure((size_t)out_off + 64));
-    CU(ctx->d_item_len.ensure(sizeof(int32_t) * (size_t)std::max(n, 1)));
-    CU(ctx->d_item_status.ensure(sizeof(int32_t) * (size_t)std::max(n, 1)));
-    CU(ctx->d_rle_len.ensure(sizeof(int32_t) * (size_t)std::max(n, 1)));
-    CU(ctx->d_rle_which.ensure(sizeof(int32_t) * (size_t)std::max(n, 1)));
-    CU(ctx->d_ops_off.ensure(sizeof(int64_t) * (size_t)(n + 1)));
-    CU(ctx->d_rle_off.ensure(sizeof(int64_t) * (size_t)(n + 1)));
+    for (DevBuf *d : {&ctx->d_scratch_ops, &ctx->d_ops}) CU(d->ensure((size_t)out_off + 64));
+    for (DevBuf *d : {&ctx->d_item_len, &ctx->d_item_status, &ctx->d_rle_len, &ctx->d_rle_which}) CU(d->ensure(sizeof(int32_t) * (size_t)std::max(n, 1)));
+    for (DevBuf *d : {&ctx->d_ops_off, &ctx->d_rle_off}) CU(d->ensure(sizeof(int64_t) * (size_t)(n + 1)));
 
     CU(cudaMemsetAsync(ctx->d_bits.p, 0, sizeof(uint32_t) * (size_t)(words + 128), ctx->stream));   // incl. the read-ahead padding
-    CU(cudaEventRecord(ctx->ev[0], ctx->stream));
+    CU(cudaEventRecord(ctx->ev[EV_COPY_BEGIN], ctx->stream));
     if (n) CU(cudaMemcpyAsync(ctx->d_items.p, ctx->items.data(), sizeof(ItemDesc) * n, cudaMemcpyHostToDevice, ctx->stream));
     if (b->ref_total) CU(cudaMemcpyAsync(ctx->d_ref.p, b->ref_codes, (size_t)b->ref_total, cudaMemcpyHostToDevice, ctx->stream));
     if (packed_seq) {
@@ -448,18 +723,16 @@ int npore_upload(npore_ctx *ctx, const npore_batch *b)
     if (ctx->total_rle)
         CU(cudaMemcpyAsync(ctx->d_rle.p, b->cigar_rle + b->cigar_off[0], sizeof(uint32_t) * (size_t)ctx->total_rle, cudaMemcpyHostToDevice, ctx->stream));
     if (nchunks) CU(cudaMemcpyAsync(ctx->d_order.p, ctx->order.data(), sizeof(int32_t) * (size_t)nchunks, cudaMemcpyHostToDevice, ctx->stream));
-    CU(cudaEventRecord(ctx->ev[1], ctx->stream));
+    CU(cudaEventRecord(ctx->ev[EV_COPY_END], ctx->stream));
     CU(cudaStreamSynchronize(ctx->stream));
     npore_stats &S = ctx->stats;
     S = npore_stats{};
     S.n_items = n; S.n_chunks = nchunks; S.n_cu = n_cu; S.sm_count = ctx->sm_count;
     S.h2d_bytes = (int64_t)sizeof(ItemDesc) * n + b->ref_total + (packed_seq ? b->seq_nib_bytes + 8 * (int64_t)n : b->seq_total) + 4 * ctx->total_rle + 4 * nchunks;
-    cudaEventElapsedTime(&S.ms_h2d, ctx->ev[0], ctx->ev[1]);
+    cudaEventElapsedTime(&S.ms_h2d, ctx->ev[EV_COPY_BEGIN], ctx->ev[EV_COPY_END]);
     ctx->uploaded = true;
     return NPORE_OK;
 }
-
-static int run_pass(npore_ctx *ctx, uint32_t flags, bool wide, int *n_sat);
 
 int npore_run(npore_ctx *ctx, uint32_t flags)
 {
@@ -472,277 +745,9 @@ int npore_run(npore_ctx *ctx, uint32_t flags)
     // limit): the batch is redone with the WIDE forward kernels, which carry runs unsaturated and keep the true run of such records
     // in an overflow list.  Costs a second pass for that batch only; status 8 remains only if that list overflows (65,536 records).
     if (rc == NPORE_OK && n_sat > 0) rc = run_pass(ctx, flags, true, &n_sat);
+    // drain what an error left queued: the context stays reusable, and npore_download reports NPORE_ERR_STATE (ran is false)
+    if (rc != NPORE_OK) { cudaStreamSynchronize(ctx->stream); cudaGetLastError(); }
     return rc;
-}
-
-static int run_pass(npore_ctx *ctx, uint32_t flags, bool wide, int *n_sat)
-{
-    CU(cudaSetDevice(ctx->device));
-    ctx->ran = false;
-    // an error half-way leaves work queued on the stream and events unrecorded: drain it, so that the context is reusable
-    // (upload again or run again) and npore_download reports NPORE_ERR_STATE instead of reading half-written results
-    struct RunGuard {
-        npore_ctx *c; bool ok = false;
-        ~RunGuard() { if (!ok) { cudaStreamSynchronize(c->stream); cudaGetLastError(); c->ran = false; } }
-    } guard{ctx};
-    // this pass's entry in g_par_inflight: set per sub-batch, withdrawn when the pass has synchronised (or failed)
-    struct InFlight {
-        std::atomic<long long> *g; long long mine = 0;
-        long long set(long long par) { const long long before = g ? g->fetch_add(par - mine) : mine; const long long o = before - mine; mine = par; return o > 0 ? o : 0; }
-        ~InFlight() { if (g && mine) g->fetch_sub(mine); }
-    } inflight{ctx->device < 64 ? &g_par_inflight[ctx->device] : nullptr};
-    const int n = (int)ctx->items.size();
-    const int64_t nchunks = ctx->n_chunks;
-    const int NC = 32 * ctx->cpl;
-    npore_stats &S = ctx->stats;
-    S.launches = 0; S.tb_bytes = 0;
-    ctx->run_flags = flags;
-    const bool need_rle = (flags & (NPORE_OUT_RLE | NPORE_OUT_STANDARDIZE)) != 0;
-    const bool want_ops = !(flags & NPORE_OUT_NO_EXPANDED), want_rle = (flags & NPORE_OUT_RLE) != 0;
-    if (need_rle) {
-        CU(ctx->d_rleA.ensure(sizeof(uint32_t) * (size_t)(ctx->total_ops + 64)));
-        CU(ctx->d_rleB.ensure(sizeof(uint32_t) * (size_t)(ctx->total_ops + 64)));
-    }
-    if (want_ops) CU(ctx->d_pack_ops.ensure((size_t)ctx->total_ops + 64));
-    if (want_rle) CU(ctx->d_pack_rle.ensure(sizeof(uint32_t) * (size_t)(ctx->total_ops + 64)));
-
-    // ---- sub-batches: greedy over `order` under the scratch budget (sizes from the host-side upper bounds).  The budget is
-    // this context's share of the device (contexts on one device run side by side: PipelinedRealigner); if the scratch still
-    // does not fit (other tenants of the device), the batch is re-cut with half the budget instead of failing.
-    size_t budget = ctx->scratch_budget;
-    if (!ctx->budget_fixed && ctx->device < 64) budget /= (size_t)std::max(1, g_ctx_on_device[ctx->device].load());
-    for (int attempt = 0;; attempt++) {
-        ctx->slots.assign(nchunks, ChunkSlot{});
-        ctx->subs.clear();
-        size_t max_col = 0, max_row = 0, max_tb = 0;
-        const size_t per_entry = 32 + 8 + 8 + 4 + 8;   // colrec, relaid, raw_ref, rowrec, raw_seq
-        size_t col = 0, row = 0, tb = 0; int first = 0;
-        for (int64_t k = 0; k < nchunks; k++) {
-            const int bm = ctx->chunk_bmax[ctx->order[k]];
-            const size_t ent = (size_t)((bm + NC + 128 + 31) & ~31);
-            const size_t need = (col + ent) * per_entry + (tb + bm) * (size_t)(64 * ctx->tbs);
-            if (k > first && need > budget) {
-                ctx->subs.push_back({first, (int)(k - first)});
-                max_col = std::max(max_col, col); max_row = std::max(max_row, row); max_tb = std::max(max_tb, tb);
-                col = row = tb = 0; first = (int)k;
-            }
-            ChunkSlot &sl = ctx->slots[k];
-            sl.col_off = (int64_t)col; sl.row_off = (int64_t)row; sl.tb_off = (int64_t)tb;
-            sl.col_cap = sl.row_cap = (int32_t)ent;
-            col += ent; row += ent; tb += bm;
-        }
-        if (nchunks > first) {
-            ctx->subs.push_back({first, (int)(nchunks - first)});
-            max_col = std::max(max_col, col); max_row = std::max(max_row, row); max_tb = std::max(max_tb, tb);
-        }
-        cudaError_t e = ctx->d_colrec.ensure(max_col * 32 + 64);
-        if (e == cudaSuccess) e = ctx->d_relaid.ensure(max_col * 8 + 64);
-        if (e == cudaSuccess) e = ctx->d_raw_ref.ensure(max_col * 8 + 64);
-        if (e == cudaSuccess) e = ctx->d_rowrec.ensure(max_row * 4 + 64);
-        if (e == cudaSuccess) e = ctx->d_raw_seq.ensure(max_row * 8 + 64);
-        if (e == cudaSuccess) e = ctx->d_tb.ensure(max_tb * (size_t)(64 * ctx->tbs) + 256);
-        if (e == cudaSuccess) break;
-        cudaGetLastError();
-        if (e != cudaErrorMemoryAllocation || attempt >= 4 || ctx->subs.size() >= (size_t)std::max<int64_t>(nchunks, 1))
-            return fail(ctx, e == cudaErrorMemoryAllocation ? NPORE_ERR_OOM : NPORE_ERR_CUDA, "scratch allocation", e);
-        ctx->d_tb.release(); ctx->d_colrec.release();          // give back what the failed attempt may have grabbed
-        budget /= 2;
-    }
-    int max_sub = 1;
-    for (const SubBatch &sb : ctx->subs) max_sub = std::max(max_sub, sb.count);
-    int rr_cap = 1;
-    while (rr_cap < 2 * max_sub + 16384) rr_cap <<= 1;
-    CU(ctx->d_rr_q.ensure(sizeof(int) * (size_t)rr_cap));
-    CU(ctx->d_rr_ctl.ensure(64));
-    CU(ctx->d_rr_state.ensure(sizeof(uint32_t) * fwd_rr_state_words(ctx->cpl) * (size_t)max_sub));
-    if (nchunks) CU(cudaMemcpyAsync(ctx->d_slots.p, ctx->slots.data(), sizeof(ChunkSlot) * (size_t)nchunks, cudaMemcpyHostToDevice, ctx->stream));
-
-    CU(cudaMemsetAsync(ctx->d_counter.p, 0, 16, ctx->stream));     // [0] forward-kernel error flag  [1] overflow records  [2] saturated chunks
-    if (wide) CU(ctx->d_ovf.ensure(sizeof(uint4) * 65536));
-    CU(cudaEventRecord(ctx->ev[2], ctx->stream));
-    // ---- plan
-    int max_ops = 1;
-    for (const ItemDesc &I : ctx->items) max_ops = std::max(max_ops, I.total_ops);
-    const int parts = std::min(FIN_MAX_PARTS, (max_ops + 32767) / 32768);     // slices per item for the per-item kernels
-    if (n) {
-        CU(ctx->d_part_cnt.ensure(sizeof(int32_t) * (size_t)n * parts));
-        PlanArgs pa{};
-        pa.items = ctx->d_items.as<ItemDesc>(); pa.n_items = n; pa.rle = ctx->d_rle.as<uint32_t>(); pa.grp_off = ctx->d_grp.as<int32_t>();
-        pa.bits = ctx->d_bits.as<uint32_t>(); pa.cum = ctx->d_cum.as<uint32_t>(); pa.chunks = ctx->d_chunks.as<ChunkDesc>();
-        pa.max_b_rows = ctx->P.max_b_rows; pa.parts = parts; pa.part_cnt = ctx->d_part_cnt.as<int32_t>();
-        const dim3 grid_np(n, parts);
-        plan_groups_kernel<<<n, PLAN_THREADS, 0, ctx->stream>>>(pa);
-        plan_bits_kernel<<<grid_np, PLAN_THREADS, 0, ctx->stream>>>(pa);
-        plan_cum_kernel<<<grid_np, PLAN_THREADS, 0, ctx->stream>>>(pa);
-        plan_chunks_kernel<<<grid_np, PLAN_THREADS, 0, ctx->stream>>>(pa);
-        CU(cudaGetLastError()); S.launches += 4;
-    }
-    CU(cudaEventRecord(ctx->ev[3], ctx->stream));
-    float ms_ann = 0, ms_fwd = 0, ms_tb = 0;
-    while (ctx->sub_ev.size() < 4 * ctx->subs.size()) {
-        cudaEvent_t e; CU(cudaEventCreate(&e)); ctx->sub_ev.push_back(e);
-    }
-    for (size_t si = 0; si < ctx->subs.size(); si++) {
-        const SubBatch &sb = ctx->subs[si];
-        cudaEvent_t e0 = ctx->sub_ev[4 * si], e1 = ctx->sub_ev[4 * si + 1], e2 = ctx->sub_ev[4 * si + 2], e3 = ctx->sub_ev[4 * si + 3];
-        AnnotateArgs aa{};
-        aa.chunks = ctx->d_chunks.as<ChunkDesc>(); aa.slots = ctx->d_slots.as<ChunkSlot>() + sb.first;
-        aa.order = ctx->d_order.as<int32_t>() + sb.first; aa.n = sb.count; aa.items = ctx->d_items.as<ItemDesc>();
-        aa.ref_codes = ctx->d_ref.as<uint8_t>(); aa.seq_codes = ctx->d_seq.as<uint8_t>();
-        aa.raw_ref = ctx->d_raw_ref.as<uint8_t>(); aa.raw_seq = ctx->d_raw_seq.as<uint8_t>();
-        aa.colrec = ctx->d_colrec.as<uint4>(); aa.relaid = ctx->d_relaid.as<uint2>(); aa.rowrec = ctx->d_rowrec.as<uint32_t>();
-        aa.max_n = ctx->P.max_n; aa.max_l = ctx->P.max_l; aa.nc = NC; aa.inf_row = ctx->P.np_rows;
-        int bm = 1;
-        double bsum = 0.0;
-        for (int k = 0; k < sb.count; k++) { const int b = ctx->chunk_bmax[ctx->order[sb.first + k]]; bm = std::max(bm, b); bsum += b; }
-        const long long par = (long long)(bsum / bm) + 1;
-        const long long others = inflight.set(par);                  // the other contexts' launches on this device
-        const int team = forward_team(ctx, ctx->cpl, sb.count, (double)par, (double)others);      // warps per chunk of this sub-batch's forward launch
-        aa.cpl = ctx->cpl / team;
-        CU(cudaEventRecord(e0, ctx->stream));
-        {   // equality words of all periods in dynamic shared memory: 6 planes of (longest slice / 32 + 2) words
-            aa.e6_stride = (bm + 1 + 31) / 32 + 2;
-            const size_t dyn = (size_t)NP_MAXN * aa.e6_stride * sizeof(uint32_t);
-            if (dyn > 48 * 1024) CU(cudaFuncSetAttribute(annotate_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn));
-            annotate_kernel<<<2 * sb.count, ANN_THREADS, dyn, ctx->stream>>>(aa);
-        }
-        CU(cudaGetLastError()); S.launches++;
-        CU(cudaEventRecord(e1, ctx->stream));
-
-        ForwardArgs fa{};
-        fa.chunks = aa.chunks; fa.slots = aa.slots; fa.order = aa.order; fa.n = sb.count;
-        fa.items = aa.items; fa.bits = ctx->d_bits.as<uint32_t>(); fa.err = ctx->d_counter.as<int>();
-        fa.ovf = wide ? ctx->d_ovf.as<uint4>() : nullptr; fa.ovf_cap = 65536; fa.ovf_cnt = ctx->d_counter.as<int>() + 1;
-        fa.ref_codes = aa.ref_codes; fa.seq_codes = aa.seq_codes; fa.colrec = aa.colrec; fa.relaid = aa.relaid; fa.rowrec = aa.rowrec;
-        fa.tb = ctx->d_tb.as<uint16_t>(); fa.tab = ctx->d_np.as<float>(); fa.sub_tab = ctx->d_sub.as<float>();
-        fa.out = ctx->d_chunk_out.as<ChunkOut>();
-        fa.P = ctx->P;
-        fa.rr_q = ctx->d_rr_q.as<int>(); fa.rr_mask = rr_cap - 1; fa.rr_ctl = ctx->d_rr_ctl.as<int>();
-        fa.rr_state = ctx->d_rr_state.as<uint32_t>(); fa.rr_slice = ctx->rr_slice;
-        CU(cudaMemsetAsync(ctx->d_rr_state.p, 0, sizeof(uint32_t) * fwd_rr_state_words(ctx->cpl) * (size_t)sb.count, ctx->stream));
-        rr_init_kernel<<<64, 256, 0, ctx->stream>>>(fa.rr_q, rr_cap, sb.count, fa.rr_ctl);
-        CU(cudaGetLastError()); S.launches++;
-        int rc = NPORE_OK;
-        switch ((ctx->cpl * 10 + team) * (wide ? -1 : 1)) {
-        case 11: rc = launch_forward<1, 1, false>(ctx, fa, sb.count); break;
-        case 21: rc = launch_forward<2, 1, false>(ctx, fa, sb.count); break;
-        case 22: rc = launch_forward<1, 2, false>(ctx, fa, sb.count); break;
-        case 41: rc = launch_forward<4, 1, false>(ctx, fa, sb.count); break;
-        case 42: rc = launch_forward<2, 2, false>(ctx, fa, sb.count); break;
-        case 81: rc = launch_forward<8, 1, false>(ctx, fa, sb.count); break;
-        case 82: rc = launch_forward<4, 2, false>(ctx, fa, sb.count); break;
-        case 84: rc = launch_forward<2, 4, false>(ctx, fa, sb.count); break;
-        // the fallback for a batch in which a traceback met a saturated n-polymer run (forward.cuh: WIDE)
-        case -11: rc = launch_forward<1, 1, true>(ctx, fa, sb.count); break;
-        case -21: rc = launch_forward<2, 1, true>(ctx, fa, sb.count); break;
-        case -22: rc = launch_forward<1, 2, true>(ctx, fa, sb.count); break;
-        case -41: rc = launch_forward<4, 1, true>(ctx, fa, sb.count); break;
-        case -42: rc = launch_forward<2, 2, true>(ctx, fa, sb.count); break;
-        case -82: rc = launch_forward<4, 2, true>(ctx, fa, sb.count); break;
-        default: rc = launch_forward<2, 4, true>(ctx, fa, sb.count); break;      // (-84, and -81: a team form carries W > 128)
-        }
-        if (rc != NPORE_OK) return rc;
-        S.launches++;
-        CU(cudaEventRecord(e2, ctx->stream));
-
-        TracebackArgs ta{};
-        ta.chunks = aa.chunks; ta.slots = aa.slots; ta.order = aa.order; ta.n = sb.count; ta.items = aa.items;
-        ta.bits = fa.bits; ta.cum = ctx->d_cum.as<uint32_t>(); ta.ref_codes = aa.ref_codes; ta.seq_codes = aa.seq_codes;
-        ta.tb = fa.tb; ta.ops = ctx->d_scratch_ops.as<uint8_t>(); ta.out = fa.out;
-        ta.r = ctx->P.r; ta.W = ctx->P.W; ta.cpl = ctx->cpl; ta.tbs = ctx->tbs;
-        ta.ovf = fa.ovf; ta.ovf_cnt = fa.ovf_cnt; ta.ovf_cap = fa.ovf_cap; ta.n_sat = ctx->d_counter.as<int>() + 2;
-        traceback_kernel<<<(sb.count + TB_THREADS / 32 - 1) / (TB_THREADS / 32), TB_THREADS, 0, ctx->stream>>>(ta);
-        CU(cudaGetLastError()); S.launches++;
-        CU(cudaEventRecord(e3, ctx->stream));
-        for (int k = 0; k < sb.count; k++) S.tb_bytes += (int64_t)ctx->chunk_bmax[ctx->order[sb.first + k]] * 64 * ctx->tbs;
-    }
-    // ---- finish
-    cudaEvent_t e0 = ctx->ev[4], e1 = ctx->ev[5];
-    CU(cudaEventRecord(e0, ctx->stream));
-    const size_t small_bytes = (size_t)n * 12 + (size_t)ctx->n_chunks * sizeof(ChunkOut) + 64;      // + three counters in the last 16 bytes
-    CU(ctx->h_small.ensure(small_bytes));
-    if (n) {
-        FinishArgs fa{};
-        fa.items = ctx->d_items.as<ItemDesc>(); fa.n_items = n; fa.chunk_out = ctx->d_chunk_out.as<ChunkOut>();
-        fa.scratch = ctx->d_scratch_ops.as<uint8_t>(); fa.ops = ctx->d_ops.as<uint8_t>();
-        fa.item_len = ctx->d_item_len.as<int32_t>(); fa.item_status = ctx->d_item_status.as<int32_t>();
-        fa.ref_codes = ctx->d_ref.as<uint8_t>(); fa.seq_codes = ctx->d_seq.as<uint8_t>();
-        fa.rleA = ctx->d_rleA.as<uint32_t>(); fa.rleB = ctx->d_rleB.as<uint32_t>();
-        fa.rle_len = ctx->d_rle_len.as<int32_t>(); fa.rle_which = ctx->d_rle_which.as<int32_t>();
-        fa.to_m = (flags & NPORE_OUT_STANDARDIZE) ? 1 : 0;
-        fa.ops_off = ctx->d_ops_off.as<int64_t>(); fa.rle_off = ctx->d_rle_off.as<int64_t>();
-        fa.pack_ops = ctx->d_pack_ops.as<uint8_t>(); fa.pack_rle = ctx->d_pack_rle.as<uint32_t>();
-        CU(ctx->d_chunk_dst.ensure(sizeof(int32_t) * (size_t)std::max<int64_t>(ctx->n_chunks, 1)));
-        CU(ctx->d_part_cnt.ensure(sizeof(int32_t) * (size_t)n * parts));
-        fa.chunks = ctx->d_chunks.as<ChunkDesc>(); fa.n_chunks = (int)ctx->n_chunks;
-        fa.chunk_dst = ctx->d_chunk_dst.as<int32_t>(); fa.parts = parts; fa.part_cnt = ctx->d_part_cnt.as<int32_t>();
-        const dim3 grid_np(n, parts);
-        item_len_kernel<<<n, FIN_THREADS, 0, ctx->stream>>>(fa);
-        CU(cudaGetLastError()); S.launches++;
-        if (ctx->n_chunks) {
-            gather_kernel<<<(unsigned)ctx->n_chunks, FIN_THREADS, 0, ctx->stream>>>(fa);
-            CU(cudaGetLastError()); S.launches++;
-        }
-        if (need_rle) {
-            if (parts > 1) { rle_count_kernel<<<grid_np, FIN_WIDE, 0, ctx->stream>>>(fa); S.launches++; }
-            rle_start_kernel<<<grid_np, FIN_WIDE, 0, ctx->stream>>>(fa);
-            rle_word_kernel<<<grid_np, FIN_WIDE, 0, ctx->stream>>>(fa);
-            CU(cudaGetLastError()); S.launches += 2;
-        } else CU(cudaMemsetAsync(ctx->d_rle_len.p, 0, sizeof(int32_t) * (size_t)n, ctx->stream));
-        if (flags & NPORE_OUT_STANDARDIZE) {
-            // items with many run-length groups (haplotypes) get a whole CTA each; NPORE_STD_LONG_MIN overrides the split (tests)
-            int long_min = 4096;
-            if (const char *e = getenv("NPORE_STD_LONG_MIN")) long_min = std::max(1, atoi(e));
-            const bool any_long = max_ops >= long_min;              // an item cannot have more groups than ops
-            // the long-item kernel goes first and marks its items (rle_which = 1); the per-warp kernel takes what is left.
-            // (Both look at the group count BEFORE standardisation: the sweeps change it.)
-            if (any_long) {
-                standardize_long_kernel<<<n, FIN_WIDE, 0, ctx->stream>>>(fa, long_min);
-                CU(cudaGetLastError()); S.launches++;
-            }
-            standardize_kernel<<<(n + FIN_THREADS / 32 - 1) / (FIN_THREADS / 32), FIN_THREADS, 0, ctx->stream>>>(fa);
-            CU(cudaGetLastError()); S.launches++;
-            if (want_ops) {
-                if (parts > 1) { expand_count_kernel<<<grid_np, FIN_WIDE, 0, ctx->stream>>>(fa); S.launches++; }
-                expand_fill_kernel<<<grid_np, FIN_WIDE, 0, ctx->stream>>>(fa);
-                CU(cudaGetLastError()); S.launches++;
-            }
-        }
-        scan_kernel<<<1, 1024, 0, ctx->stream>>>(fa);
-        CU(cudaGetLastError()); S.launches++;
-        if (want_ops || want_rle) {
-            pack_kernel<<<grid_np, FIN_WIDE, 0, ctx->stream>>>(fa, want_ops ? 1 : 0, want_rle ? 1 : 0);
-            CU(cudaGetLastError()); S.launches++;
-        }
-        // per-item sizes / status / chunk results travel with the run so that download() knows exact sizes
-        int32_t *h_len = (int32_t *)ctx->h_small.p, *h_status = h_len + n, *h_rlen = h_status + n;
-        ChunkOut *h_co = (ChunkOut *)(h_rlen + n + (n & 1));
-        CU(cudaMemcpyAsync(h_len, ctx->d_item_len.p, 4 * (size_t)n, cudaMemcpyDeviceToHost, ctx->stream));
-        CU(cudaMemcpyAsync(h_status, ctx->d_item_status.p, 4 * (size_t)n, cudaMemcpyDeviceToHost, ctx->stream));
-        CU(cudaMemcpyAsync(h_rlen, ctx->d_rle_len.p, 4 * (size_t)n, cudaMemcpyDeviceToHost, ctx->stream));
-        if (ctx->n_chunks) CU(cudaMemcpyAsync(h_co, ctx->d_chunk_out.p, sizeof(ChunkOut) * (size_t)ctx->n_chunks, cudaMemcpyDeviceToHost, ctx->stream));
-    }
-    int *h_cnt = reinterpret_cast<int *>(static_cast<char *>(ctx->h_small.p) + small_bytes - 16);
-    h_cnt[0] = h_cnt[1] = h_cnt[2] = 0;
-    CU(cudaMemcpyAsync(h_cnt, ctx->d_counter.p, 12, cudaMemcpyDeviceToHost, ctx->stream));
-    CU(cudaEventRecord(e1, ctx->stream));
-    CU(cudaStreamSynchronize(ctx->stream));
-    if (h_cnt[0]) return fail(ctx, NPORE_ERR_CUDA, "forward kernel: shared-memory window smaller than the history rings");
-    *n_sat = h_cnt[2];
-    for (size_t si = 0; si < ctx->subs.size(); si++) {
-        float t;
-        cudaEventElapsedTime(&t, ctx->sub_ev[4 * si], ctx->sub_ev[4 * si + 1]); ms_ann += t;
-        cudaEventElapsedTime(&t, ctx->sub_ev[4 * si + 1], ctx->sub_ev[4 * si + 2]); ms_fwd += t;
-        cudaEventElapsedTime(&t, ctx->sub_ev[4 * si + 2], ctx->sub_ev[4 * si + 3]); ms_tb += t;
-    }
-    cudaEventElapsedTime(&S.ms_plan, ctx->ev[2], ctx->ev[3]);
-    cudaEventElapsedTime(&S.ms_finish, e0, e1);
-    cudaEventElapsedTime(&S.ms_kernels_total, ctx->ev[2], e1);
-    S.ms_annotate = ms_ann; S.ms_forward = ms_fwd; S.ms_traceback = ms_tb;
-    S.n_sub_batches = (int)ctx->subs.size();
-    ctx->ran = true;
-    guard.ok = true;
-    return NPORE_OK;
 }
 
 int npore_download(npore_ctx *ctx, npore_result *res)
@@ -755,19 +760,18 @@ int npore_download(npore_ctx *ctx, npore_result *res)
     const bool want_ops = !(flags & NPORE_OUT_NO_EXPANDED) && res->ops && res->ops_off;
     const bool want_rle = (flags & NPORE_OUT_RLE) && res->rle && res->rle_off;
     npore_stats &S = ctx->stats;
-    const int32_t *h_len = (const int32_t *)ctx->h_small.p, *h_status = h_len + n, *h_rlen = h_status + n;
-    const ChunkOut *h_co = (const ChunkOut *)(h_rlen + n + (n & 1));
+    const SmallBlock hs(ctx->h_small.p, n, ctx->n_chunks);
     // offsets first (sizes arrived with npore_run), then one exact-size copy per output straight into the caller's buffers
     int64_t o = 0, ro = 0, so = 0;
     for (int i = 0; i < n; i++) {
-        if (res->status) res->status[i] = h_status[i];
-        if (want_ops) { res->ops_off[i] = o; o += h_len[i]; }
-        if (want_rle) { res->rle_off[i] = ro; ro += h_rlen[i]; }
+        if (res->status) res->status[i] = hs.status[i];
+        if (want_ops) { res->ops_off[i] = o; o += hs.len[i]; }
+        if (want_rle) { res->rle_off[i] = ro; ro += hs.rle_len[i]; }
         if (res->chunk_scores && res->score_off) {
             const ItemDesc &I = ctx->items[i];
             res->score_off[i] = so;
             if (so + I.n_chunks > res->score_capacity) return fail(ctx, NPORE_ERR_CAPACITY, "score buffer too small");
-            for (int k = 0; k < I.n_chunks; k++) res->chunk_scores[so + k] = h_co[I.chunk_first + k].score;
+            for (int k = 0; k < I.n_chunks; k++) res->chunk_scores[so + k] = hs.chunk_out[I.chunk_first + k].score;
             so += I.n_chunks;
         }
     }
@@ -775,12 +779,12 @@ int npore_download(npore_ctx *ctx, npore_result *res)
     if (want_rle) { res->rle_off[n] = ro; if (ro > res->rle_capacity) return fail(ctx, NPORE_ERR_CAPACITY, "rle buffer too small"); }
     if (res->chunk_scores && res->score_off) res->score_off[n] = so;
     S.d2h_bytes = (int64_t)n * 12 + (int64_t)ctx->n_chunks * sizeof(ChunkOut);
-    CU(cudaEventRecord(ctx->ev[0], ctx->stream));
+    CU(cudaEventRecord(ctx->ev[EV_COPY_BEGIN], ctx->stream));
     if (want_ops && o) { CU(cudaMemcpyAsync(res->ops, ctx->d_pack_ops.p, (size_t)o, cudaMemcpyDeviceToHost, ctx->stream)); S.d2h_bytes += o; }
     if (want_rle && ro) { CU(cudaMemcpyAsync(res->rle, ctx->d_pack_rle.p, 4 * (size_t)ro, cudaMemcpyDeviceToHost, ctx->stream)); S.d2h_bytes += 4 * ro; }
-    CU(cudaEventRecord(ctx->ev[1], ctx->stream));
+    CU(cudaEventRecord(ctx->ev[EV_COPY_END], ctx->stream));
     CU(cudaStreamSynchronize(ctx->stream));
-    cudaEventElapsedTime(&S.ms_d2h, ctx->ev[0], ctx->ev[1]);
+    cudaEventElapsedTime(&S.ms_d2h, ctx->ev[EV_COPY_BEGIN], ctx->ev[EV_COPY_END]);
     return NPORE_OK;
 }
 
@@ -803,23 +807,23 @@ int npore_get_np_info_batch(npore_ctx *ctx, int32_t n_seqs, const uint8_t *codes
         if (off[i + 1] < off[i] || off[i + 1] - off[i] > 0x7ffffff0ll) return fail(ctx, NPORE_ERR_BAD_ARG, "bad sequence offsets");
     if (total == 0) return NPORE_OK;
     CU(cudaSetDevice(ctx->device));
-    // staging lives in the context (grow-only, shared with npore_confusion_batch's slots): no cudaMalloc / cudaFree per call
-    DevBuf &d_s = ctx->d_cm[4], &d_off = ctx->d_cm[3], &d_raw = ctx->d_cm[5], &d_out = ctx->d_cm[21], &d_e = ctx->d_cm[6];
+    // staging lives in the context (grow-only, shared with npore_confusion_batch): no cudaMalloc / cudaFree per call
+    auto &d = ctx->pileup;
     const size_t ob = (size_t)total * 2 * ctx->P.max_n * sizeof(int32_t);
     int rc = NPORE_OK;
-    if (d_s.ensure((size_t)total) != cudaSuccess || d_off.ensure(sizeof(int64_t) * (size_t)(n_seqs + 1)) != cudaSuccess ||
-        d_raw.ensure((size_t)total * 8) != cudaSuccess || d_out.ensure(std::max<size_t>(ob, 4)) != cudaSuccess ||
-        d_e.ensure(sizeof(uint32_t) * (size_t)(total / 32 + 2 * (size_t)n_seqs + 8)) != cudaSuccess)
+    if (d.ref_codes.ensure((size_t)total) != cudaSuccess || d.ref_off.ensure(sizeof(int64_t) * (size_t)(n_seqs + 1)) != cudaSuccess ||
+        d.raw.ensure((size_t)total * 8) != cudaSuccess || d.out.ensure(std::max<size_t>(ob, 4)) != cudaSuccess ||
+        d.ebits.ensure(sizeof(uint32_t) * (size_t)(total / 32 + 2 * (size_t)n_seqs + 8)) != cudaSuccess)
         rc = fail(ctx, NPORE_ERR_OOM, "np_info scratch");
     if (rc == NPORE_OK) {
-        cudaError_t e = cudaMemcpyAsync(d_s.p, codes, (size_t)total, cudaMemcpyHostToDevice, ctx->stream);
-        if (e == cudaSuccess) e = cudaMemcpyAsync(d_off.p, off, sizeof(int64_t) * (size_t)(n_seqs + 1), cudaMemcpyHostToDevice, ctx->stream);
+        cudaError_t e = cudaMemcpyAsync(d.ref_codes.p, codes, (size_t)total, cudaMemcpyHostToDevice, ctx->stream);
+        if (e == cudaSuccess) e = cudaMemcpyAsync(d.ref_off.p, off, sizeof(int64_t) * (size_t)(n_seqs + 1), cudaMemcpyHostToDevice, ctx->stream);
         if (e == cudaSuccess) {
-            np_info_kernel<<<n_seqs, ANN_THREADS, 0, ctx->stream>>>(d_s.as<uint8_t>(), d_off.as<int64_t>(), ctx->P.max_n, ctx->P.max_l,
-                                                                    d_raw.as<uint8_t>(), d_out.as<int32_t>(), d_e.as<uint32_t>());
+            np_info_kernel<<<n_seqs, ANN_THREADS, 0, ctx->stream>>>(d.ref_codes.as<uint8_t>(), d.ref_off.as<int64_t>(), ctx->P.max_n, ctx->P.max_l,
+                                                                    d.raw.as<uint8_t>(), d.out.as<int32_t>(), d.ebits.as<uint32_t>());
             e = cudaGetLastError();
         }
-        if (e == cudaSuccess && ob) e = cudaMemcpyAsync(out, d_out.p, ob, cudaMemcpyDeviceToHost, ctx->stream);
+        if (e == cudaSuccess && ob) e = cudaMemcpyAsync(out, d.out.p, ob, cudaMemcpyDeviceToHost, ctx->stream);
         if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
         if (e != cudaSuccess) rc = fail(ctx, NPORE_ERR_CUDA, "np_info", e);
     }
@@ -869,58 +873,54 @@ int npore_confusion_batch(npore_ctx *ctx, const npore_pileup_batch *b, int64_t *
             return fail(ctx, NPORE_ERR_BAD_ARG, "confusion: bad read offsets");
     const int64_t seq_total = n ? b->seq_off[n] : 0, n_words = n ? b->cigar_off[n] : 0;
     CU(cudaSetDevice(ctx->device));
-    DevBuf *d = ctx->d_cm;
-    auto put = [&](int slot, const void *src, size_t bytes) -> cudaError_t {
-        cudaError_t e = d[slot].ensure(std::max<size_t>(bytes, 16));
-        if (e == cudaSuccess && bytes) e = cudaMemcpyAsync(d[slot].p, src, bytes, cudaMemcpyHostToDevice, ctx->stream);
-        return e;
-    };
-    auto zero = [&](int slot, size_t bytes) -> cudaError_t {
-        cudaError_t e = d[slot].ensure(std::max<size_t>(bytes, 16));
-        if (e == cudaSuccess) e = cudaMemsetAsync(d[slot].p, 0, std::max<size_t>(bytes, 16), ctx->stream);
+    auto &d = ctx->pileup;
+    auto put = [&](DevBuf &buf, const void *src, size_t bytes) -> cudaError_t {
+        cudaError_t e = buf.ensure(std::max<size_t>(bytes, 16));
+        if (e == cudaSuccess && bytes) e = cudaMemcpyAsync(buf.p, src, bytes, cudaMemcpyHostToDevice, ctx->stream);
         return e;
     };
     cudaError_t e = cudaSuccess;
     int rc = NPORE_OK;
     const bool have_q = b->qual != nullptr;
 #define CM_TRY(x) do { if (e == cudaSuccess) e = (x); } while (0)
-    CM_TRY(put(0, b->range_start, sizeof(int64_t) * R));
-    CM_TRY(put(1, b->range_end, sizeof(int64_t) * R));
-    CM_TRY(put(2, b->ref_ascii, (size_t)total_ref));
-    CM_TRY(put(3, b->ref_off, sizeof(int64_t) * (R + 1)));
-    CM_TRY(d[4].ensure(std::max<size_t>((size_t)total_ref, 16)));                       // codes
-    CM_TRY(d[5].ensure(std::max<size_t>((size_t)total_ref * 8, 16)));                   // raw np_info
-    CM_TRY(d[6].ensure(sizeof(uint32_t) * (size_t)(total_ref / 32 + 2 * (size_t)R + 8)));   // equality words
-    CM_TRY(put(7, b->read_pos, sizeof(int64_t) * n));
-    CM_TRY(put(8, b->seq_ascii, (size_t)seq_total));
-    if (have_q) CM_TRY(put(9, b->qual, (size_t)seq_total));
-    CM_TRY(put(10, b->seq_off, sizeof(int64_t) * (n + 1)));
-    CM_TRY(put(11, b->cigar_rle, sizeof(uint32_t) * (size_t)n_words));
-    CM_TRY(put(12, b->cigar_off, sizeof(int64_t) * (n + 1)));
-    CM_TRY(d[13].ensure(std::max<size_t>(sizeof(int32_t) * (size_t)n_words, 16)));
-    CM_TRY(d[14].ensure(std::max<size_t>(sizeof(int32_t) * (size_t)n_words, 16)));
-    CM_TRY(d[15].ensure(std::max<size_t>(sizeof(int64_t) * (size_t)n, 16)));
-    CM_TRY(put(16, b->range_reads, sizeof(int32_t) * (size_t)n_list));
-    CM_TRY(put(17, b->range_reads_off, sizeof(int64_t) * (R + 1)));
-    CM_TRY(d[18].ensure(std::max<size_t>(sizeof(int64_t) * (size_t)n_list, 16)));
-    CM_TRY(d[19].ensure(std::max<size_t>(sizeof(int32_t) * (size_t)total_pos, 16)));
-    CM_TRY(put(20, pos_off.data(), sizeof(int64_t) * (R + 1)));
-    CM_TRY(zero(21, sizeof(int32_t) * (size_t)(total_pos + R) + sizeof(unsigned long long) * n_out + 16));
+    CM_TRY(put(d.range_start, b->range_start, sizeof(int64_t) * R));
+    CM_TRY(put(d.range_end, b->range_end, sizeof(int64_t) * R));
+    CM_TRY(put(d.ref_ascii, b->ref_ascii, (size_t)total_ref));
+    CM_TRY(put(d.ref_off, b->ref_off, sizeof(int64_t) * (R + 1)));
+    CM_TRY(d.ref_codes.ensure(std::max<size_t>((size_t)total_ref, 16)));
+    CM_TRY(d.raw.ensure(std::max<size_t>((size_t)total_ref * 8, 16)));
+    CM_TRY(d.ebits.ensure(sizeof(uint32_t) * (size_t)(total_ref / 32 + 2 * (size_t)R + 8)));
+    CM_TRY(put(d.read_pos, b->read_pos, sizeof(int64_t) * n));
+    CM_TRY(put(d.seq, b->seq_ascii, (size_t)seq_total));
+    if (have_q) CM_TRY(put(d.qual, b->qual, (size_t)seq_total));
+    CM_TRY(put(d.seq_off, b->seq_off, sizeof(int64_t) * (n + 1)));
+    CM_TRY(put(d.rle, b->cigar_rle, sizeof(uint32_t) * (size_t)n_words));
+    CM_TRY(put(d.cig_off, b->cigar_off, sizeof(int64_t) * (n + 1)));
+    for (DevBuf *g : {&d.g_roff, &d.g_qoff}) CM_TRY(g->ensure(std::max<size_t>(sizeof(int32_t) * (size_t)n_words, 16)));
+    CM_TRY(d.read_end.ensure(std::max<size_t>(sizeof(int64_t) * (size_t)n, 16)));
+    CM_TRY(put(d.range_reads, b->range_reads, sizeof(int32_t) * (size_t)n_list));
+    CM_TRY(put(d.range_reads_off, b->range_reads_off, sizeof(int64_t) * (R + 1)));
+    CM_TRY(d.list_maxend.ensure(std::max<size_t>(sizeof(int64_t) * (size_t)n_list, 16)));
+    CM_TRY(d.line_of.ensure(std::max<size_t>(sizeof(int32_t) * (size_t)total_pos, 16)));
+    CM_TRY(put(d.pos_off, pos_off.data(), sizeof(int64_t) * (R + 1)));
+    const size_t out_bytes = sizeof(int32_t) * (size_t)(total_pos + R) + sizeof(unsigned long long) * n_out + 16;
+    CM_TRY(d.out.ensure(out_bytes));
+    CM_TRY(cudaMemsetAsync(d.out.p, 0, out_bytes, ctx->stream));
     if (e != cudaSuccess) rc = fail(ctx, e == cudaErrorMemoryAllocation ? NPORE_ERR_OOM : NPORE_ERR_CUDA, "confusion staging", e);
     std::vector<unsigned long long> h_out(n_out + 2);
     if (rc == NPORE_OK) {
         ConfusionArgs a;
         a.n_ranges = R; a.n_reads = n;
-        a.range_start = d[0].as<int64_t>(); a.range_end = d[1].as<int64_t>();
-        a.ref_ascii = d[2].as<uint8_t>(); a.ref_off = d[3].as<int64_t>(); a.ref_codes = d[4].as<uint8_t>();
-        a.raw = d[5].as<uint8_t>(); a.ebits = d[6].as<uint32_t>();
-        a.read_pos = d[7].as<int64_t>(); a.seq = d[8].as<uint8_t>(); a.qual = have_q ? d[9].as<uint8_t>() : nullptr;
-        a.seq_off = d[10].as<int64_t>(); a.rle = d[11].as<uint32_t>(); a.cig_off = d[12].as<int64_t>();
-        a.g_roff = d[13].as<int32_t>(); a.g_qoff = d[14].as<int32_t>(); a.read_end = d[15].as<int64_t>();
-        a.range_reads = d[16].as<int32_t>(); a.range_reads_off = d[17].as<int64_t>(); a.list_maxend = d[18].as<int64_t>();
-        a.line_of = d[19].as<int32_t>(); a.pos_off = d[20].as<int64_t>();
+        a.range_start = d.range_start.as<int64_t>(); a.range_end = d.range_end.as<int64_t>();
+        a.ref_ascii = d.ref_ascii.as<uint8_t>(); a.ref_off = d.ref_off.as<int64_t>(); a.ref_codes = d.ref_codes.as<uint8_t>();
+        a.raw = d.raw.as<uint8_t>(); a.ebits = d.ebits.as<uint32_t>();
+        a.read_pos = d.read_pos.as<int64_t>(); a.seq = d.seq.as<uint8_t>(); a.qual = have_q ? d.qual.as<uint8_t>() : nullptr;
+        a.seq_off = d.seq_off.as<int64_t>(); a.rle = d.rle.as<uint32_t>(); a.cig_off = d.cig_off.as<int64_t>();
+        a.g_roff = d.g_roff.as<int32_t>(); a.g_qoff = d.g_qoff.as<int32_t>(); a.read_end = d.read_end.as<int64_t>();
+        a.range_reads = d.range_reads.as<int32_t>(); a.range_reads_off = d.range_reads_off.as<int64_t>(); a.list_maxend = d.list_maxend.as<int64_t>();
+        a.line_of = d.line_of.as<int32_t>(); a.pos_off = d.pos_off.as<int64_t>();
         // zeroed block: outputs first (8-byte aligned), then the coverage difference array
-        unsigned long long *o = d[21].as<unsigned long long>();
+        unsigned long long *o = d.out.as<unsigned long long>();
         a.subs = o; a.nps = o + 25; a.inss = a.nps + (size_t)ctx->P.max_n * T * T; a.dels = a.inss + T;
         a.bad = reinterpret_cast<int *>(o + n_out);
         a.diff = reinterpret_cast<int32_t *>(o + n_out + 2);

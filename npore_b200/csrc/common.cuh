@@ -73,3 +73,10 @@ struct AlignParams {
 #define NP_FULL 0xffffffffu
 
 static __host__ __device__ __forceinline__ int np_tbs(int cpl) { return cpl <= 1 ? 1 : cpl <= 2 ? 2 : cpl <= 4 ? 4 : 8; }
+
+// [lo, hi) of slice `part` of n elements cut into `parts` slices of ceil(n / parts) (per-item kernels on a grid (items, parts))
+__device__ __forceinline__ void np_slice(int n, int parts, int part, int &lo, int &hi)
+{
+    const int per = (n + parts - 1) / parts;
+    lo = min(n, part * per); hi = min(n, lo + per);
+}

@@ -60,12 +60,6 @@ __device__ __forceinline__ int fin_block_scan(int v, int *s_w, int &total)
     return pre + x;
 }
 
-__device__ __forceinline__ void fin_slice(int n, int parts, int part, int &lo, int &hi)
-{
-    const int per = (n + parts - 1) / parts;
-    lo = min(n, part * per); hi = min(n, lo + per);
-}
-
 // where each chunk's op string goes inside its item (aln.pyx:742 `full_aln += aln[::-1]`), the item's length and status
 __global__ void __launch_bounds__(FIN_THREADS) item_len_kernel(const FinishArgs a)
 {
@@ -123,7 +117,7 @@ __global__ void __launch_bounds__(FIN_WIDE) rle_count_kernel(const FinishArgs a)
     const int it = blockIdx.x, part = blockIdx.y;
     const uint8_t *c = a.ops + a.items[it].out_off;
     int lo, hi;
-    fin_slice(a.item_len[it], a.parts, part, lo, hi);
+    np_slice(a.item_len[it], a.parts, part, lo, hi);
     int cnt = 0;
     for (int k = lo + threadIdx.x; k < hi; k += FIN_WIDE) cnt += (k == 0) || (op_code(c[k], a.to_m) != op_code(c[k - 1], a.to_m));
     int tot;
@@ -140,7 +134,7 @@ __global__ void __launch_bounds__(FIN_WIDE) rle_start_kernel(const FinishArgs a)
     const uint8_t *c = a.ops + I.out_off;
     uint32_t *startp = a.rleB + I.out_off;
     int lo, hi;
-    fin_slice(a.item_len[it], a.parts, part, lo, hi);
+    np_slice(a.item_len[it], a.parts, part, lo, hi);
     int carry = 0;
     if (a.parts > 1) for (int q = 0; q < part; q++) carry += a.part_cnt[it * a.parts + q];
     for (int base = lo; base < hi; base += FIN_WIDE * 4) {
@@ -174,7 +168,7 @@ __global__ void __launch_bounds__(FIN_WIDE) rle_word_kernel(const FinishArgs a)
     const uint32_t *startp = a.rleB + I.out_off;
     const int n = a.item_len[it], m = a.rle_len[it];
     int lo, hi;
-    fin_slice(m, a.parts, blockIdx.y, lo, hi);
+    np_slice(m, a.parts, blockIdx.y, lo, hi);
     for (int g = lo + threadIdx.x; g < hi; g += FIN_WIDE) {
         const uint32_t st = startp[g], en = (g + 1 < m) ? startp[g + 1] : (uint32_t)n;
         w[g] = ((en - st) << 4) | op_code(c[st], a.to_m);
@@ -449,7 +443,7 @@ __global__ void __launch_bounds__(FIN_WIDE) expand_count_kernel(const FinishArgs
     const int it = blockIdx.x, part = blockIdx.y;
     const uint32_t *w = (a.rle_which[it] ? a.rleB : a.rleA) + a.items[it].out_off;
     int lo, hi;
-    fin_slice(a.rle_len[it], a.parts, part, lo, hi);
+    np_slice(a.rle_len[it], a.parts, part, lo, hi);
     int cnt = 0;
     for (int g = lo + threadIdx.x; g < hi; g += FIN_WIDE) cnt += (int)(w[g] >> 4);
     int tot;
@@ -468,7 +462,7 @@ __global__ void __launch_bounds__(FIN_WIDE) expand_fill_kernel(const FinishArgs 
     const uint32_t *w = (a.rle_which[it] ? a.rleB : a.rleA) + I.out_off;
     uint8_t *c = a.ops + I.out_off;
     int lo, hi;
-    fin_slice(a.rle_len[it], a.parts, part, lo, hi);
+    np_slice(a.rle_len[it], a.parts, part, lo, hi);
     int carry = 0;
     if (a.parts > 1) for (int q = 0; q < part; q++) carry += a.part_cnt[it * a.parts + q];
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
@@ -528,12 +522,12 @@ __global__ void __launch_bounds__(FIN_WIDE) pack_kernel(const FinishArgs a, int 
     int lo, hi;
     if (want_ops) {
         const uint8_t *src = a.ops + I.out_off; uint8_t *dst = a.pack_ops + a.ops_off[it];
-        fin_slice(a.item_len[it], a.parts, blockIdx.y, lo, hi);
+        np_slice(a.item_len[it], a.parts, blockIdx.y, lo, hi);
         for (int t = lo + threadIdx.x; t < hi; t += FIN_WIDE) dst[t] = src[t];
     }
     if (want_rle) {
         const uint32_t *src = (a.rle_which[it] ? a.rleB : a.rleA) + I.out_off; uint32_t *dst = a.pack_rle + a.rle_off[it];
-        fin_slice(a.rle_len[it], a.parts, blockIdx.y, lo, hi);
+        np_slice(a.rle_len[it], a.parts, blockIdx.y, lo, hi);
         for (int t = lo + threadIdx.x; t < hi; t += FIN_WIDE) dst[t] = src[t];
     }
 }

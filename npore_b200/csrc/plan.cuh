@@ -50,12 +50,6 @@ struct PlanArgs {
     int parts; int32_t *part_cnt;        // [n_items * parts] popcount of the part's words
 };
 
-__device__ __forceinline__ void plan_slice(int n, int parts, int part, int &lo, int &hi)
-{
-    const int per = (n + parts - 1) / parts;
-    lo = min(n, part * per); hi = min(n, lo + per);
-}
-
 // phase A: bit offset of every RLE group; consistency with ref_len / seq_len (status 16 and invalid chunks otherwise)
 __global__ void __launch_bounds__(PLAN_THREADS) plan_groups_kernel(const PlanArgs a)
 {
@@ -112,7 +106,7 @@ __global__ void __launch_bounds__(PLAN_THREADS) plan_bits_kernel(const PlanArgs 
     const int P = I.total_ops;
     const int nwords = (P >> 5) + 1;
     int wlo, whi;
-    plan_slice(nwords, a.parts, part, wlo, whi);
+    np_slice(nwords, a.parts, part, wlo, whi);
     int cnt = 0;
     for (int w = wlo + threadIdx.x; w < whi; w += PLAN_THREADS) {
         uint32_t word = 0;
@@ -161,7 +155,7 @@ __global__ void __launch_bounds__(PLAN_THREADS) plan_cum_kernel(const PlanArgs a
     uint32_t *g_cum = a.cum + I.bit_word_off;
     const int nwords = (I.total_ops >> 5) + 1;
     int wlo, whi;
-    plan_slice(nwords, a.parts, part, wlo, whi);
+    np_slice(nwords, a.parts, part, wlo, whi);
     int carry = 0;
     for (int q = 0; q < part; q++) carry += a.part_cnt[it * a.parts + q];
     for (int base = wlo; base < whi; base += PLAN_THREADS) {
@@ -185,7 +179,7 @@ __global__ void __launch_bounds__(PLAN_THREADS) plan_chunks_kernel(const PlanArg
     const int P = I.total_ops;
     const int step = a.max_b_rows - 1;
     int klo, khi;
-    plan_slice(I.n_chunks, a.parts, blockIdx.y, klo, khi);
+    np_slice(I.n_chunks, a.parts, blockIdx.y, klo, khi);
     for (int k = klo + threadIdx.x; k < khi; k += PLAN_THREADS) {
         int brk = k * step, nxt = (k + 1 < I.n_chunks) ? (k + 1) * step : P;
         if (k > 0 && ((g_bits[brk >> 5] >> (brk & 31)) & 1u) && !((g_bits[(brk - 1) >> 5] >> ((brk - 1) & 31)) & 1u)) brk--;

@@ -2,6 +2,7 @@
 against (a) the golden vectors produced by the unmodified reference and (b) the CPU oracle on seeded inputs.
 Bit-exact for CIGARs / op strings / np_info; DP scores compared bit-for-bit too (stricter than the 1e-5 relative
 tolerance north_star allows: the recurrence is fp32 add + compare in the reference's order)."""
+import gc
 import os
 
 import numpy as np
@@ -214,11 +215,8 @@ def test_long_indel_runs(tables, engine_factory):
     _check(engine_factory(), cases, _oracle_all(cases, S, NP))
 
 
-def test_npolymer_runs_beyond_the_record_field(tables, engine_factory):
-    """LEN / SHR runs of thousands of ops (whole copies of an adjacent tract's unit inserted / deleted): the 11-bit RUN field of
-    the traceback record saturates at 2047, the batch is transparently redone with the WIDE kernels (overflow list), and the
-    result is the reference's -- status 0, no partial CIGAR (round 1 reported status 8 here)."""
-    S, NP = tables
+def _long_npolymer_cases():
+    """(ref, seq, expanded CIGAR) items whose realignment has LEN / SHR runs of 2,047 ops or more, and one ordinary item."""
     rng = np.random.default_rng(8)
     a = synth.make_reference(300, rng, 0.0, "CGT"); b = synth.make_reference(300, rng, 0.0, "CGT")
     cases = []
@@ -229,12 +227,77 @@ def test_npolymer_runs_beyond_the_record_field(tables, engine_factory):
         cases.append((ref, a + tract + unit * extra + b, "=" * (len(a) + len(tract)) + "I" * (len(unit) * extra) + "=" * len(b)))
         cases.append((a + tract + unit * extra + b, ref, "=" * (len(a) + len(tract)) + "D" * (len(unit) * extra) + "=" * len(b)))
     cases.append((a + b, a + b, "=" * 600))                       # an ordinary item in the same batch
+    return cases
+
+
+def test_npolymer_runs_beyond_the_record_field(tables, engine_factory):
+    """LEN / SHR runs of thousands of ops (whole copies of an adjacent tract's unit inserted / deleted): the 11-bit RUN field of
+    the traceback record saturates at 2047, the batch is transparently redone with the WIDE kernels (overflow list), and the
+    result is the reference's -- status 0, no partial CIGAR (round 1 reported status 8 here)."""
+    S, NP = tables
+    cases = _long_npolymer_cases()
     want = _oracle_all(cases, S, NP)
     long_runs = [w[0] for w in want if "I" * 2047 in w[0] or "D" * 2047 in w[0]]
     assert len(long_runs) >= 4
     _check(engine_factory(), cases, want)
     small = engine_factory(max_b_rows=1500)                       # several chunks per item: runs cannot span a chunk border
     _check(small, cases, _oracle_all(cases, S, NP, max_b_rows=1500))
+
+
+def _nib_pack(seqs):
+    """Reads in BAM's 4-bit packing (A=1 C=2 G=4 T=8 N=15), each from the high nibble of a byte: (bytes, nibble starts)."""
+    code = np.zeros(256, np.uint8)
+    code[np.frombuffer(b"ACGTN", np.uint8)] = [1, 2, 4, 8, 15]
+    parts, starts, at = [], [], 0
+    for s in seqs:
+        v = code[np.frombuffer(s.encode(), np.uint8)]
+        v = np.append(v, np.zeros(len(v) & 1, np.uint8))
+        parts.append((v[0::2] << 4) | v[1::2])
+        starts.append(2 * at)
+        at += len(v) // 2
+    return np.concatenate(parts), np.array(starts, np.int64)
+
+
+def test_closed_context_returns_its_device_memory(tables):
+    """A closed context frees every buffer it grew: the run scratch and outputs of packed reads with run-length and standardised
+    outputs, the WIDE pass and its overflow list, the np-info and confusion staging.  The device's free memory after the third
+    create / use / close round equals that after the first, which absorbs the driver's one-time allocations (module loads).
+    What this cannot see: the pinned host staging (host memory), and small buffers (counters, run-queue control) whose leak
+    stays inside memory the driver had already reserved; the scratch, output and staging buffers are large enough to show."""
+    import torch
+    from npore_b200 import confusion
+    from npore_b200.engine import NPORE_OUT_RLE, NPORE_OUT_STANDARDIZE, PackedBatch, Realigner, cigars_to_rle_batch
+    S, NP = tables
+    rng = np.random.default_rng(31)
+    ref, tr = synth.make_reference_with_tracts(40_000, rng)
+    reads = synth.make_reads(ref, 24, 3000, rng, synth.call_length_model(NP), tracts=tr)
+    nib, nib_start = _nib_pack([r[7] for r in reads])
+    words, off = cigars_to_rle_batch([r[5] for r in reads])
+    packed = PackedBatch.from_flat_shared_nib(cig.bases_to_int(ref), np.array([r[3] for r in reads], np.int64),
+                                              np.array([r[6] - r[3] for r in reads], np.int32), nib, nib_start,
+                                              np.array([len(r[7]) for r in reads], np.int32), words, off)
+    long_cases = _long_npolymer_cases()
+    contig = synth.make_reference(3000, rng, p_np=0.4)
+    aligned = confusion.AlignedReads([r[:5] for r in synth.make_aligned_reads(contig, 40, 600, rng)])
+    pileup = confusion.PileupPack([("c", 0, 1500), ("c", 1500, 3000)], {"c": contig}, {"c": aligned}, 6)
+    gc.collect()                                                  # contexts that earlier tests dropped are closed before counting
+    torch.cuda.init()
+    free = []
+    for _ in range(3):
+        eng = Realigner(S, NP)
+        res = eng.align_packed(packed, NPORE_OUT_STANDARDIZE | NPORE_OUT_RLE)
+        assert not res.status[:packed.n].any() and res.rle_off[packed.n] > 0
+        outs, _, status = eng.align_many([oracle.bases_to_int(c[0]) for c in long_cases], [oracle.bases_to_int(c[1]) for c in long_cases],
+                                         [c[2] for c in long_cases])
+        # runs past the 2,047 ops of the record field with status 0 come only from the WIDE pass and its overflow list
+        assert not status.any() and any("I" * 2048 in o or "D" * 2048 in o for o in outs)
+        info = eng.get_np_info_batch([cig.bases_to_int(ref[:5000]), cig.bases_to_int(ref[5000:9000])])
+        assert [len(x) for x in info] == [5000, 4000]
+        subs, _, _, _ = eng.confusion_batch(pileup)
+        assert subs.sum() > 0
+        eng.close()
+        free.append(torch.cuda.mem_get_info()[0])
+    assert free[2] == free[0], f"free device memory after each round: {free}"
 
 
 def test_bad_cigar_is_reported_not_ub(tables, engine_factory):
