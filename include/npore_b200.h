@@ -23,6 +23,8 @@
  *                            (src/bam.pyx:149-164), computed from the alignments themselves instead of the text of
  *                            `samtools mpileup | cut -f5` (src/bam.pyx:300-314); the sum over the ranges is what
  *                            src/bam.pyx:184-192 get_confusion_matrices() reduces to.
+ *   npore_bgzf_*          <- the BGZF compression of `samtools view -b` (SAM spec section 4.1) that users ran on the
+ *                            reference's SAM output: the realigned records are written as BAM, deflated on the device.
  *   npore_last_stats      <- the wall-clock prints of src/realign.py:109,115 (per-phase device times,
  *                            cell-update counts).
  *
@@ -172,6 +174,19 @@ typedef struct npore_pileup_batch {
 /* outputs (int64, overwritten with the totals of this call): subs[5][5] indexed [ref][call], nps[max_n][max_l+1][max_l+1]
  * indexed [n-1][ref copies][called copies], inss[max_l+1], dels[max_l+1] */
 int  npore_confusion_batch(npore_ctx *ctx, const npore_pileup_batch *batch, int64_t *subs, int64_t *nps, int64_t *inss, int64_t *dels);
+
+/* BGZF compression on the device (SAM spec section 4.1).  The input is cut into members of at most 65,280 bytes; each member is
+ * a gzip member with the BC extra field, one final deflate block (dynamic Huffman codes with LZ77 matches, or stored when that
+ * is not larger) and CRC32 / ISIZE.  The output depends only on the input bytes.  No EOF block is appended.
+ * A handle has its own stream and device buffers (grown on demand); it is not a context and may live beside them.  The
+ * pointers are host pointers; the call returns when out holds *out_len bytes.  n == 0 writes nothing.  device_ms (may be
+ * NULL) receives the kernel time. */
+typedef struct npore_bgzf npore_bgzf;
+int     npore_bgzf_create(npore_bgzf **out, int device);
+void    npore_bgzf_destroy(npore_bgzf *z);
+int64_t npore_bgzf_bound(int64_t n);   /* worst case: every member stored */
+int     npore_bgzf_compress(npore_bgzf *z, const uint8_t *in, int64_t n, uint8_t *out, int64_t out_capacity,
+                            int64_t *out_len, float *device_ms /* may be NULL */);
 
 int  npore_last_stats(const npore_ctx *ctx, npore_stats *stats);
 const char *npore_strerror(int code);

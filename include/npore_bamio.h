@@ -12,6 +12,7 @@
  *   npore_sam_format / npore_sam_format_fd <- the record print of src/bam.pyx:81-84 realign_read():
  *                                           name flag rname start+1 mapq CIGAR * 0 (stop-start) seq quals HP:i:hap
  *                                           for a whole batch, in input order, from the run-length words the GPU returns.
+ *   npore_bam_format                     <- the same records as BAM (what `samtools view -b` makes of that SAM text).
  *
  * Plain C ABI; all pointers are caller-owned host memory.  Functions return 0 or a negative code; the text of the last
  * error of the calling thread is npore_io_last_error().  No CUDA involved.
@@ -95,6 +96,21 @@ int64_t  npore_sam_format_fd(int64_t n, int n_threads,
                              const uint32_t *rle, const int64_t *rle_off,
                              const uint8_t *seq_ascii, const uint8_t *qual_ascii, const int64_t *seq_off, const int32_t *has_qual,
                              const int32_t *hp, uint8_t *scratch, int64_t scratch_capacity, int fd, int64_t file_offset);
+
+/* The records of npore_sam_format as binary BAM records (SAM spec 4.2, each with its block_size), same arguments, same order.
+ * The fields are encoded as htslib's SAM -> BAM conversion encodes that SAM line: refID -1 where RNAME is '*', next_refID and
+ * next_pos -1, tlen = end - pos, bin = reg2bin(pos, pos + reference span of the CIGAR, 1 if 0), SEQ in 4 bits, QUAL phred or
+ * 0xFF * l_seq without qualities, HP as the smallest integer type holding the value (C/S/I, c/s/i when negative).
+ * Returns the bytes written; out_capacity must be at least npore_bam_bound(...).  A read name longer than 254 bytes or a CIGAR
+ * of more than 65535 operations is an error. */
+int64_t  npore_bam_bound(int64_t n, const int64_t *name_off, const int64_t *seq_off, const int64_t *rle_off);
+int64_t  npore_bam_format(int64_t n, int n_threads,
+                          const uint8_t *names, const int64_t *name_off, const int32_t *flag, const int32_t *ref_id,
+                          const uint8_t *ref_names, const int64_t *ref_name_off, int32_t n_refs,
+                          const int32_t *pos, const int32_t *end, const int32_t *mapq,
+                          const uint32_t *rle, const int64_t *rle_off,
+                          const uint8_t *seq_ascii, const uint8_t *qual_ascii, const int64_t *seq_off, const int32_t *has_qual,
+                          const int32_t *hp, uint8_t *out, int64_t out_capacity);
 
 #ifdef __cplusplus
 }

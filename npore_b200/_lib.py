@@ -48,10 +48,12 @@ class PileupBatch(C.Structure):
 
 
 EXPORTS = ["npore_ctx_create", "npore_ctx_destroy", "npore_set_stream", "npore_count_chunks", "npore_upload", "npore_run", "npore_download",
-           "npore_align_batch", "npore_get_np_info", "npore_get_np_info_batch", "npore_confusion_batch", "npore_last_stats", "npore_strerror", "npore_last_error", "npore_version"]
+           "npore_align_batch", "npore_get_np_info", "npore_get_np_info_batch", "npore_confusion_batch", "npore_last_stats", "npore_strerror", "npore_last_error", "npore_version",
+           "npore_bgzf_create", "npore_bgzf_destroy", "npore_bgzf_bound", "npore_bgzf_compress"]
 
 IO_EXPORTS = ["npore_io_last_error", "npore_bam_open", "npore_bam_advance", "npore_bam_prefetch", "npore_bam_close", "npore_bam_header_text", "npore_bam_n_refs", "npore_bam_ref",
-              "npore_bam_n_records", "npore_bam_columns", "npore_bam_gather", "npore_bam_gather_nib", "npore_sam_bound", "npore_sam_format", "npore_sam_format_fd"]
+              "npore_bam_n_records", "npore_bam_columns", "npore_bam_gather", "npore_bam_gather_nib", "npore_sam_bound", "npore_sam_format", "npore_sam_format_fd",
+              "npore_bam_bound", "npore_bam_format"]
 
 _lib = None
 
@@ -83,6 +85,13 @@ def lib():
         L.npore_last_error.argtypes = [C.c_void_p]
         L.npore_last_error.restype = C.c_char_p
         L.npore_version.restype = C.c_char_p
+        L.npore_bgzf_create.argtypes = [C.POINTER(C.c_void_p), C.c_int]
+        L.npore_bgzf_destroy.argtypes = [C.c_void_p]
+        L.npore_bgzf_destroy.restype = None
+        L.npore_bgzf_bound.argtypes = [C.c_int64]
+        L.npore_bgzf_bound.restype = C.c_int64
+        L.npore_bgzf_compress.argtypes = [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.POINTER(C.c_int64),
+                                          C.POINTER(C.c_float)]
         # include/npore_bamio.h
         vp = C.c_void_p
         L.npore_io_last_error.restype = C.c_char_p
@@ -108,5 +117,9 @@ def lib():
         L.npore_sam_format.restype = C.c_int64
         L.npore_sam_format_fd.argtypes = [C.c_int64, C.c_int] + [vp] * 6 + [C.c_int32] + [vp] * 11 + [C.c_int64, C.c_int, C.c_int64]
         L.npore_sam_format_fd.restype = C.c_int64
+        L.npore_bam_bound.argtypes = [C.c_int64, vp, vp, vp]
+        L.npore_bam_bound.restype = C.c_int64
+        L.npore_bam_format.argtypes = L.npore_sam_format.argtypes
+        L.npore_bam_format.restype = C.c_int64
         _lib = L
     return _lib

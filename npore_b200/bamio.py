@@ -6,12 +6,14 @@
                                  secondary / supplementary / unmapped; soft clips stripped from SEQ/QUAL like pysam's
                                  query_alignment_sequence; reference slice = fasta[start:stop].upper(), which is what
                                  get_reference_sequence().upper() yields)
-  create_header(...)             bam.pyx:127-145: @HD VN:1.6 SO:coordinate, @SQ per contig, @PG realigner
+  create_header(...)             bam.pyx:127-145: @HD VN:1.6 SO:coordinate, @SQ per contig, @PG realigner (header_text)
   write_bam(path, ...)           minimal BGZF/BAM writer (fixtures for the tests; records in input order)
   realign_bam(...)               ingest -> GPU batches -> ordered SAM: what realign.py:75-115 does end to end.  Uses the
                                  native reader / writer of libnpore_b200.so (include/npore_bamio.h: multi-threaded BGZF
                                  inflate, record decode into flat arrays, batch SAM formatting) and never builds
                                  per-read Python objects; the pure-Python functions above remain as the tuple API.
+                                 out_format="bam" writes the same records as BAM: batch BAM encoding on the host, BGZF
+                                 compression on the device (engine.BgzfCompressor).
                                  One batch pipeline (_realign_segments) serves both forms: the streamed windows of one
                                  device, and with devices=[...] one region shard per device (_realign_sharded).
 The GPU path is entered through npore_b200.engine (realign_bam) or npore_b200.bam.realign_reads (tuples).
@@ -36,6 +38,8 @@ _SEQ16 = "=ACMGRSVTWYHKDBN"
 _OPS = "MIDNSHP=XB"
 _SEQ_PAIR = np.frombuffer("".join(a + b for a in _SEQ16 for b in _SEQ16).encode(), dtype=np.uint8).reshape(256, 2)
 _PIPES = {}                     # _pipeline's cache
+_BGZF = {}                      # _compressor's cache
+BGZF_EOF = bytes.fromhex("1f8b08040000000000ff0600424302001b0003000000000000000000")   # SAM spec 4.1.2
 _PIPE_LOCK = threading.Lock()   # contexts of different devices are created one after the other
 _MALLOC_TUNED = False           # _keep_freed_buffers_mapped has run
 
@@ -154,15 +158,28 @@ def get_read_data(bam_fn, fasta, regions=None, max_reads=0):
                    fa[rname][rstart:rstop].upper(), 0 if hp is None else int(hp))
 
 
+def header_text(refs, argv=None):
+    """bam.pyx:127-145: the @HD / @SQ / @PG lines of the output.  refs: [(name, length)]."""
+    lines = ["@HD\tVN:1.6\tSO:coordinate\n"] + [f"@SQ\tSN:{name}\tLN:{length}\n" for name, length in refs]
+    lines.append(f"@PG\tID:realigner\tPN:realigner\tVN:{cfg.__version__}\tCL:{' '.join(argv if argv is not None else sys.argv)}\n")
+    return "".join(lines)
+
+
 def create_header(outfile, refs, argv=None):
     """bam.pyx:127-145: (re)creates the SAM with @HD / @SQ / @PG lines.  refs: [(name, length)]."""
     if os.path.dirname(outfile):
         os.makedirs(os.path.dirname(outfile), exist_ok=True)
     with open(outfile, "w") as fh:
-        fh.write("@HD\tVN:1.6\tSO:coordinate\n")
-        for name, length in refs:
-            fh.write(f"@SQ\tSN:{name}\tLN:{length}\n")
-        fh.write(f"@PG\tID:realigner\tPN:realigner\tVN:{cfg.__version__}\tCL:{' '.join(argv if argv is not None else sys.argv)}\n")
+        fh.write(header_text(refs, argv))
+
+
+def bam_header(refs, argv=None):
+    """The uncompressed BAM header (SAM spec 4.2): magic, the text of header_text, the reference list."""
+    text = header_text(refs, argv).encode()
+    out = [b"BAM\1", struct.pack("<i", len(text)), text, struct.pack("<i", len(refs))]
+    for name, length in refs:
+        out.append(struct.pack("<i", len(name.encode()) + 1) + name.encode() + b"\0" + struct.pack("<i", length))
+    return b"".join(out)
 
 
 class NativeBam:
@@ -260,10 +277,11 @@ class NativeBam:
         return o
 
 
-def format_sam(bam, sel, g, rle, rle_off, n_threads=0, cols=None, fd=None, offset=0):
+def format_sam(bam, sel, g, rle, rle_off, n_threads=0, cols=None, fd=None, offset=0, binary=False):
     """bam.pyx:83 for the selected records as one bytes-like block (npore_sam_format).  cols: the records' column values
     taken earlier (dict of int32 arrays: flag ref_id pos end mapq has_qual hp) when the reader has moved on since.
-    fd: also append the block to that file descriptor at `offset` while formatting (npore_sam_format_fd)."""
+    fd: also append the block to that file descriptor at `offset` while formatting (npore_sam_format_fd).
+    binary: the same records as uncompressed BAM records instead (npore_bam_format; fd must be None)."""
     L = bam._L
     names = "".join(n for n, _ in bam.refs).encode()
     rn_off = np.concatenate(([0], np.cumsum([len(n.encode()) for n, _ in bam.refs], dtype=np.int64)))
@@ -273,7 +291,10 @@ def format_sam(bam, sel, g, rle, rle_off, n_threads=0, cols=None, fd=None, offse
     if cols is None:
         cols = take_columns(bam, sel)
     n = len(cols["flag"])
-    cap = int(L.npore_sam_bound(n, g["name_off"].ctypes.data, g["seq_off"].ctypes.data, rle_off.ctypes.data, max([len(x) for x, _ in bam.refs] + [1])))
+    if binary:
+        cap = int(L.npore_bam_bound(n, g["name_off"].ctypes.data, g["seq_off"].ctypes.data, rle_off.ctypes.data))
+    else:
+        cap = int(L.npore_sam_bound(n, g["name_off"].ctypes.data, g["seq_off"].ctypes.data, rle_off.ctypes.data, max([len(x) for x, _ in bam.refs] + [1])))
     out = np.empty(max(cap, 1), np.uint8)
     flag, ref_id, pos, end, mapq, hq, hp = (cols[k] for k in ("flag", "ref_id", "pos", "end", "mapq", "has_qual", "hp"))
     qual = g["qual_ascii"] if g["qual_ascii"] is not None else g["seq_ascii"]
@@ -283,7 +304,10 @@ def format_sam(bam, sel, g, rle, rle_off, n_threads=0, cols=None, fd=None, offse
             rn.ctypes.data, rn_off.ctypes.data, len(bam.refs), pos.ctypes.data, end.ctypes.data, mapq.ctypes.data,
             rle.ctypes.data if len(rle) else None, rle_off.ctypes.data, g["seq_ascii"].ctypes.data, qual.ctypes.data,
             g["seq_off"].ctypes.data, hq.ctypes.data, hp.ctypes.data, out.ctypes.data, cap)
-    got = L.npore_sam_format(*args) if fd is None else L.npore_sam_format_fd(*args, int(fd), int(offset))
+    if binary:
+        got = L.npore_bam_format(*args)
+    else:
+        got = L.npore_sam_format(*args) if fd is None else L.npore_sam_format_fd(*args, int(fd), int(offset))
     if got < 0:
         raise RuntimeError(L.npore_io_last_error().decode())
     return out[:got]
@@ -323,6 +347,25 @@ def _pipeline(sub, npt, n_inflight, device=None):
     return p
 
 
+def _compressor(device, slot):
+    """Cached BgzfCompressor per (device, writer slot): the writer threads that run at the same time use different slots."""
+    from .engine import BgzfCompressor
+    dev = int(getattr(cfg.args, "device", 0) or 0) if device is None else int(device)
+    with _PIPE_LOCK:
+        z = _BGZF.get((dev, slot))
+        if z is None:
+            z = _BGZF[(dev, slot)] = BgzfCompressor(dev)
+    return z
+
+
+def _write_all(fd, data, offset):
+    view = memoryview(data).cast("B")
+    while len(view):
+        n = os.pwrite(fd, view, offset)
+        view, offset = view[n:], offset + n
+    return offset
+
+
 def _record_ops(bam, sel):
     """D/I ops of each selected record (reference span + aligned read length), from the record columns alone."""
     return (bam.end[sel] - bam.pos[sel]).astype(np.int64) + bam.aln_len[sel]
@@ -334,10 +377,12 @@ def _read_loads(bam, sel, max_b_rows=20000, r=30):
     return (ops + -(-ops // (max_b_rows - 1))) * (2 * r + 1)
 
 
-def _realign_segments(bam, segments, fa, pipe, open_out, tm, n_threads, nt_text, max_batch_ops, n_inflight, mark, t0):
+def _realign_segments(bam, segments, fa, pipe, open_out, tm, n_threads, nt_text, max_batch_ops, n_inflight, mark, t0, compressor=None):
     """The three-stage pipeline over (contig, record indices) segments, which may be produced lazily: gather batch k+1 while
     batch k is on the GPU and a writer thread formats batch k-1 and appends it to the file descriptor that open_out() returns.
-    The writer calls open_out() before its first batch and writes from the descriptor's current size on.  The descriptor must
+    The writer calls open_out(z) before its first batch and writes from the descriptor's current size on.  compressor: None
+    writes SAM text (z is None); otherwise a callable that returns the writer's BgzfCompressor z, and every batch is written as
+    BAM records compressed into BGZF members (tm["compress"]: seconds in the compressor).  The descriptor must
     not be in append mode: Linux ignores the offset of a pwrite on an append-mode descriptor, and the formatter threads place
     their slices by offset.  Records are written in segment order and counted into cfg.counter batch by batch.  n_threads:
     threads of the nibble / CIGAR gathers and of formatting; nt_text: threads of the SAM-text gather that runs beside the
@@ -353,7 +398,8 @@ def _realign_segments(bam, segments, fa, pipe, open_out, tm, n_threads, nt_text,
     def retire_loop():
         fd = -1
         try:
-            fd = open_out()
+            z = compressor() if compressor is not None else None
+            fd = open_out(z)
             end = os.fstat(fd).st_size
         except Exception as e:                        # noqa: BLE001
             state["error"] = e
@@ -372,10 +418,19 @@ def _realign_segments(bam, segments, fa, pipe, open_out, tm, n_threads, nt_text,
                      f"warps/SM={st_['fwd_warps_per_sm']} context from {1e3 * (st_['wall'][0] - t0):.1f} ms, buffers {1e3 * (st_['wall'][1] - t0):.1f}, "
                      f"to {1e3 * (st_['wall'][2] - t0):.1f} ms")
                 _report(res.status[:n], "realign_read")
-                end += len(format_sam(bam, None, g, res.rle, res.rle_off[:n + 1], n_threads, cols=cols, fd=fd, offset=end))
-                t3 = time.perf_counter()
-                mark("formatted + written")
-                tm["gpu_wait"] += t2 - t1; tm["format"] += t3 - t2; tm["write"] += time.perf_counter() - t3
+                if z is None:
+                    end += len(format_sam(bam, None, g, res.rle, res.rle_off[:n + 1], n_threads, cols=cols, fd=fd, offset=end))
+                    t3 = time.perf_counter()
+                    mark("formatted + written")
+                    tm["gpu_wait"] += t2 - t1; tm["format"] += t3 - t2; tm["write"] += time.perf_counter() - t3
+                else:
+                    raw = format_sam(bam, None, g, res.rle, res.rle_off[:n + 1], n_threads, cols=cols, binary=True)
+                    t3 = time.perf_counter()
+                    blob = z.compress(raw)
+                    t4 = time.perf_counter()
+                    end = _write_all(fd, blob, end)
+                    mark("formatted + written")
+                    tm["gpu_wait"] += t2 - t1; tm["format"] += t3 - t2; tm["compress"] += t4 - t3; tm["write"] += time.perf_counter() - t4
                 state["written"] += n
                 with cfg.counter.get_lock():
                     cfg.counter.value += n
@@ -384,6 +439,8 @@ def _realign_segments(bam, segments, fa, pipe, open_out, tm, n_threads, nt_text,
         if fd >= 0:
             os.close(fd)
 
+    if compressor is not None:
+        tm.setdefault("compress", 0.0)
     retire = threading.Thread(target=retire_loop, daemon=True)
     retire.start()
     try:
@@ -421,13 +478,14 @@ def _realign_segments(bam, segments, fa, pipe, open_out, tm, n_threads, nt_text,
     return state["written"]
 
 
-def _realign_sharded(bam, fa, pipes, devices, open_out, regions, max_reads, max_batch_ops, n_threads, n_inflight, tm, mark, t0):
+def _realign_sharded(bam, fa, pipes, devices, open_out, regions, max_reads, max_batch_ops, n_threads, n_inflight, tm, mark, t0, ext="sam"):
     """realign.py:75-115 on several GPUs of one host (SURVEY.md 8(e)): the coordinate-sorted reads are cut into len(devices)
     contiguous genomic regions of equal cell-update load (the reference's own unit of distribution is the region,
     util.py:44-93 / bam.pyx:27-28); every region is an independent ingest -> GPU -> SAM-text pipeline on its own device (no
     data-path collective) and host threads; the host gathers the per-region SAM bodies in region order into ONE file,
     byte-identical to the single-GPU output.  Region 0 writes into the output itself (open_out), the others into part files,
-    which are removed whether the call succeeds or fails.  tm: per phase, summed over the shards, plus
+    which are removed whether the call succeeds or fails.  ext "bam": every shard compresses its records on its own device and
+    the part files hold BGZF members only (no header, no EOF block), so their concatenation is valid BGZF.  tm: per phase, summed over the shards, plus
     'shards': [{device, reads, cell_updates, seconds}] and 'concat' seconds."""
     from .scheduler import cut_balanced
     tm.setdefault("concat", 0.0)
@@ -448,17 +506,20 @@ def _realign_sharded(bam, fa, pipes, devices, open_out, regions, max_reads, max_
             shard_load[int(gidx)] += int(ld[m].sum())
         done += float(ld.sum())
     tm["open"] += time.perf_counter() - t1
-    out = f"{cfg.args.out_prefix}.sam"
-    parts = [f"{cfg.args.out_prefix}.part{g}.sam" for g in range(G)]
-    opens = [open_out] + [lambda p=p: os.open(p, os.O_WRONLY | os.O_CREAT | os.O_TRUNC, 0o644) for p in parts[1:]]
+    out = f"{cfg.args.out_prefix}.{ext}"
+    parts = [f"{cfg.args.out_prefix}.part{g}.{ext}" for g in range(G)]
+    opens = [open_out] + [lambda z, p=p: os.open(p, os.O_WRONLY | os.O_CREAT | os.O_TRUNC, 0o644) for p in parts[1:]]
     nt = max(1, (n_threads or os.cpu_count() or 1) // G)
     results = [None] * G
-    shard_tm = [{k: 0.0 for k in ("gather", "gpu_wait", "format", "write")} for _ in range(G)]
+    phases = ("gather", "gpu_wait", "format", "write") + (("compress",) if ext == "bam" else ())
+    shard_tm = [{k: 0.0 for k in phases} for _ in range(G)]
 
     def shard_main(g):
         t2 = time.perf_counter()
         try:
-            n = _realign_segments(bam, shard_segs[g], fa, pipes[g], opens[g], shard_tm[g], nt, nt, max_batch_ops, n_inflight, mark, t0)
+            comp = (lambda: _compressor(devices[g], g)) if ext == "bam" else None
+            n = _realign_segments(bam, shard_segs[g], fa, pipes[g], opens[g], shard_tm[g], nt, nt, max_batch_ops, n_inflight, mark, t0,
+                                  compressor=comp)
             results[g] = (n, time.perf_counter() - t2, None)
         except Exception as e:      # noqa: BLE001
             results[g] = (0, time.perf_counter() - t2, e)
@@ -500,8 +561,8 @@ def _realign_sharded(bam, fa, pipes, devices, open_out, regions, max_reads, max_
         for part in parts[1:]:
             with contextlib.suppress(FileNotFoundError):
                 os.remove(part)
-    for k in ("gather", "gpu_wait", "format", "write"):
-        tm[k] += sum(x[k] for x in shard_tm)
+    for k in phases:
+        tm[k] = tm.get(k, 0.0) + sum(x[k] for x in shard_tm)
     tm["shards"] = [{"device": int(devices[g]), "reads": int(results[g][0]), "cell_updates": int(shard_load[g]), "seconds": round(results[g][1], 4)}
                     for g in range(G)]
     return sum(n for n, _, _ in results)
@@ -528,7 +589,7 @@ def _keep_freed_buffers_mapped():
 
 
 def realign_bam(bam_fn, fasta, out_prefix=None, regions=None, max_reads=0, argv=None, max_batch_ops=64_000_000, n_threads=0,
-                timings=None, window_bytes=16 << 20, n_inflight=3, devices=None):
+                timings=None, window_bytes=16 << 20, n_inflight=3, devices=None, out_format="sam"):
     """realign.py:75-115 without pysam / Pool: header, ingest, GPU realignment, records appended in input order
     (= coordinate order for a sorted BAM, which is what the header claims).  Returns the number of records written.
     Flat arrays all the way, as a pipeline: the reader streams the file in windows of ~window_bytes of inflated records
@@ -537,7 +598,12 @@ def realign_bam(bam_fn, fasta, out_prefix=None, regions=None, max_reads=0, argv=
     timings: optional dict that receives host seconds per phase (open, gather, gpu_wait, format = formatting + the append to the
     file, write = 0 since the formatter threads write themselves); timings["trace"] = [] collects (seconds, event) of every step.
     devices: CUDA device indices; more than one: one region-shard pipeline per device, gathered in order into one file
-    (_realign_sharded; the whole file is loaded, no streaming)."""
+    (_realign_sharded; the whole file is loaded, no streaming).
+    out_format: "sam" writes {out_prefix}.sam; "bam" writes the same header and records to {out_prefix}.bam as BAM, each batch
+    encoded on the host and compressed into BGZF members on the batch's device, with one BGZF EOF block at the end; timings then
+    also has "compress", the seconds spent in the compressor."""
+    if out_format not in ("sam", "bam"):
+        raise ValueError(f"out_format must be 'sam' or 'bam', not {out_format!r}")
     from .bam import _tables
     tm = timings if timings is not None else {}
     for k in ("open", "gather", "gpu_wait", "format", "write"):
@@ -558,12 +624,18 @@ def realign_bam(bam_fn, fasta, out_prefix=None, regions=None, max_reads=0, argv=
     streaming = len(devices) == 1 and not (regions and len(regions) > 1)
     bam = NativeBam(bam_fn, n_threads, window_bytes=window_bytes if streaming else 0)
     mark("bam open")
-    out = f"{cfg.args.out_prefix}.sam"
+    out = f"{cfg.args.out_prefix}.{out_format}"
 
-    def open_out():
+    def open_out(z):
         # called by the writer thread: the header (and the truncation of a previous output: ~2 ms for a 60 MB file) is written
         # beside the first window's inflate
-        create_header(out, bam.refs, argv)
+        if z is None:
+            create_header(out, bam.refs, argv)
+        else:
+            if os.path.dirname(out):
+                os.makedirs(os.path.dirname(out), exist_ok=True)
+            with open(out, "wb") as fh:
+                fh.write(z.compress(bam_header(bam.refs, argv)))
         mark("header written")
         return os.open(out, os.O_WRONLY)
 
@@ -575,7 +647,7 @@ def realign_bam(bam_fn, fasta, out_prefix=None, regions=None, max_reads=0, argv=
         mark("opened")
         if len(devices) > 1:
             written = _realign_sharded(bam, fa, pipes, devices, open_out, regions, max_reads, max_batch_ops, n_threads, n_inflight,
-                                       tm, mark, t0)
+                                       tm, mark, t0, ext=out_format)
         else:
             def segments():
                 kept = 0
@@ -596,7 +668,15 @@ def realign_bam(bam_fn, fasta, out_prefix=None, regions=None, max_reads=0, argv=
             # the text gather runs right after a submit: leave cores to the GPU worker thread that has just been woken (on 16
             # cores a 16-thread gather delayed the start of the upload by 2 ms) and to the writer
             nt_text = max(1, (n_threads or os.cpu_count() or 1) - int(os.environ.get("NPORE_SPARE_CORES", "3")))
-            written = _realign_segments(bam, segments(), fa, pipes[0], open_out, tm, n_threads, nt_text, max_batch_ops, n_inflight, mark, t0)
+            comp = (lambda: _compressor(devices[0], 0)) if out_format == "bam" else None
+            written = _realign_segments(bam, segments(), fa, pipes[0], open_out, tm, n_threads, nt_text, max_batch_ops, n_inflight, mark, t0,
+                                        compressor=comp)
+        if out_format == "bam":
+            fd = os.open(out, os.O_WRONLY)
+            try:
+                _write_all(fd, BGZF_EOF, os.fstat(fd).st_size)
+            finally:
+                os.close(fd)
     finally:
         bam.close()
     mark("closed")

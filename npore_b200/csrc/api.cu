@@ -10,6 +10,8 @@
 //                traceback_kernel (aln.pyx:671-742)
 //              gather / standardize / rle kernels (aln.pyx:742, bam.pyx:65-78, cig.pyx:13-38)
 //   download : per-item op strings, run-length words, chunk scores, status -> host
+// The BGZF compressor (npore_bgzf_*, bgzf.cuh) is a separate handle with its own stream: it is not a context, so it does not
+// count among the device's live contexts that share the scratch budget.
 // There is no CPU fallback: every entry point fails with NPORE_ERR_NO_DEVICE / NPORE_ERR_CUDA without a GPU.
 #include <algorithm>
 #include <atomic>
@@ -27,6 +29,7 @@
 #include "traceback.cuh"
 #include "finish.cuh"
 #include "confusion.cuh"
+#include "bgzf.cuh"
 
 namespace {
 
@@ -124,6 +127,18 @@ struct npore_ctx {
     cudaEvent_t ev[N_EVENTS]{};
     std::vector<cudaEvent_t> sub_ev;     // 4 per sub-batch
     std::string err;
+};
+
+struct npore_bgzf {
+    int device = 0;
+    cudaStream_t stream = nullptr;
+    cudaEvent_t ev[2]{};
+    DevBuf d_in, d_tok, d_slots, d_sizes, d_out, d_total;
+    ~npore_bgzf()
+    {
+        for (auto &e : ev) if (e) cudaEventDestroy(e);
+        if (stream) cudaStreamDestroy(stream);
+    }
 };
 
 namespace {
@@ -945,6 +960,84 @@ int npore_confusion_batch(npore_ctx *ctx, const npore_pileup_batch *b, int64_t *
     std::memcpy(nps, h_out.data() + 25, (size_t)ctx->P.max_n * T * T * sizeof(int64_t));
     std::memcpy(inss, h_out.data() + 25 + (size_t)ctx->P.max_n * T * T, T * sizeof(int64_t));
     std::memcpy(dels, h_out.data() + 25 + (size_t)ctx->P.max_n * T * T + T, T * sizeof(int64_t));
+    return NPORE_OK;
+}
+
+int npore_bgzf_create(npore_bgzf **out, int device)
+{
+    if (!out) return NPORE_ERR_BAD_ARG;
+    *out = nullptr;
+    int ndev = 0;
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0) { cudaGetLastError(); return NPORE_ERR_NO_DEVICE; }
+    if (device < 0 || device >= ndev) return NPORE_ERR_BAD_ARG;
+    npore_bgzf *z = new npore_bgzf();
+    z->device = device;
+    if (cudaSetDevice(device) != cudaSuccess || cudaStreamCreateWithFlags(&z->stream, cudaStreamNonBlocking) != cudaSuccess ||
+        cudaEventCreate(&z->ev[0]) != cudaSuccess || cudaEventCreate(&z->ev[1]) != cudaSuccess ||
+        cudaFuncSetAttribute(bgzf::bgzf_deflate_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, bgzf::kDynSmem) != cudaSuccess ||
+        z->d_total.ensure(sizeof(int64_t)) != cudaSuccess) {
+        cudaGetLastError();
+        npore_bgzf_destroy(z);
+        return NPORE_ERR_CUDA;
+    }
+    *out = z;
+    return NPORE_OK;
+}
+
+void npore_bgzf_destroy(npore_bgzf *z)
+{
+    if (!z) return;
+    cudaSetDevice(z->device);
+    delete z;                            // frees the buffers, on the device set above
+}
+
+int64_t npore_bgzf_bound(int64_t n)
+{
+    if (n <= 0) return 0;
+    return (n + BGZF_BLOCK - 1) / BGZF_BLOCK * (BGZF_MEMBER_OVERHEAD + 5) + n;
+}
+
+int npore_bgzf_compress(npore_bgzf *z, const uint8_t *in, int64_t n, uint8_t *out, int64_t out_capacity, int64_t *out_len,
+                        float *device_ms)
+{
+    if (!z || n < 0 || !out_len || (n && (!in || !out))) return NPORE_ERR_BAD_ARG;
+    *out_len = 0;
+    if (device_ms) *device_ms = 0.0f;
+    if (!n) return NPORE_OK;
+    const int64_t members = (n + BGZF_BLOCK - 1) / BGZF_BLOCK;
+    if (members > (1 << 30)) return NPORE_ERR_BAD_ARG;
+    auto check = [&](cudaError_t e) {
+        if (e == cudaSuccess) return NPORE_OK;
+        cudaGetLastError();
+        return e == cudaErrorMemoryAllocation ? NPORE_ERR_OOM : NPORE_ERR_CUDA;
+    };
+    int rc;
+    if ((rc = check(cudaSetDevice(z->device))) ||
+        (rc = check(z->d_in.ensure((size_t)n))) ||
+        (rc = check(z->d_tok.ensure((size_t)members * BGZF_BLOCK * sizeof(uint32_t)))) ||
+        (rc = check(z->d_slots.ensure((size_t)members * BGZF_SLOT))) ||
+        (rc = check(z->d_sizes.ensure((size_t)members * sizeof(int32_t)))) ||
+        (rc = check(z->d_out.ensure((size_t)npore_bgzf_bound(n)))))
+        return rc;
+    int64_t total = 0;
+    if ((rc = check(cudaMemcpyAsync(z->d_in.p, in, (size_t)n, cudaMemcpyHostToDevice, z->stream))) ||
+        (rc = check(cudaEventRecord(z->ev[0], z->stream))))
+        return rc;
+    bgzf::bgzf_deflate_kernel<<<(unsigned)members, BGZF_THREADS, bgzf::kDynSmem, z->stream>>>(
+        z->d_in.as<uint8_t>(), n, z->d_tok.as<uint32_t>(), z->d_slots.as<uint8_t>(), z->d_sizes.as<int32_t>());
+    bgzf::bgzf_gather_kernel<<<(unsigned)members, BGZF_THREADS, 0, z->stream>>>(
+        z->d_slots.as<uint8_t>(), z->d_sizes.as<int32_t>(), (int)members, z->d_out.as<uint8_t>(), z->d_total.as<int64_t>());
+    if ((rc = check(cudaGetLastError())) ||
+        (rc = check(cudaEventRecord(z->ev[1], z->stream))) ||
+        (rc = check(cudaMemcpyAsync(&total, z->d_total.p, sizeof(total), cudaMemcpyDeviceToHost, z->stream))) ||
+        (rc = check(cudaStreamSynchronize(z->stream))))
+        return rc;
+    if (total > out_capacity) return NPORE_ERR_CAPACITY;
+    if ((rc = check(cudaMemcpyAsync(out, z->d_out.p, (size_t)total, cudaMemcpyDeviceToHost, z->stream))) ||
+        (rc = check(cudaStreamSynchronize(z->stream))))
+        return rc;
+    if (device_ms && (rc = check(cudaEventElapsedTime(device_ms, z->ev[0], z->ev[1])))) return rc;
+    *out_len = total;
     return NPORE_OK;
 }
 

@@ -10,7 +10,9 @@
 
 #include <algorithm>
 #include <atomic>
+#include <cctype>
 #include <cerrno>
+#include <climits>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -588,6 +590,87 @@ int64_t npore_sam_format_fd(int64_t n, int n_threads,
     if (fd < 0 || file_offset < 0) return io_fail(NPORE_IO_ERR_ARG, "bad file descriptor / offset");
     return sam_format_impl(n, n_threads, names, name_off, flag, ref_id, ref_names, ref_name_off, n_refs, pos, end, mapq, rle, rle_off,
                            seq_ascii, qual_ascii, seq_off, has_qual, hp, scratch, scratch_capacity, fd, file_offset);
+}
+
+int64_t npore_bam_bound(int64_t n, const int64_t *name_off, const int64_t *seq_off, const int64_t *rle_off)
+{
+    if (n < 0 || (n && (!name_off || !seq_off || !rle_off))) return NPORE_IO_ERR_ARG;
+    if (!n) return 0;
+    // per record: block_size + 32 fixed bytes + the name's NUL + the HP tag (at most 7 bytes); SEQ + QUAL <= 2 bytes per base
+    return (name_off[n] - name_off[0]) + 2 * (seq_off[n] - seq_off[0]) + 4 * (rle_off[n] - rle_off[0]) + n * 48;
+}
+
+int64_t npore_bam_format(int64_t n, int n_threads,
+                         const uint8_t *names, const int64_t *name_off, const int32_t *flag, const int32_t *ref_id,
+                         const uint8_t *ref_names, const int64_t *ref_name_off, int32_t n_refs,
+                         const int32_t *pos, const int32_t *end, const int32_t *mapq,
+                         const uint32_t *rle, const int64_t *rle_off,
+                         const uint8_t *seq_ascii, const uint8_t *qual_ascii, const int64_t *seq_off, const int32_t *has_qual,
+                         const int32_t *hp, uint8_t *out, int64_t out_capacity)
+{
+    (void)ref_names; (void)ref_name_off;
+    if (n < 0) return io_fail(NPORE_IO_ERR_ARG, "negative count");
+    if (!n) return 0;
+    if (!names || !name_off || !flag || !ref_id || !pos || !end || !mapq || !rle_off || !seq_off || !has_qual || !hp || !out)
+        return io_fail(NPORE_IO_ERR_ARG, "null argument");
+    uint8_t nt16[256];
+    for (int c = 0; c < 256; c++) nt16[c] = 15;
+    for (int i = 0; i < 16; i++) { nt16[kNt16[i]] = (uint8_t)i; nt16[std::tolower(kNt16[i])] = (uint8_t)i; }
+    auto hp_bytes = [](int32_t v) { return v < 0 ? (v >= -128 ? 1 : v >= -32768 ? 2 : 4) : (v <= 255 ? 1 : v <= 65535 ? 2 : 4); };
+    std::vector<int64_t> at((size_t)n + 1, 0);
+    std::atomic<int> bad{0};
+    // pass 1: exact record lengths
+    parallel_for(n, n_threads, [&](int64_t lo, int64_t hi) {
+        for (int64_t k = lo; k < hi; k++) {
+            const int64_t nl = name_off[k + 1] - name_off[k], nc = rle_off[k + 1] - rle_off[k], sl = seq_off[k + 1] - seq_off[k];
+            if (nl > 254 || nc > 65535 || sl > INT32_MAX) { bad = 1; continue; }
+            at[(size_t)k + 1] = 4 + 32 + nl + 1 + 4 * nc + (sl + 1) / 2 + sl + 3 + hp_bytes(hp[k]);
+        }
+    });
+    if (bad) return io_fail(NPORE_IO_ERR_ARG, "record not representable in BAM (read name > 254 bytes or CIGAR > 65535 operations)");
+    for (int64_t k = 0; k < n; k++) at[(size_t)k + 1] += at[(size_t)k];
+    if (at[(size_t)n] > out_capacity) return io_fail(NPORE_IO_ERR_ARG, "output buffer too small (use npore_bam_bound)");
+    // pass 2: write (SAM spec 4.2; the fields of the SAM line of npore_sam_format, encoded as htslib's SAM -> BAM conversion does)
+    parallel_for(n, n_threads, [&](int64_t lo, int64_t hi) {
+        for (int64_t k = lo; k < hi; k++) {
+            uint8_t *o = out + at[(size_t)k];
+            const int64_t nl = name_off[k + 1] - name_off[k], nc = rle_off[k + 1] - rle_off[k], sl = seq_off[k + 1] - seq_off[k];
+            int64_t span = 0;
+            for (int64_t g = rle_off[k]; g < rle_off[k + 1]; g++) {
+                const uint32_t op = rle[g] & 15u;
+                if (op == 0 || op == 2 || op == 3 || op == 7 || op == 8) span += rle[g] >> 4;
+            }
+            const int32_t p = pos[k];
+            const int32_t rid = ref_id[k] >= 0 && ref_id[k] < n_refs ? ref_id[k] : -1;
+            const int64_t e = (int64_t)p + (span ? span : 1) - 1;       // hts_reg2bin(beg, end) of the 0-based half-open span
+            const int bin = (p >> 14 == e >> 14) ? 4681 + (p >> 14) : (p >> 17 == e >> 17) ? 585 + (p >> 17) :
+                            (p >> 20 == e >> 20) ? 73 + (p >> 20) : (p >> 23 == e >> 23) ? 9 + (p >> 23) :
+                            (p >> 26 == e >> 26) ? 1 + (p >> 26) : 0;
+            const int32_t fixed[9] = {(int32_t)(at[(size_t)k + 1] - at[(size_t)k] - 4), rid, p, 0, 0, (int32_t)sl, -1, -1, end[k] - p};
+            std::memcpy(o, fixed, 12);
+            o[12] = (uint8_t)(nl + 1); o[13] = (uint8_t)mapq[k];
+            const uint16_t bn = (uint16_t)bin, ncig = (uint16_t)nc, fl = (uint16_t)flag[k];
+            std::memcpy(o + 14, &bn, 2); std::memcpy(o + 16, &ncig, 2); std::memcpy(o + 18, &fl, 2);
+            std::memcpy(o + 20, fixed + 5, 16);
+            o += 36;
+            std::memcpy(o, names + name_off[k], (size_t)nl); o += nl; *o++ = 0;
+            if (nc) std::memcpy(o, rle + rle_off[k], (size_t)nc * 4);
+            o += 4 * nc;
+            const uint8_t *sq = seq_ascii + seq_off[k];
+            for (int64_t i = 0; i + 1 < sl; i += 2) *o++ = (uint8_t)(nt16[sq[i]] << 4 | nt16[sq[i + 1]]);
+            if (sl & 1) *o++ = (uint8_t)(nt16[sq[sl - 1]] << 4);
+            if (has_qual[k] && sl) {
+                const uint8_t *q = qual_ascii + seq_off[k];
+                for (int64_t i = 0; i < sl; i++) o[i] = (uint8_t)(q[i] - 33);
+            } else std::memset(o, 0xFF, (size_t)sl);
+            o += sl;
+            const int32_t v = hp[k];
+            const int nb = hp_bytes(v);
+            o[0] = 'H'; o[1] = 'P'; o[2] = (uint8_t)(v < 0 ? (nb == 1 ? 'c' : nb == 2 ? 's' : 'i') : (nb == 1 ? 'C' : nb == 2 ? 'S' : 'I'));
+            std::memcpy(o + 3, &v, (size_t)nb);          // little-endian: the low bytes of the value
+        }
+    });
+    return at[(size_t)n];
 }
 
 }  // extern "C"

@@ -422,6 +422,47 @@ class Realigner:
         return outs, [res.scores(i).copy() for i in range(packed.n)], res.status[:packed.n].copy()
 
 
+class BgzfCompressor:
+    """BGZF compression on one device (npore_bgzf_*): compress(buf) returns the BGZF members of buf (no EOF block) as a
+    view of a pinned buffer that the next call reuses.  last_device_ms: kernel time of the last call."""
+
+    def __init__(self, device=0):
+        self._L = _lib.lib()
+        self._z = C.c_void_p()
+        self.device = int(device)
+        rc = self._L.npore_bgzf_create(C.byref(self._z), self.device)
+        if rc != 0:
+            self._z = C.c_void_p()
+            raise NporeError(f"npore_bgzf_create failed: {self._L.npore_strerror(rc).decode()} "
+                             "(npore_b200 needs a CUDA device; there is no CPU fallback)")
+        self._in = self._out = None
+        self.last_device_ms = 0.0
+
+    def compress(self, buf):
+        src = np.frombuffer(buf, dtype=np.uint8) if not isinstance(buf, np.ndarray) else buf.reshape(-1).view(np.uint8)
+        n = len(src)
+        if self._in is None or len(self._in[0]) < n:
+            self._in = _pinned(n + n // 4, np.uint8)
+        cap = int(self._L.npore_bgzf_bound(n))
+        if self._out is None or len(self._out[0]) < cap:
+            self._out = _pinned(cap + cap // 4, np.uint8)
+        pin_in, pin_out = self._in[0], self._out[0]
+        pin_in[:n] = src
+        got, ms = C.c_int64(), C.c_float()
+        rc = self._L.npore_bgzf_compress(self._z, pin_in.ctypes.data, n, pin_out.ctypes.data, len(pin_out), C.byref(got), C.byref(ms))
+        if rc != 0:
+            raise NporeError(f"npore_bgzf_compress: {self._L.npore_strerror(rc).decode()}")
+        self.last_device_ms = float(ms.value)
+        return pin_out[:got.value]
+
+    def close(self):
+        if getattr(self, "_z", None) and self._z.value:
+            self._L.npore_bgzf_destroy(self._z)
+            self._z = C.c_void_p()
+
+    __del__ = close
+
+
 class PipelinedRealigner:
     """Several batches in flight on one GPU: `n_inflight` independent contexts, each with its own CUDA stream and host
     thread.  While one batch is in its kernels, the next one's host->device copies and the previous one's device->host
