@@ -170,6 +170,17 @@ typedef struct npore_pileup_batch {
     const int32_t *range_reads;      /* per range: indices of the reads overlapping it, ascending position       */
     const int64_t *range_reads_off;  /* [R+1]                                                                    */
     int32_t        min_base_q;       /* samtools mpileup -Q (default 13)                                         */
+    /* Optional: the reads in BAM's own packing, as npore_bam_gather_nib / npore_bam_gather write them, so that the host does
+     * no per-base work.  When seq_nib is not NULL, seq_ascii is ignored: read i's bases are the seq_off[i+1] - seq_off[i]
+     * nibbles starting at nibble seq_nib_start[i] of seq_nib (same layout as npore_batch.seq_nib), decoded through
+     * "=ACMGRSVTWYHKDBN" into the letter the ASCII form would hold (so N is base 0 and =, IUPAC codes drop the rest of the
+     * line, as in the ASCII form).  qual then holds phred+33 bytes (npore_bam_gather's qual_ascii) at seq_off, and has_qual
+     * [n] is required with it: a read with has_qual[i] == 0 (QUAL 0xFF in the file) passes every base, as qual == NULL does
+     * for all reads.  Leave all four zero for the ASCII form. */
+    const uint8_t *seq_nib;
+    const int64_t *seq_nib_start;    /* [n] nibble offsets                                                        */
+    int64_t        seq_nib_bytes;    /* bytes in seq_nib                                                          */
+    const int32_t *has_qual;         /* [n] nibble form only                                                      */
 } npore_pileup_batch;
 /* outputs (int64, overwritten with the totals of this call): subs[5][5] indexed [ref][call], nps[max_n][max_l+1][max_l+1]
  * indexed [n-1][ref copies][called copies], inss[max_l+1], dels[max_l+1] */

@@ -44,7 +44,8 @@ class PileupBatch(C.Structure):
                 ("ref_ascii", C.c_void_p), ("ref_off", C.c_void_p),
                 ("n_reads", C.c_int32), ("read_pos", C.c_void_p), ("seq_ascii", C.c_void_p), ("qual", C.c_void_p),
                 ("seq_off", C.c_void_p), ("cigar_rle", C.c_void_p), ("cigar_off", C.c_void_p),
-                ("range_reads", C.c_void_p), ("range_reads_off", C.c_void_p), ("min_base_q", C.c_int32)]
+                ("range_reads", C.c_void_p), ("range_reads_off", C.c_void_p), ("min_base_q", C.c_int32),
+                ("seq_nib", C.c_void_p), ("seq_nib_start", C.c_void_p), ("seq_nib_bytes", C.c_int64), ("has_qual", C.c_void_p)]
 
 
 EXPORTS = ["npore_ctx_create", "npore_ctx_destroy", "npore_set_stream", "npore_count_chunks", "npore_upload", "npore_run", "npore_download",

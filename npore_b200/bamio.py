@@ -258,13 +258,15 @@ class NativeBam:
             raise RuntimeError(self._L.npore_io_last_error().decode())
         return cig[:int(off[-1])], off
 
-    def gather(self, sel, n_threads=0, want_qual=True, want_names=True, want_codes=True, want_cigar=True):
+    def gather(self, sel, n_threads=0, want_qual=True, want_names=True, want_codes=True, want_cigar=True, want_seq=True):
         """Flat arrays of the selected records: dict with seq_ascii, seq_codes, qual_ascii, seq_off, cigar, cig_off, names,
-        name_off (soft clips removed, S/H dropped from the CIGAR; bam.pyx:41-44, 59)."""
+        name_off (soft clips removed, S/H dropped from the CIGAR; bam.pyx:41-44, 59).  want_seq=False: no seq_ascii (None),
+        so that e.g. a qualities-only gather does no per-base decode.  qual_ascii of a record without qualities (has_qual 0)
+        is left unwritten."""
         sel = np.ascontiguousarray(sel, dtype=np.int64)
         off = lambda col: np.concatenate(([0], np.cumsum(col[sel], dtype=np.int64)))   # noqa: E731
         o = {"seq_off": off(self.aln_len), "cig_off": off(self.n_cigar), "name_off": off(self.name_len)}
-        o["seq_ascii"] = np.empty(max(int(o["seq_off"][-1]), 1), np.uint8)
+        o["seq_ascii"] = np.empty(max(int(o["seq_off"][-1]), 1), np.uint8) if want_seq else None
         o["seq_codes"] = np.empty(max(int(o["seq_off"][-1]), 1), np.uint8) if want_codes else None
         o["qual_ascii"] = np.empty(max(int(o["seq_off"][-1]), 1), np.uint8) if want_qual else None
         o["cigar"] = np.empty(max(int(o["cig_off"][-1]), 1), np.uint32) if want_cigar else None

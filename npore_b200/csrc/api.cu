@@ -112,6 +112,7 @@ struct npore_ctx {
     struct {
         DevBuf range_start, range_end, ref_ascii, ref_off, ref_codes, raw, ebits;
         DevBuf read_pos, seq, qual, seq_off, rle, cig_off, g_roff, g_qoff, read_end;
+        DevBuf nib_start, has_qual;    // the nibble form's extra arrays (seq then holds the packed bases)
         DevBuf range_reads, range_reads_off, list_maxend, line_of, pos_off;
         DevBuf out;                    // zeroed: the counts, the error flag, the coverage difference array
     } pileup;
@@ -857,13 +858,16 @@ int npore_confusion_batch(npore_ctx *ctx, const npore_pileup_batch *b, int64_t *
 {
     if (!ctx || !b || !subs || !nps || !inss || !dels || b->n_ranges < 0 || b->n_reads < 0) return NPORE_ERR_BAD_ARG;
     const int R = b->n_ranges, n = b->n_reads, T = ctx->P.max_l + 1;
+    const bool nib = b->seq_nib != nullptr;     // BAM's 4-bit bases and phred+33 qualities instead of ASCII and phred
     const size_t n_out = 25 + (size_t)ctx->P.max_n * T * T + 2 * (size_t)T;
     std::memset(subs, 0, 25 * sizeof(int64_t)); std::memset(nps, 0, (size_t)ctx->P.max_n * T * T * sizeof(int64_t));
     std::memset(inss, 0, T * sizeof(int64_t)); std::memset(dels, 0, T * sizeof(int64_t));
     if (R == 0) return NPORE_OK;
     if (!b->range_start || !b->range_end || !b->ref_ascii || !b->ref_off || !b->range_reads_off ||
-        (n && (!b->read_pos || !b->seq_ascii || !b->seq_off || !b->cigar_rle || !b->cigar_off)))
+        (n && (!b->read_pos || (nib ? !b->seq_nib_start : !b->seq_ascii) || !b->seq_off || !b->cigar_rle || !b->cigar_off)))
         return fail(ctx, NPORE_ERR_BAD_ARG, "confusion: null array");
+    if (nib && n && b->qual && !b->has_qual) return fail(ctx, NPORE_ERR_BAD_ARG, "confusion: has_qual is required with packed bases and qualities");
+    if (nib && b->seq_nib_bytes < 0) return fail(ctx, NPORE_ERR_BAD_ARG, "confusion: negative seq_nib_bytes");
     if (b->ref_off[0] != 0 || b->range_reads_off[0] != 0 || (n && (b->seq_off[0] != 0 || b->cigar_off[0] != 0)))
         return fail(ctx, NPORE_ERR_BAD_ARG, "confusion: offsets must start at 0");
     std::vector<int64_t> pos_off((size_t)R + 1, 0);
@@ -886,6 +890,10 @@ int npore_confusion_batch(npore_ctx *ctx, const npore_pileup_batch *b, int64_t *
     for (int i = 0; i < n; i++)
         if (b->seq_off[i + 1] < b->seq_off[i] || b->cigar_off[i + 1] < b->cigar_off[i] || b->seq_off[i + 1] - b->seq_off[i] > 0x7ffffff0ll)
             return fail(ctx, NPORE_ERR_BAD_ARG, "confusion: bad read offsets");
+    if (nib)
+        for (int i = 0; i < n; i++)
+            if (b->seq_nib_start[i] < 0 || b->seq_nib_start[i] + (b->seq_off[i + 1] - b->seq_off[i]) > 2 * b->seq_nib_bytes)
+                return fail(ctx, NPORE_ERR_BAD_ARG, "confusion: packed read outside seq_nib");
     const int64_t seq_total = n ? b->seq_off[n] : 0, n_words = n ? b->cigar_off[n] : 0;
     CU(cudaSetDevice(ctx->device));
     auto &d = ctx->pileup;
@@ -906,7 +914,11 @@ int npore_confusion_batch(npore_ctx *ctx, const npore_pileup_batch *b, int64_t *
     CM_TRY(d.raw.ensure(std::max<size_t>((size_t)total_ref * 8, 16)));
     CM_TRY(d.ebits.ensure(sizeof(uint32_t) * (size_t)(total_ref / 32 + 2 * (size_t)R + 8)));
     CM_TRY(put(d.read_pos, b->read_pos, sizeof(int64_t) * n));
-    CM_TRY(put(d.seq, b->seq_ascii, (size_t)seq_total));
+    if (nib) {
+        CM_TRY(put(d.seq, b->seq_nib, (size_t)b->seq_nib_bytes));
+        CM_TRY(put(d.nib_start, b->seq_nib_start, sizeof(int64_t) * n));
+        if (have_q) CM_TRY(put(d.has_qual, b->has_qual, sizeof(int32_t) * n));
+    } else CM_TRY(put(d.seq, b->seq_ascii, (size_t)seq_total));
     if (have_q) CM_TRY(put(d.qual, b->qual, (size_t)seq_total));
     CM_TRY(put(d.seq_off, b->seq_off, sizeof(int64_t) * (n + 1)));
     CM_TRY(put(d.rle, b->cigar_rle, sizeof(uint32_t) * (size_t)n_words));
@@ -940,13 +952,16 @@ int npore_confusion_batch(npore_ctx *ctx, const npore_pileup_batch *b, int64_t *
         a.bad = reinterpret_cast<int *>(o + n_out);
         a.diff = reinterpret_cast<int32_t *>(o + n_out + 2);
         a.max_n = ctx->P.max_n; a.max_l = ctx->P.max_l; a.min_bq = b->min_base_q;
+        a.seq_nib_start = nib ? d.nib_start.as<int64_t>() : nullptr; a.has_qual = nib && have_q ? d.has_qual.as<int32_t>() : nullptr;
         const int sm = ctx->stats.sm_count > 0 ? ctx->stats.sm_count : 148;
         cm_codes_kernel<<<sm * 4, 256, 0, ctx->stream>>>(a.ref_ascii, a.ref_codes, total_ref);
         cm_np_kernel<<<R, ANN_THREADS, 0, ctx->stream>>>(a);
         if (n) cm_read_kernel<<<(n + CM_THREADS / 32 - 1) / (CM_THREADS / 32), CM_THREADS, 0, ctx->stream>>>(a);
         cm_range_kernel<<<R, CM_THREADS, 0, ctx->stream>>>(a);
         const int64_t want = (total_pos + CM_THREADS / 32 - 1) / (CM_THREADS / 32);
-        cm_pileup_kernel<<<(int)std::min<int64_t>(want, (int64_t)sm * 8), CM_THREADS, 0, ctx->stream>>>(a);
+        const int grid = (int)std::min<int64_t>(want, (int64_t)sm * 8);
+        if (nib) cm_pileup_kernel<CmNibRead><<<grid, CM_THREADS, 0, ctx->stream>>>(a);
+        else cm_pileup_kernel<CmAsciiRead><<<grid, CM_THREADS, 0, ctx->stream>>>(a);
         e = cudaGetLastError();
         CM_TRY(cudaMemcpyAsync(h_out.data(), o, sizeof(unsigned long long) * (n_out + 2), cudaMemcpyDeviceToHost, ctx->stream));
         CM_TRY(cudaStreamSynchronize(ctx->stream));

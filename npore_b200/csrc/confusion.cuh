@@ -42,6 +42,34 @@ struct ConfusionArgs {
     unsigned long long *subs, *nps, *inss, *dels; // outputs
     int *bad;                                     // set when an unsupported CIGAR op (P, B) is seen
     int max_n, max_l, min_bq;
+    // nibble form (CmNibRead): seq holds BAM's 4-bit bases, read rd's base i is nibble seq_nib_start[rd] + i; qual is phred+33
+    // and only read for reads with has_qual[rd] != 0.  Last in the struct so that the ASCII form's parameter offsets stay put.
+    const int64_t *seq_nib_start; const int32_t *has_qual;
+};
+
+// How cm_pileup_kernel reads a read's bases and qualities.  load() runs once per (position, read); base() returns the letter
+// the ASCII form would hold at query offset off + i (upper case for the nibble form), qual() the phred value at query offset i.
+struct CmAsciiRead {
+    __device__ __forceinline__ void load(const ConfusionArgs &, int) {}
+    __device__ __forceinline__ uint8_t base(const ConfusionArgs &a, int64_t sb, int64_t off, int i) const { return a.seq[sb + off + i]; }
+    __device__ __forceinline__ int qual(const ConfusionArgs &a, int64_t sb, int i) const { return a.qual ? (int)a.qual[sb + i] : 255; }
+};
+
+// BAM's base table "=ACMGRSVTWYHKDBN" (SAM spec 4.2.3), eight letters per 64-bit immediate (byte k = letter k): the decode
+// reads no memory, and no __constant__ table shifts the constant-bank layout of the other kernels of the module
+constexpr uint64_t cm_pack8(const char *s) { uint64_t v = 0; for (int k = 7; k >= 0; k--) v = v << 8 | (uint8_t)s[k]; return v; }
+constexpr uint64_t kCmNt16Lo = cm_pack8("=ACMGRSV"), kCmNt16Hi = cm_pack8("TWYHKDBN");
+__device__ __forceinline__ uint8_t cm_nt16(uint32_t nib) { return (uint8_t)(((nib & 8u) ? kCmNt16Hi : kCmNt16Lo) >> (8 * (nib & 7u))); }
+
+struct CmNibRead {
+    int64_t nb = 0; bool hq = false;
+    __device__ __forceinline__ void load(const ConfusionArgs &a, int rd) { nb = a.seq_nib_start[rd]; hq = a.qual && a.has_qual[rd]; }
+    __device__ __forceinline__ uint8_t base(const ConfusionArgs &a, int64_t, int64_t off, int i) const {
+        const int64_t k = nb + off + i;
+        const uint8_t v = a.seq[k >> 1];
+        return cm_nt16((k & 1) ? (v & 15u) : (v >> 4u));      // SAM spec 4.2.3: first base in the high nibble
+    }
+    __device__ __forceinline__ int qual(const ConfusionArgs &a, int64_t sb, int i) const { return hq ? (int)(uint8_t)(a.qual[sb + i] - 33) : 255; }
 };
 
 __global__ void cm_codes_kernel(const uint8_t *ascii, uint8_t *codes, int64_t n)
@@ -162,7 +190,8 @@ __global__ void __launch_bounds__(CM_THREADS) cm_range_kernel(const ConfusionArg
 
 __device__ __forceinline__ uint32_t cm_below(int k) { return k >= 32 ? 0xffffffffu : ((1u << k) - 1u); }
 
-// one warp per reference position; CTA-local histograms for the hot counters
+// one warp per reference position; CTA-local histograms for the hot counters.  Rd: CmAsciiRead or CmNibRead.
+template <typename Rd>
 __global__ void __launch_bounds__(CM_THREADS) cm_pileup_kernel(const ConfusionArgs a)
 {
     __shared__ unsigned int s_subs[25];
@@ -211,6 +240,7 @@ __global__ void __launch_bounds__(CM_THREADS) cm_pileup_kernel(const ConfusionAr
             bool entry = false, err = false, isbase = false;
             int code = 0, indel = 0;
             int64_t q0 = 0, sb = 0; int lq = 0;
+            Rd rdr;
             if (k < hi) {
                 const int rd = a.range_reads[k];
                 if (p < a.read_end[rd]) {
@@ -224,16 +254,17 @@ __global__ void __launch_bounds__(CM_THREADS) cm_pileup_kernel(const ConfusionAr
                     const int qoff = a.g_qoff[u];
                     const int qpos = is_del ? qoff : qoff + t;
                     sb = a.seq_off[rd]; lq = (int)(a.seq_off[rd + 1] - sb);
+                    rdr.load(a, rd);
                     if (t == n - 1 && u + 1 < c1) {        // announcement of the next op (htslib resolve_cigar2)
                         const int op2 = (int)(a.rle[u + 1] & 15u);
                         if (op2 == 2 && op != 2) { for (int64_t g = u + 1; g < c1 && (a.rle[g] & 15u) == 2u; g++) indel -= (int)(a.rle[g] >> 4); }
                         else if (op2 == 1) { for (int64_t g = u + 1; g < c1 && (a.rle[g] & 15u) == 1u; g++) indel += (int)(a.rle[g] >> 4); }
                     }
-                    const int q = qpos < lq ? (a.qual ? (int)a.qual[sb + qpos] : 255) : 0;
+                    const int q = qpos < lq ? rdr.qual(a, sb, qpos) : 0;
                     entry = q >= a.min_bq;
                     if (is_del) err = (op == 3);
                     else {
-                        uint8_t ch = qpos < lq ? a.seq[sb + qpos] : (uint8_t)'N';
+                        uint8_t ch = qpos < lq ? rdr.base(a, sb, qpos, 0) : (uint8_t)'N';
                         if (ch >= 'a' && ch <= 'z') ch -= 32;
                         code = ch == 'N' ? 0 : ch == 'A' ? 1 : ch == 'C' ? 2 : ch == 'G' ? 3 : ch == 'T' ? 4 : -1;
                         err = code < 0; isbase = !err;
@@ -287,7 +318,7 @@ __global__ void __launch_bounds__(CM_THREADS) cm_pileup_kernel(const ConfusionAr
                     else if (cnv) {
                         if ((int64_t)line + 1 + n > have) cnv = false;       // unit clipped at the contig end never matches
                         for (int i = 0; cnv && i < len; i++) {
-                            uint8_t ch = (q0 + i) < lq ? a.seq[sb + q0 + i] : (uint8_t)0;
+                            uint8_t ch = (q0 + i) < lq ? rdr.base(a, sb, q0, i) : (uint8_t)0;
                             if (ch >= 'a' && ch <= 'z') ch -= 32;
                             cnv = ch == refa[line + 1 + (i % n)];
                         }

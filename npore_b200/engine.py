@@ -392,7 +392,9 @@ class Realigner:
 
     def confusion_batch(self, pb):
         """calc_confusion_matrices (bam.pyx:351-510) for the ranges of a confusion.PileupPack; returns int64
-        subs[5,5], nps[max_n,max_l+1,max_l+1], inss[max_l+1], dels[max_l+1] summed over the ranges."""
+        subs[5,5], nps[max_n,max_l+1,max_l+1], inss[max_l+1], dels[max_l+1] summed over the ranges.
+        A pack with a `seq_nib` attribute (not None) is in the nibble form of npore_pileup_batch: bases in BAM's 4-bit packing
+        (seq_nib, seq_nib_start), phred+33 qualities and has_qual; its seq_ascii is ignored."""
         from ._lib import PileupBatch
         T = self.params["max_l"] + 1
         subs = np.zeros((5, 5), np.int64); nps = np.zeros((self.params["max_n"], T, T), np.int64)
@@ -402,6 +404,10 @@ class Realigner:
                         len(pb.read_pos), ptr(pb.read_pos), ptr(pb.seq_ascii), ptr(pb.qual), pb.seq_off.ctypes.data,
                         ptr(pb.cigar_rle), pb.cigar_off.ctypes.data, ptr(pb.range_reads), pb.range_reads_off.ctypes.data,
                         int(pb.min_base_q))
+        nib = getattr(pb, "seq_nib", None)
+        if nib is not None:                  # the pointer must be set even when every read is empty
+            b.seq_nib, b.seq_nib_start, b.seq_nib_bytes = nib.ctypes.data, ptr(pb.seq_nib_start), len(nib)
+            b.has_qual = ptr(pb.has_qual)
         self._check(self._L.npore_confusion_batch(self._ctx, C.byref(b), subs.ctypes.data, nps.ctypes.data, inss.ctypes.data,
                                                   dels.ctypes.data), "npore_confusion_batch")
         return subs, nps, inss, dels
