@@ -9,13 +9,14 @@
 
 #define NP_MAXN 6          // compile-time ceiling for cfg.args.max_n (realign.py:47-49 default 6)
 #define NP_RING 8          // anti-diagonals of history kept for the LEN/SHR gathers (needs >= max_n + 1)
-// packed traceback record (uint16): [15:13] TYP  [12] DEL state extended (val2 < val1, aln.pyx:558)  [11] INS state extended
-// (aln.pyx:536)  [10:0] RUN of a MAT / LEN / SHR record.  INS/DEL run lengths are not stored: they are the number of
-// consecutive 'extended' bits walked by the traceback (equal to the reference's RUN by its recurrence aln.pyx:537-543).
+// packed traceback record (uint16): [15] INS state extended (aln.pyx:536)  [14] DEL state extended (val2 < val1, aln.pyx:558)
+// [13:11] TYP  [10:0] RUN of a MAT / LEN / SHR record.  INS/DEL run lengths are not stored: they are the number of consecutive
+// 'extended' bits walked by the traceback (equal to the reference's RUN by its recurrence aln.pyx:537-543).  The flags sit on
+// top because the forward kernel gets them as float sign bits (forward.cuh).
 #define NP_RUN_SAT 2047
-#define NP_REC_TYP 13
-#define NP_REC_IE 0x0800u
-#define NP_REC_DE 0x1000u
+#define NP_REC_TYP 11
+#define NP_REC_IE 0x8000u
+#define NP_REC_DE 0x4000u
 #define NP_PAD 96          // zero records after every colrec/rowrec slice (band prefetch runs ahead)
 #define NP_TABQ 2048       // q = trunc(run/n) entries of the re-laid score tables (run saturates at NP_RUN_SAT < NP_TABQ; forward.cuh)
 

@@ -77,9 +77,11 @@ struct ForwardArgs {
 #define FWD_SPIN_NS 256
 #endif
 // words of saved per-lane state per cell: Mv1 Iv1 Dv1 dgv Mr1 dgr cc(8) rw
-#define FWD_IE_BIT 27      // NP_REC_IE / NP_REC_DE in the upper half word of a record
-#define FWD_DE_BIT 28
+#define FWD_IE_BIT 31      // NP_REC_IE / NP_REC_DE in the upper half word of a record: IE is the sign bit of the INS difference as it
+#define FWD_DE_BIT 30      // stands, DE the sign bit of the DEL difference moved down by one
+#define FWD_TYP_SH (NP_REC_TYP + 16)
 static_assert((NP_REC_IE << 16) == (1u << FWD_IE_BIT) && (NP_REC_DE << 16) == (1u << FWD_DE_BIT), "record flag bits");
+static_assert(((7u << FWD_TYP_SH) | ((uint32_t)NP_RUN_SAT << 16)) < (1u << FWD_DE_BIT), "TYP and RUN below the flag bits");
 #define FWD_RR_WORDS 15
 #define FWD_RR_HDR 32      // uint32 words: d, Id, Dd
 static __host__ __device__ inline size_t fwd_rr_state_words(int cpl) { return (size_t)FWD_RR_HDR + (size_t)FWD_RR_WORDS * cpl * 32 + (size_t)32 * cpl * 32; }
@@ -123,6 +125,9 @@ __device__ __forceinline__ uint4 lds128(uint32_t a)
 // a ? b : c per bit (one LOP3)
 __device__ __forceinline__ uint32_t bitsel(uint32_t m, uint32_t x, uint32_t y) { return (x & m) | (y & ~m); }
 __device__ __forceinline__ float bitsel_f(uint32_t m, float x, float y) { return __uint_as_float((__float_as_uint(x) & m) | (__float_as_uint(y) & ~m)); }
+// a | (b & M) as one LOP3 (left to itself, ptxas ORs two such masked words together first: one LOP3 more)
+template <uint32_t M> __device__ __forceinline__ uint32_t or_masked(uint32_t a, uint32_t b)
+{ uint32_t d; asm("lop3.b32 %0, %1, %2, %3, 0xf8;" : "=r"(d) : "r"(a), "r"(b), "n"(M)); return d; }
 
 #define FWD_INF_BITS 0x7f800000u
 #define FWD_SAT16 ((uint32_t)NP_RUN_SAT << 16)
@@ -360,6 +365,9 @@ __global__ void __launch_bounds__(fwd_warps(CPL, T) * 32, T == 4 ? 2 : CPL <= 2 
         // ------------------------------------------------------------------------------------------------ one step
         auto step = [&](auto steady_tag, const uint32_t o, const bool first, uint32_t &nrow_buf, int &nrow_i) {
             constexpr bool STEADY = decltype(steady_tag)::value;
+            // steady block: edge and spare slots compute like interior ones and are overridden where read (ring store below).  Not at
+            // CPL 8: that form already runs at 255 registers, and the second ring store's extra live values cost it more spills
+            constexpr bool LEAN_EDGE = STEADY && CPL <= 4;
             float lMv[CPL], lDv[CPL]; uint32_t lMr[CPL];
             if (STEADY || !first) {
                 infd += 100.f;
@@ -438,7 +446,10 @@ __global__ void __launch_bounds__(fwd_warps(CPL, T) * 32, T == 4 ? 2 : CPL <= 2 
 #pragma unroll
             for (int k = 0; k < CPL; k++) {
                 Sv[k] = infd; Lv[k] = infd; Sb[k] = __uint_as_float(FWD_INF_BITS); Lb[k] = __uint_as_float(FWD_INF_BITS); Sr[k] = 0u; Lr[k] = 0u;
-                lwm[k] = in[k] ? (rw[k] & cb[k].w & 0x03f00000u) : 0u;    // one-hot LEN period vs the row's "tract present" bits, interior cells only
+                // one-hot LEN period vs the row's "tract present" bits, interior cells only -- except in a steady block, where the
+                // other slots (b_col 0, b_col 2r, spares) may evaluate a LEN candidate: their value is replaced by the edge value,
+                // their record by 0, their match run by 0, and their ring slot by the all-INF one below, so it is never read
+                lwm[k] = (LEAN_EDGE || in[k]) ? (rw[k] & cb[k].w & 0x03f00000u) : 0u;
                 any1 |= ca[k].w ^ empty_A; anyl |= lwm[k]; anyg |= cb[k].z;      // (votes on the unmasked words: slightly conservative)
             }
             // ---- SHR gather: descriptor 0 (largest period), then descriptor 1 if any lane has one
@@ -555,15 +566,17 @@ __global__ void __launch_bounds__(fwd_warps(CPL, T) * 32, T == 4 ? 2 : CPL <= 2 
                 }
                 // MAT = the first minimum in the order diag, INS, LEN, DEL, SHR (strict '<' chain of aln.pyx:585-592)
                 const float best = fmin3(fmin3(dg, Iv[k], Lv[k]), Dv[k], Sv[k]);
-                uint32_t p = ((uint32_t)T_SHR << 29) | (WIDE ? min(Sr[k], FWD_SAT16) : Sr[k]);
-                if (Dv[k] == best) p = (uint32_t)T_DEL << 29;
-                if (Lv[k] == best) p = ((uint32_t)T_LEN << 29) | (WIDE ? min(Lr[k], FWD_SAT16) : Lr[k]);
-                if (Iv[k] == best) p = (uint32_t)T_INS << 29;
+                uint32_t p = ((uint32_t)T_SHR << FWD_TYP_SH) | (WIDE ? min(Sr[k], FWD_SAT16) : Sr[k]);
+                if (Dv[k] == best) p = (uint32_t)T_DEL << FWD_TYP_SH;
+                if (Lv[k] == best) p = ((uint32_t)T_LEN << FWD_TYP_SH) | (WIDE ? min(Lr[k], FWD_SAT16) : Lr[k]);
+                if (Iv[k] == best) p = (uint32_t)T_INS << FWD_TYP_SH;
                 if (dg == best) p = pm;
-                p |= ((iext >> (31 - FWD_IE_BIT)) & (1u << FWD_IE_BIT)) | ((dext >> (31 - FWD_DE_BIT)) & (1u << FWD_DE_BIT));
+                // the flags are sign bits: IE stays where it is, DE moves down one bit, dext >> 1 written as the high word of
+                // dext * 2^31 so that it is an IMAD.HI on the FMA pipe, not a SHF on the busy ALU pipe.  Two LOP3s are left.
+                p = or_masked<1u << FWD_DE_BIT>(or_masked<1u << FWD_IE_BIT>(p, iext), __umulhi(dext, 1u << (FWD_DE_BIT + 1)));
                 if (!in[k]) p = 0u;
                 if (WIDE) {      // a LEN / SHR record whose run does not fit the field: the true run goes to the overflow list
-                    const uint32_t t3 = p >> 29, full = t3 == (uint32_t)T_LEN ? Lr[k] : Sr[k];
+                    const uint32_t t3 = (p >> FWD_TYP_SH) & 7u, full = t3 == (uint32_t)T_LEN ? Lr[k] : Sr[k];
                     if ((t3 == (uint32_t)T_LEN || t3 == (uint32_t)T_SHR) && full >= FWD_SAT16) {
                         const int e = atomicAdd(a.ovf_cnt, 1);
                         if (e < a.ovf_cap) a.ovf[e] = make_uint4((uint32_t)cid, dsh / ROWB, (uint32_t)((wt * 32 + lane) * CPL + k), full >> 16);
@@ -571,9 +584,17 @@ __global__ void __launch_bounds__(fwd_warps(CPL, T) * 32, T == 4 ? 2 : CPL <= 2 
                 }
                 Mr1[k] = dg == best && in[k] ? pm : 0u;                              // match run of this cell (0 unless TYP == MAT)
                 pk[k] = p;
-                // history ring: every slot writes; +INF unless the cell is interior
-                sts_slot(rowad + mypos[k], in[k] ? best : __uint_as_float(FWD_INF_BITS), Lb[k], in[k] ? Sb[k] : __uint_as_float(FWD_INF_BITS),
-                         __byte_perm(Lr[k], Sr[k], 0x7632));
+                // history ring: every slot writes; +INF unless the cell is interior.  The lean step stores every slot as computed and
+                // lets the few non-interior slots store again, all three values +INF (same lane, program order: the second store
+                // wins): one predicated STS instead of two FSELs per cell.  Their run word is then never used (a source whose
+                // values are +INF yields a +INF candidate whatever its run).
+                if (LEAN_EDGE) {
+                    sts_slot(rowad + mypos[k], best, Lb[k], Sb[k], __byte_perm(Lr[k], Sr[k], 0x7632));
+                    if (!in[k]) sts_slot(rowad + mypos[k], __uint_as_float(FWD_INF_BITS), __uint_as_float(FWD_INF_BITS), __uint_as_float(FWD_INF_BITS), 0u);
+                } else {
+                    sts_slot(rowad + mypos[k], in[k] ? best : __uint_as_float(FWD_INF_BITS), Lb[k], in[k] ? Sb[k] : __uint_as_float(FWD_INF_BITS),
+                             __byte_perm(Lr[k], Sr[k], 0x7632));
+                }
                 // EDGE (b_col 0 / 2r): every state INF*(b_row+1), TYP MAT, RUN 0 (aln.pyx:502-507).  Cells outside the chunk
                 // (aln.pyx:497-499) are never read by interior cells; they get the same harmless value.
                 Mv[k] = in[k] ? best : edgev;

@@ -1,4 +1,4 @@
-// traceback.cuh -- align() traceback (reference: src/aln.pyx:671-742) over the packed (TYP:3,RUN:13) records
+// traceback.cuh -- align() traceback (reference: src/aln.pyx:671-742) over the packed 16-bit records (common.cuh)
 // the forward kernel streamed to HBM.  Separate kernel, one walker thread per chunk: pointer chasing that
 // jumps RUN cells at a time (MAT-typed runs are diagonal steps re-evaluated as '='/'X' by base compare,
 // aln.pyx:727-736).  Ops are emitted right-aligned into the chunk's slice of the item's op scratch
@@ -52,7 +52,7 @@ __global__ void __launch_bounds__(TB_THREADS) traceback_kernel(const TracebackAr
         // records are stored per anti-diagonal in slot order: slot = column index mod NC (forward.cuh)
         const int d = i + j;
         const uint32_t rec = TB_REC(d, j);
-        const int typ = (int)(rec >> NP_REC_TYP);
+        const int typ = (int)((rec >> NP_REC_TYP) & 7u);
         int run = (int)(rec & (uint32_t)NP_RUN_SAT);
         if (typ == T_INS) {             // RUN = number of consecutive extensions up the column + 1 (aln.pyx:537-543)
             run = 1;
