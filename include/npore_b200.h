@@ -199,6 +199,28 @@ int64_t npore_bgzf_bound(int64_t n);   /* worst case: every member stored */
 int     npore_bgzf_compress(npore_bgzf *z, const uint8_t *in, int64_t n, uint8_t *out, int64_t out_capacity,
                             int64_t *out_len, float *device_ms /* may be NULL */);
 
+/* The BAM index (SAM spec section 5.2) contribution of the records compressed by the handle's last npore_bgzf_compress call,
+ * computed on the device from the input and member sizes still there.  rec_off[n_rec+1]: offset of every record's block_size
+ * field in that input, rec_off[n_rec] = its length (npore_bam_format_offsets).  base: file offset of the first member.
+ * Virtual offsets are (file offset of the member << 16 | offset inside it); the end of the input takes the form
+ * (base + compressed length) << 16, where the next member starts.  Records must be in (ref_id, pos) order and placed.
+ * Results, in host memory owned by the handle and valid until its next call, as rows of uint64:
+ *   chunks [n_chunks][4]   (ref_id, bin, vbeg, vend): one per run of consecutive records with the same (ref_id, bin),
+ *                          in (ref_id, bin, vbeg) order, chunks of one bin merged when the first ends in the BGZF member
+ *                          where the second begins (htslib's rule);
+ *   refs [n_refs][7]       (ref_id, first vbeg, last vend, mapped records, unmapped records, first 16 kb window, windows);
+ *   windows [n_windows]    the refs' windows in turn: the smallest vbeg of a mapped record overlapping it, ~0 where none does.
+ * Returns NPORE_ERR_BAD_ARG with error_bits set (1 unsorted, 2 inconsistent record bytes, 4 unplaced record) when the records
+ * cannot be indexed.  device_ms (may be NULL) receives the time of the index kernels. */
+typedef struct {
+    const uint64_t *chunks; int64_t n_chunks;
+    const uint64_t *refs; int64_t n_refs;
+    const uint64_t *windows; int64_t n_windows;
+    uint64_t error_bits;
+} npore_bai_lists;
+int     npore_bgzf_index(npore_bgzf *z, const int64_t *rec_off, int64_t n_rec, uint64_t base, npore_bai_lists *out,
+                         float *device_ms /* may be NULL */);
+
 int  npore_last_stats(const npore_ctx *ctx, npore_stats *stats);
 const char *npore_strerror(int code);
 const char *npore_last_error(const npore_ctx *ctx);   /* detail of the last failure (e.g. the CUDA error string) */

@@ -49,6 +49,15 @@ int      npore_bam_ref(const npore_bam *b, int32_t i, const char **name, int64_t
  * npore_bam_columns / npore_bam_gather); the next npore_bam_advance then only swaps it in.  max_bytes as for npore_bam_advance. */
 int      npore_bam_prefetch(npore_bam *b, int64_t max_bytes);
 int64_t  npore_bam_n_records(const npore_bam *b);
+/* Read only through a BAM index: after this call (before the first npore_bam_advance, once) windows hold only the records whose
+ * start virtual offset lies in one of the n chunks [vbeg, vend) (sorted, disjoint; bamio.read_bai(...).query gives them).  The
+ * reader seeks to vbeg >> 16, skips vbeg & 0xffff inflated bytes and inflates members until the last record that starts before
+ * vend is complete; members between chunks are not read.  n == 0: no record. */
+int      npore_bam_restrict(npore_bam *b, int64_t n, const uint64_t *vbeg, const uint64_t *vend);
+/* virtual offset of every record of the current window (file offset of its member << 16 | offset inside the member) */
+int      npore_bam_voffsets(const npore_bam *b, uint64_t *out);
+/* BGZF member bytes read from the file so far (the header's included) */
+int64_t  npore_bam_bytes_read(const npore_bam *b);
 
 /* one value per record of the current window, file order.  end = pos + reference span of the CIGAR (M D N = X); aln_len = SEQ length without
  * the soft-clipped ends (pysam query_alignment_sequence); n_cigar = CIGAR words once S and H are dropped (bam.pyx:59);
@@ -111,6 +120,15 @@ int64_t  npore_bam_format(int64_t n, int n_threads,
                           const uint32_t *rle, const int64_t *rle_off,
                           const uint8_t *seq_ascii, const uint8_t *qual_ascii, const int64_t *seq_off, const int32_t *has_qual,
                           const int32_t *hp, uint8_t *out, int64_t out_capacity);
+/* npore_bam_format that also fills rec_off[n+1]: the offset of record k's block_size field inside `out`, and the bytes written
+ * at [n].  These are the positions a BAM index needs (npore_bgzf_index, include/npore_b200.h). */
+int64_t  npore_bam_format_offsets(int64_t n, int n_threads,
+                                  const uint8_t *names, const int64_t *name_off, const int32_t *flag, const int32_t *ref_id,
+                                  const uint8_t *ref_names, const int64_t *ref_name_off, int32_t n_refs,
+                                  const int32_t *pos, const int32_t *end, const int32_t *mapq,
+                                  const uint32_t *rle, const int64_t *rle_off,
+                                  const uint8_t *seq_ascii, const uint8_t *qual_ascii, const int64_t *seq_off, const int32_t *has_qual,
+                                  const int32_t *hp, uint8_t *out, int64_t out_capacity, int64_t *rec_off);
 
 #ifdef __cplusplus
 }

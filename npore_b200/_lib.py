@@ -39,6 +39,11 @@ class Stats(C.Structure):
         return {k: getattr(self, k) for k, _ in self._fields_}
 
 
+class BaiLists(C.Structure):
+    _fields_ = [("chunks", C.c_void_p), ("n_chunks", C.c_int64), ("refs", C.c_void_p), ("n_refs", C.c_int64),
+                ("windows", C.c_void_p), ("n_windows", C.c_int64), ("error_bits", C.c_uint64)]
+
+
 class PileupBatch(C.Structure):
     _fields_ = [("n_ranges", C.c_int32), ("range_start", C.c_void_p), ("range_end", C.c_void_p),
                 ("ref_ascii", C.c_void_p), ("ref_off", C.c_void_p),
@@ -50,11 +55,12 @@ class PileupBatch(C.Structure):
 
 EXPORTS = ["npore_ctx_create", "npore_ctx_destroy", "npore_set_stream", "npore_count_chunks", "npore_upload", "npore_run", "npore_download",
            "npore_align_batch", "npore_get_np_info", "npore_get_np_info_batch", "npore_confusion_batch", "npore_last_stats", "npore_strerror", "npore_last_error", "npore_version",
-           "npore_bgzf_create", "npore_bgzf_destroy", "npore_bgzf_bound", "npore_bgzf_compress"]
+           "npore_bgzf_create", "npore_bgzf_destroy", "npore_bgzf_bound", "npore_bgzf_compress", "npore_bgzf_index"]
 
 IO_EXPORTS = ["npore_io_last_error", "npore_bam_open", "npore_bam_advance", "npore_bam_prefetch", "npore_bam_close", "npore_bam_header_text", "npore_bam_n_refs", "npore_bam_ref",
               "npore_bam_n_records", "npore_bam_columns", "npore_bam_gather", "npore_bam_gather_nib", "npore_sam_bound", "npore_sam_format", "npore_sam_format_fd",
-              "npore_bam_bound", "npore_bam_format"]
+              "npore_bam_bound", "npore_bam_format", "npore_bam_format_offsets",
+              "npore_bam_restrict", "npore_bam_voffsets", "npore_bam_bytes_read"]
 
 _lib = None
 
@@ -93,6 +99,7 @@ def lib():
         L.npore_bgzf_bound.restype = C.c_int64
         L.npore_bgzf_compress.argtypes = [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.POINTER(C.c_int64),
                                           C.POINTER(C.c_float)]
+        L.npore_bgzf_index.argtypes = [C.c_void_p, C.c_void_p, C.c_int64, C.c_uint64, C.POINTER(BaiLists), C.POINTER(C.c_float)]
         # include/npore_bamio.h
         vp = C.c_void_p
         L.npore_io_last_error.restype = C.c_char_p
@@ -110,6 +117,10 @@ def lib():
         L.npore_bam_n_records.restype = C.c_int64
         L.npore_bam_columns.argtypes = [vp] * 11
         L.npore_bam_prefetch.argtypes = [vp, C.c_int64]
+        L.npore_bam_restrict.argtypes = [vp, C.c_int64, vp, vp]
+        L.npore_bam_voffsets.argtypes = [vp, vp]
+        L.npore_bam_bytes_read.argtypes = [vp]
+        L.npore_bam_bytes_read.restype = C.c_int64
         L.npore_bam_gather.argtypes = [vp, C.c_int64, vp, C.c_int, vp, vp, vp, vp, vp, vp, vp, vp]
         L.npore_bam_gather_nib.argtypes = [vp, C.c_int64, vp, C.c_int, vp, vp, vp]
         L.npore_sam_bound.argtypes = [C.c_int64, vp, vp, vp, C.c_int64]
@@ -122,5 +133,7 @@ def lib():
         L.npore_bam_bound.restype = C.c_int64
         L.npore_bam_format.argtypes = L.npore_sam_format.argtypes
         L.npore_bam_format.restype = C.c_int64
+        L.npore_bam_format_offsets.argtypes = L.npore_sam_format.argtypes + [vp]
+        L.npore_bam_format_offsets.restype = C.c_int64
         _lib = L
     return _lib

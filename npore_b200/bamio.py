@@ -13,7 +13,9 @@
                                  inflate, record decode into flat arrays, batch SAM formatting) and never builds
                                  per-read Python objects; the pure-Python functions above remain as the tuple API.
                                  out_format="bam" writes the same records as BAM: batch BAM encoding on the host, BGZF
-                                 compression on the device (engine.BgzfCompressor).
+                                 compression on the device (engine.BgzfCompressor); index=True adds the .bai index,
+                                 computed on the device batch by batch (BgzfCompressor.index, BaiBuilder).
+  read_bai(path).query(..)       a BAM index and the chunks hts_itr_query would read for a region
                                  One batch pipeline (_realign_segments) serves both forms: the streamed windows of one
                                  device, and with devices=[...] one region shard per device (_realign_sharded).
 The GPU path is entered through npore_b200.engine (realign_bam) or npore_b200.bam.realign_reads (tuples).
@@ -187,9 +189,14 @@ class NativeBam:
 
     COLUMNS = ("ref_id", "pos", "end", "flag", "mapq", "aln_len", "n_cigar", "name_len", "hp", "has_qual")
 
-    def __init__(self, path, n_threads=0, window_bytes=0):
+    def __init__(self, path, n_threads=0, window_bytes=0, regions=None):
         """window_bytes == 0: the whole file is loaded now.  window_bytes > 0: nothing is loaded yet; every advance() call
-        loads the next ~window_bytes of (inflated) records, so files larger than memory stream through."""
+        loads the next ~window_bytes of (inflated) records, so files larger than memory stream through.
+        regions: [(contig, start, stop)]; when the file has a BAM index ({path}.bai, else {path without .bam}.bai, as htslib
+        looks them up), only the index chunks of the regions are read (npore_bam_restrict): the records are those whose start
+        lies in a chunk, a superset of the records overlapping the regions, in file order.  An index older than the BAM is not
+        used (the whole file is read then); a malformed one raises ValueError.  self.index: the index file used, or None;
+        self.bytes_read: compressed bytes read so far."""
         from ._lib import lib
         self._L = lib()
         h = C.c_void_p()
@@ -209,8 +216,25 @@ class NativeBam:
         self.n = 0
         for k in self.COLUMNS:
             setattr(self, k, np.zeros(0, np.int32))
+        self.index = find_index(path) if regions else None
+        if self.index is not None:
+            ch = region_chunks(read_bai(self.index), self.refs, regions)
+            beg, end = np.ascontiguousarray(ch[:, 0]), np.ascontiguousarray(ch[:, 1])
+            if self._L.npore_bam_restrict(h, len(ch), beg.ctypes.data, end.ctypes.data):
+                raise ValueError(f"{self.index}: {self._L.npore_io_last_error().decode()}")
         if not self.window_bytes:
             self.advance()
+
+    @property
+    def bytes_read(self):
+        """BGZF member bytes read from the file so far."""
+        return int(self._L.npore_bam_bytes_read(self._h))
+
+    def voffsets(self):
+        """Virtual offset of every record of the current window (uint64)."""
+        out = np.zeros(max(self.n, 1), np.uint64)
+        self._L.npore_bam_voffsets(self._h, out.ctypes.data)
+        return out[:self.n]
 
     def advance(self):
         """Load the next window; returns the number of records in it (0 at end of file)."""
@@ -279,11 +303,13 @@ class NativeBam:
         return o
 
 
-def format_sam(bam, sel, g, rle, rle_off, n_threads=0, cols=None, fd=None, offset=0, binary=False):
+def format_sam(bam, sel, g, rle, rle_off, n_threads=0, cols=None, fd=None, offset=0, binary=False, offsets=False):
     """bam.pyx:83 for the selected records as one bytes-like block (npore_sam_format).  cols: the records' column values
     taken earlier (dict of int32 arrays: flag ref_id pos end mapq has_qual hp) when the reader has moved on since.
     fd: also append the block to that file descriptor at `offset` while formatting (npore_sam_format_fd).
-    binary: the same records as uncompressed BAM records instead (npore_bam_format; fd must be None)."""
+    binary: the same records as uncompressed BAM records instead (npore_bam_format; fd must be None).
+    offsets (with binary): returns (block, rec_off) with every record's offset in the block and the block length at the end
+    (npore_bam_format_offsets)."""
     L = bam._L
     names = "".join(n for n, _ in bam.refs).encode()
     rn_off = np.concatenate(([0], np.cumsum([len(n.encode()) for n, _ in bam.refs], dtype=np.int64)))
@@ -306,17 +332,59 @@ def format_sam(bam, sel, g, rle, rle_off, n_threads=0, cols=None, fd=None, offse
             rn.ctypes.data, rn_off.ctypes.data, len(bam.refs), pos.ctypes.data, end.ctypes.data, mapq.ctypes.data,
             rle.ctypes.data if len(rle) else None, rle_off.ctypes.data, g["seq_ascii"].ctypes.data, qual.ctypes.data,
             g["seq_off"].ctypes.data, hq.ctypes.data, hp.ctypes.data, out.ctypes.data, cap)
-    if binary:
+    rec_off = None
+    if binary and offsets:
+        rec_off = np.zeros(n + 1, np.int64)
+        got = L.npore_bam_format_offsets(*args, rec_off.ctypes.data)
+    elif binary:
         got = L.npore_bam_format(*args)
     else:
         got = L.npore_sam_format(*args) if fd is None else L.npore_sam_format_fd(*args, int(fd), int(offset))
     if got < 0:
         raise RuntimeError(L.npore_io_last_error().decode())
-    return out[:got]
+    return (out[:got], rec_off) if rec_off is not None else out[:got]
 
 
 def take_columns(bam, sel):
     return {k: np.ascontiguousarray(getattr(bam, k)[sel], dtype=np.int32) for k in ("flag", "ref_id", "pos", "end", "mapq", "has_qual", "hp")}
+
+
+def find_index(path):
+    """The BAM index of path that htslib would use ({path}.bai, then {path without .bam}.bai), if it is not older than the BAM."""
+    cands = [f"{path}.bai"] + ([f"{path[:-4]}.bai"] if path.endswith(".bam") else [])
+    for c in cands:
+        if os.path.exists(c):
+            return c if os.path.getmtime(c) >= os.path.getmtime(path) else None
+    return None
+
+
+def region_chunks(bai, refs, regions):
+    """The union of the index chunks of every region, sorted and merged: uint64 array (k, 2)."""
+    names = {n: k for k, (n, _) in enumerate(refs)}
+    got = [bai.query(names[c], int(a), int(b)) for c, a, b in regions if c in names]
+    c = np.concatenate(got) if got else np.zeros((0, 2), np.uint64)
+    c = c[np.argsort(c[:, 0], kind="stable")]
+    out = []
+    for b, e in c.tolist():
+        if out and b <= out[-1][1]:
+            out[-1][1] = max(out[-1][1], e)
+        else:
+            out.append([b, e])
+    return np.array(out, np.uint64).reshape(-1, 2)
+
+
+def _in_coordinate_order(bam, segments):
+    """segments, checked to select records in (ref_id, pos) order: an index needs a sorted file.  A read overlapping two regions
+    is selected once per region (bam.pyx:27-28), and its second copy would follow reads that start after it."""
+    last = (-1, -1)
+    for ctg, sel in segments:
+        pos = bam.pos[sel]
+        first = (int(bam.ref_id[sel[0]]), int(pos[0]))
+        if first < last or (len(pos) > 1 and bool((pos[1:] < pos[:-1]).any())):
+            raise ValueError(f"index=True: the records selected in {ctg} are not in coordinate order after the earlier ones (a read "
+                             "overlapping two regions is written once per region, or the input is not sorted); the output cannot be indexed")
+        last = (first[0], int(pos[-1]))
+        yield ctg, sel
 
 
 def select_reads(bam, regions=None, max_reads=0):
@@ -334,6 +402,213 @@ def select_reads(bam, regions=None, max_reads=0):
         kept += len(sel)
         if len(sel):
             yield ctg, sel
+
+
+# ------------------------------------------------------------------------------------------------ BAM index (SAM spec 5.2)
+BAI_MAX_REF = (1 << 29) - 1             # the BAI binning scheme covers positions below 2^29
+_PSEUDO_BIN = 37450
+_UNSET = np.uint64(0xFFFFFFFFFFFFFFFF)
+
+
+def reg2bins(beg, end):
+    """Bins that may hold records overlapping [beg, end) (hts_reg2bins, 14-bit windows, 5 levels)."""
+    beg, end = max(int(beg), 0), min(int(end), 1 << 29)
+    if end <= beg:
+        return []
+    end -= 1
+    out = []
+    for off, shift in ((0, 29), (1, 26), (9, 23), (73, 20), (585, 17), (4681, 14)):
+        out.extend(range(off + (beg >> shift), off + (end >> shift) + 1))
+    return out
+
+
+class BaiBuilder:
+    """Folds the index lists of BgzfCompressor.index (one per written batch, in file order) into a .bai file.  Lists are kept
+    as they arrive (they are small: a chunk per run of records with one bin, a few windows per batch) and folded once in
+    to_bytes(): the chunks of one bin are appended in file order and merged when the previous one ends in the BGZF member
+    where the next begins; the first value set in a 16 kb window wins; windows no record overlaps take the reference's first
+    offset before its first record and the previous window's offset after it (htslib's update_loff).  Bins are written in
+    ascending order, the pseudo-bin 37450 (first / last offset, mapped / unmapped counts) last."""
+
+    def __init__(self, n_refs):
+        self.n_refs = int(n_refs)
+        self.batches = []                 # (lists, shift): offsets are lists' + shift << 16
+
+    def add(self, lists, shift=0):
+        self.batches.append((lists, int(shift)))
+
+    def extend(self, other, shift):
+        """Appends another builder's lists (e.g. a shard's, relative to its part file) whose file starts at byte `shift`."""
+        self.batches.extend((lists, sh + int(shift)) for lists, sh in other.batches)
+
+    def to_bytes(self):
+        chunks, refs, wins = [], [], []
+        for lists, shift in self.batches:
+            sh = np.uint64(shift << 16)
+            c = lists["chunks"].astype(np.uint64, copy=True)
+            c[:, 2:] += sh
+            r = lists["refs"].astype(np.uint64, copy=True)
+            r[:, 1:3] += sh
+            w = lists["windows"].astype(np.uint64, copy=True)
+            w[w != _UNSET] += sh
+            at = 0
+            for ref, _, _, _, _, wf, nw in r.tolist():        # a batch's windows, reference by reference
+                if nw:
+                    wins.append((ref, wf, w[at:at + nw]))
+                at += nw
+            chunks.append(c); refs.append(r)
+        c = np.concatenate(chunks) if chunks else np.zeros((0, 4), np.uint64)
+        r = np.concatenate(refs) if refs else np.zeros((0, 7), np.uint64)
+        c = c[np.lexsort((c[:, 1], c[:, 0]))]                 # stable: file order within (ref_id, bin)
+        start = np.ones(len(c), bool)
+        start[1:] = (c[1:, 0] != c[:-1, 0]) | (c[1:, 1] != c[:-1, 1]) | ((c[:-1, 3] >> np.uint64(16)) < (c[1:, 2] >> np.uint64(16)))
+        first = np.flatnonzero(start)
+        last = np.r_[first[1:] - 1, len(c) - 1].astype(np.int64)
+        merged = np.stack([c[first, 0], c[first, 1], c[first, 2], c[last, 3]], axis=1) if len(c) else np.zeros((0, 4), np.uint64)
+        lin = {}
+        for ref, wf, vals in wins:
+            cur = lin.setdefault(ref, np.zeros(0, np.uint64))
+            need = wf + len(vals)
+            if len(cur) < need:
+                cur = lin[ref] = np.concatenate([cur, np.full(need - len(cur), _UNSET, np.uint64)])
+            seg = cur[wf:need]
+            fill = (seg == _UNSET) & (vals != _UNSET)                 # the first value set wins
+            seg[fill] = vals[fill]
+        out = [b"BAI\1", struct.pack("<i", self.n_refs)]
+        bounds = np.searchsorted(merged[:, 0], np.arange(self.n_refs + 1, dtype=np.uint64)) if len(merged) else np.zeros(self.n_refs + 1, np.int64)
+        for ref in range(self.n_refs):
+            rows = r[r[:, 0] == ref]
+            if not len(rows):
+                out.append(struct.pack("<ii", 0, 0))
+                continue
+            m = merged[bounds[ref]:bounds[ref + 1]]
+            bins, at, cnt = np.unique(m[:, 1], return_index=True, return_counts=True)
+            out.append(struct.pack("<i", len(bins) + 1))
+            for b, a, k in zip(bins.tolist(), at.tolist(), cnt.tolist()):
+                out.append(struct.pack("<Ii", b, k) + np.ascontiguousarray(m[a:a + k, 2:4]).astype("<u8").tobytes())
+            beg, end = int(rows[0, 1]), int(rows[-1, 2])
+            out.append(struct.pack("<IiQQQQ", _PSEUDO_BIN, 2, beg, end, int(rows[:, 3].sum()), int(rows[:, 4].sum())))
+            li = lin.get(ref, np.zeros(0, np.uint64)).copy()
+            prev = np.uint64(beg)
+            for k in range(len(li)):                                   # update_loff
+                if li[k] == _UNSET:
+                    li[k] = prev
+                prev = li[k]
+            out.append(struct.pack("<i", len(li)) + li.astype("<u8").tobytes())
+        out.append(struct.pack("<Q", 0))                               # n_no_coor: every record written has a reference
+        return b"".join(out)
+
+    def write(self, path):
+        """Writes the index atomically (a temporary file renamed over `path`)."""
+        tmp = f"{path}.tmp{os.getpid()}"
+        try:
+            with open(tmp, "wb") as fh:
+                fh.write(self.to_bytes())
+            os.replace(tmp, path)
+        finally:
+            with contextlib.suppress(FileNotFoundError):
+                os.remove(tmp)
+
+
+class Bai:
+    """A parsed .bai file (read_bai): refs[i] = (bins {bin: uint64 array (k, 2) of (vbeg, vend)}, linear uint64 array,
+    meta (first vbeg, last vend, mapped, unmapped) or None)."""
+
+    def __init__(self, refs, n_no_coor):
+        self.refs, self.n_no_coor = refs, n_no_coor
+
+    def query(self, ref_id, beg, end):
+        """Chunks (uint64 array (k, 2) of vbeg, vend; sorted, overlapping ones merged) that hold every record of reference
+        ref_id overlapping [beg, end) -- what htslib's hts_itr_query reads: the chunks of reg2bins(beg, end), less those ending
+        before the linear-index offset of window beg >> 14."""
+        if not 0 <= ref_id < len(self.refs):
+            return np.zeros((0, 2), np.uint64)
+        bins, lin, _ = self.refs[ref_id]
+        got = [bins[b] for b in reg2bins(beg, end) if b in bins]
+        if not got:
+            return np.zeros((0, 2), np.uint64)
+        c = np.concatenate(got)
+        w = max(int(beg), 0) >> 14
+        min_off = lin[min(w, len(lin) - 1)] if len(lin) else np.uint64(0)
+        c = c[c[:, 1] > min_off]
+        c = c[np.argsort(c[:, 0], kind="stable")]
+        out = []
+        for b, e in c.tolist():
+            if out and b <= out[-1][1]:
+                out[-1][1] = max(out[-1][1], e)
+            else:
+                out.append([b, e])
+        return np.array(out, np.uint64).reshape(-1, 2)
+
+
+def read_bai(path):
+    """Parses a BAM index (SAM spec 5.2) into a Bai.  A malformed file raises ValueError naming it."""
+    data = open(path, "rb").read()
+    p = 0
+
+    def take(fmt):
+        nonlocal p
+        n = struct.calcsize(fmt)
+        if p + n > len(data):
+            raise ValueError(f"{path}: truncated BAM index")
+        v = struct.unpack_from(fmt, data, p)
+        p += n
+        return v
+
+    if data[:4] != b"BAI\1":
+        raise ValueError(f"{path}: not a BAM index (bad magic)")
+    p = 4
+    (n_ref,) = take("<i")
+    if n_ref < 0:
+        raise ValueError(f"{path}: negative reference count")
+    refs = []
+    for _ in range(n_ref):
+        (n_bin,) = take("<i")
+        if n_bin < 0:
+            raise ValueError(f"{path}: negative bin count")
+        bins, meta = {}, None
+        for _ in range(n_bin):
+            b, n_chunk = take("<Ii")
+            if n_chunk < 0 or p + 16 * n_chunk > len(data):
+                raise ValueError(f"{path}: truncated BAM index")
+            c = np.frombuffer(data, "<u8", 2 * n_chunk, p).reshape(-1, 2).astype(np.uint64)
+            p += 16 * n_chunk
+            if b == _PSEUDO_BIN:
+                if n_chunk != 2:
+                    raise ValueError(f"{path}: pseudo-bin {_PSEUDO_BIN} without two chunks")
+                meta = tuple(int(x) for x in c.reshape(-1))
+            elif b > _PSEUDO_BIN:
+                raise ValueError(f"{path}: bin {b} out of range")
+            else:
+                bins[b] = c
+        (n_intv,) = take("<i")
+        if n_intv < 0 or p + 8 * n_intv > len(data):
+            raise ValueError(f"{path}: truncated BAM index")
+        lin = np.frombuffer(data, "<u8", n_intv, p).astype(np.uint64)
+        p += 8 * n_intv
+        refs.append((bins, lin, meta))
+    n_no_coor = take("<Q")[0] if p + 8 <= len(data) else None
+    if p != len(data):
+        raise ValueError(f"{path}: trailing bytes after the BAM index")
+    return Bai(refs, n_no_coor)
+
+
+def _check_indexable(refs, regions):
+    """index=True: the references must fit the BAI binning, and regions must be in header order without overlaps (a read that
+    still overlaps two of them is caught later, by _in_coordinate_order)."""
+    for name, length in refs:
+        if length > BAI_MAX_REF:
+            raise ValueError(f"index=True: contig {name} is {length} bp; a BAI index covers at most {BAI_MAX_REF} bp (CSI is not supported)")
+    order = {name: k for k, (name, _) in enumerate(refs)}
+    prev = None
+    for ctg, start, stop in regions or []:
+        if ctg not in order:
+            continue
+        key = (order[ctg], int(start), int(stop))
+        if prev is not None and (key[0] < prev[0] or (key[0] == prev[0] and key[1] < prev[2])):
+            raise ValueError(f"index=True: regions must be in header contig order and must not overlap ({ctg}:{start}-{stop} follows "
+                             f"{refs[prev[0]][0]}:{prev[1]}-{prev[2]}); the output would not be sorted")
+        prev = key
 
 
 def _pipeline(sub, npt, n_inflight, device=None):
@@ -379,14 +654,17 @@ def _read_loads(bam, sel, max_b_rows=20000, r=30):
     return (ops + -(-ops // (max_b_rows - 1))) * (2 * r + 1)
 
 
-def _realign_segments(bam, segments, fa, pipe, open_out, tm, n_threads, nt_text, max_batch_ops, n_inflight, mark, t0, compressor=None):
+def _realign_segments(bam, segments, fa, pipe, open_out, tm, n_threads, nt_text, max_batch_ops, n_inflight, mark, t0, compressor=None,
+                      bai=None):
     """The three-stage pipeline over (contig, record indices) segments, which may be produced lazily: gather batch k+1 while
     batch k is on the GPU and a writer thread formats batch k-1 and appends it to the file descriptor that open_out() returns.
     The writer calls open_out(z) before its first batch and writes from the descriptor's current size on.  compressor: None
     writes SAM text (z is None); otherwise a callable that returns the writer's BgzfCompressor z, and every batch is written as
     BAM records compressed into BGZF members (tm["compress"]: seconds in the compressor).  The descriptor must
     not be in append mode: Linux ignores the offset of a pwrite on an append-mode descriptor, and the formatter threads place
-    their slices by offset.  Records are written in segment order and counted into cfg.counter batch by batch.  n_threads:
+    their slices by offset.  bai (with a compressor): a BaiBuilder that receives every batch's index lists, computed on the
+    device right after the batch is written (z.index, tm["index"]: seconds, tm["index_device_ms"]: its kernel milliseconds); the
+    records must then be selected in coordinate order (ValueError otherwise).  Records are written in segment order and counted into cfg.counter batch by batch.  n_threads:
     threads of the nibble / CIGAR gathers and of formatting; nt_text: threads of the SAM-text gather that runs beside the
     GPU.  tm receives seconds per phase, mark(event) a trace event per step (GPU times in them count from perf_counter() = t0).
     Returns the records written."""
@@ -426,13 +704,19 @@ def _realign_segments(bam, segments, fa, pipe, open_out, tm, n_threads, nt_text,
                     mark("formatted + written")
                     tm["gpu_wait"] += t2 - t1; tm["format"] += t3 - t2; tm["write"] += time.perf_counter() - t3
                 else:
-                    raw = format_sam(bam, None, g, res.rle, res.rle_off[:n + 1], n_threads, cols=cols, binary=True)
+                    raw = format_sam(bam, None, g, res.rle, res.rle_off[:n + 1], n_threads, cols=cols, binary=True, offsets=bai is not None)
+                    raw, rec_off = raw if bai is not None else (raw, None)
                     t3 = time.perf_counter()
                     blob = z.compress(raw)
                     t4 = time.perf_counter()
-                    end = _write_all(fd, blob, end)
+                    start, end = end, _write_all(fd, blob, end)
+                    t5 = time.perf_counter()
+                    if bai is not None:
+                        bai.add(z.index(rec_off, start))
+                        tm["index"] += time.perf_counter() - t5
+                        tm["index_device_ms"] += getattr(z, "last_index_ms", 0.0)
                     mark("formatted + written")
-                    tm["gpu_wait"] += t2 - t1; tm["format"] += t3 - t2; tm["compress"] += t4 - t3; tm["write"] += time.perf_counter() - t4
+                    tm["gpu_wait"] += t2 - t1; tm["format"] += t3 - t2; tm["compress"] += t4 - t3; tm["write"] += t5 - t4
                 state["written"] += n
                 with cfg.counter.get_lock():
                     cfg.counter.value += n
@@ -443,8 +727,13 @@ def _realign_segments(bam, segments, fa, pipe, open_out, tm, n_threads, nt_text,
 
     if compressor is not None:
         tm.setdefault("compress", 0.0)
+    if bai is not None:
+        tm.setdefault("index", 0.0)
+        tm.setdefault("index_device_ms", 0.0)
     retire = threading.Thread(target=retire_loop, daemon=True)
     retire.start()
+    if bai is not None:
+        segments = _in_coordinate_order(bam, segments)
     try:
         for ctg, sel in segments:
             contig = fa[ctg]
@@ -480,7 +769,8 @@ def _realign_segments(bam, segments, fa, pipe, open_out, tm, n_threads, nt_text,
     return state["written"]
 
 
-def _realign_sharded(bam, fa, pipes, devices, open_out, regions, max_reads, max_batch_ops, n_threads, n_inflight, tm, mark, t0, ext="sam"):
+def _realign_sharded(bam, fa, pipes, devices, open_out, regions, max_reads, max_batch_ops, n_threads, n_inflight, tm, mark, t0, ext="sam",
+                     bai=None):
     """realign.py:75-115 on several GPUs of one host (SURVEY.md 8(e)): the coordinate-sorted reads are cut into len(devices)
     contiguous genomic regions of equal cell-update load (the reference's own unit of distribution is the region,
     util.py:44-93 / bam.pyx:27-28); every region is an independent ingest -> GPU -> SAM-text pipeline on its own device (no
@@ -488,12 +778,15 @@ def _realign_sharded(bam, fa, pipes, devices, open_out, regions, max_reads, max_
     byte-identical to the single-GPU output.  Region 0 writes into the output itself (open_out), the others into part files,
     which are removed whether the call succeeds or fails.  ext "bam": every shard compresses its records on its own device and
     the part files hold BGZF members only (no header, no EOF block), so their concatenation is valid BGZF.  tm: per phase, summed over the shards, plus
-    'shards': [{device, reads, cell_updates, seconds}] and 'concat' seconds."""
+    'shards': [{device, reads, cell_updates, seconds}] and 'concat' seconds.  bai: a BaiBuilder; every shard indexes its records
+    with offsets in its own file, and shard g's lists join bai shifted by the offset its part file is copied to."""
     from .scheduler import cut_balanced
     tm.setdefault("concat", 0.0)
     t1 = time.perf_counter()
     G = len(devices)
     segs = list(select_reads(bam, regions, max_reads))
+    if bai is not None:
+        segs = list(_in_coordinate_order(bam, segs))
     loads = [_read_loads(bam, sel) for _, sel in segs]
     total = float(sum(int(x.sum()) for x in loads))
     # contiguous cuts of the (contig, start)-ordered read list at equal cumulative load
@@ -513,15 +806,16 @@ def _realign_sharded(bam, fa, pipes, devices, open_out, regions, max_reads, max_
     opens = [open_out] + [lambda z, p=p: os.open(p, os.O_WRONLY | os.O_CREAT | os.O_TRUNC, 0o644) for p in parts[1:]]
     nt = max(1, (n_threads or os.cpu_count() or 1) // G)
     results = [None] * G
-    phases = ("gather", "gpu_wait", "format", "write") + (("compress",) if ext == "bam" else ())
+    phases = ("gather", "gpu_wait", "format", "write") + (("compress",) if ext == "bam" else ()) + (("index", "index_device_ms") if bai is not None else ())
     shard_tm = [{k: 0.0 for k in phases} for _ in range(G)]
+    shard_bai = [BaiBuilder(len(bam.refs)) if bai is not None else None for _ in range(G)]
 
     def shard_main(g):
         t2 = time.perf_counter()
         try:
             comp = (lambda: _compressor(devices[g], g)) if ext == "bam" else None
             n = _realign_segments(bam, shard_segs[g], fa, pipes[g], opens[g], shard_tm[g], nt, nt, max_batch_ops, n_inflight, mark, t0,
-                                  compressor=comp)
+                                  compressor=comp, bai=shard_bai[g])
             results[g] = (n, time.perf_counter() - t2, None)
         except Exception as e:      # noqa: BLE001
             results[g] = (0, time.perf_counter() - t2, e)
@@ -539,7 +833,11 @@ def _realign_sharded(bam, fa, pipes, devices, open_out, regions, max_reads, max_
         dst = os.open(out, os.O_WRONLY)                             # host gather: region order = coordinate order
         try:
             end = os.fstat(dst).st_size
-            for part in parts[1:]:
+            if bai is not None:
+                bai.extend(shard_bai[0], 0)                         # shard 0 wrote after the header: absolute offsets already
+            for g, part in enumerate(parts[1:], 1):
+                if bai is not None:
+                    bai.extend(shard_bai[g], end)
                 with open(part, "rb") as src:
                     left = os.fstat(src.fileno()).st_size
                     try:                                            # in-kernel copy (no bounce through user space)
@@ -591,7 +889,7 @@ def _keep_freed_buffers_mapped():
 
 
 def realign_bam(bam_fn, fasta, out_prefix=None, regions=None, max_reads=0, argv=None, max_batch_ops=64_000_000, n_threads=0,
-                timings=None, window_bytes=16 << 20, n_inflight=3, devices=None, out_format="sam"):
+                timings=None, window_bytes=16 << 20, n_inflight=3, devices=None, out_format="sam", index=False):
     """realign.py:75-115 without pysam / Pool: header, ingest, GPU realignment, records appended in input order
     (= coordinate order for a sorted BAM, which is what the header claims).  Returns the number of records written.
     Flat arrays all the way, as a pipeline: the reader streams the file in windows of ~window_bytes of inflated records
@@ -603,9 +901,18 @@ def realign_bam(bam_fn, fasta, out_prefix=None, regions=None, max_reads=0, argv=
     (_realign_sharded; the whole file is loaded, no streaming).
     out_format: "sam" writes {out_prefix}.sam; "bam" writes the same header and records to {out_prefix}.bam as BAM, each batch
     encoded on the host and compressed into BGZF members on the batch's device, with one BGZF EOF block at the end; timings then
-    also has "compress", the seconds spent in the compressor."""
+    also has "compress", the seconds spent in the compressor.  An index of an earlier run beside the BAM output is removed.
+    index=True (BAM only): also writes the BAM index {out_prefix}.bam.bai, computed on the device batch by batch
+    (BgzfCompressor.index) and written once the BAM is complete; timings then has "index", the seconds spent on it, and
+    "index_device_ms", its kernel time.  Regions must then be in header contig order without overlaps, and no contig may be
+    longer than 2^29 - 1 bp (ValueError before any work); a read selected by two regions makes the output unsorted and raises
+    ValueError when it is met.  A call that fails leaves no index.
+    regions and an index of the input (NativeBam): only the index chunks of the regions are read and inflated; the output is the
+    same as without the index."""
     if out_format not in ("sam", "bam"):
         raise ValueError(f"out_format must be 'sam' or 'bam', not {out_format!r}")
+    if index and out_format != "bam":
+        raise ValueError("index=True needs out_format='bam'")
     from .bam import _tables
     tm = timings if timings is not None else {}
     for k in ("open", "gather", "gpu_wait", "format", "write"):
@@ -624,9 +931,17 @@ def realign_bam(bam_fn, fasta, out_prefix=None, regions=None, max_reads=0, argv=
     # several regions are served region by region (bam.pyx:27-28), and region shards are cut from every record's span: both
     # need the whole file at hand
     streaming = len(devices) == 1 and not (regions and len(regions) > 1)
-    bam = NativeBam(bam_fn, n_threads, window_bytes=window_bytes if streaming else 0)
+    bam = NativeBam(bam_fn, n_threads, window_bytes=window_bytes if streaming else 0, regions=regions)
     mark("bam open")
     out = f"{cfg.args.out_prefix}.{out_format}"
+    bai = None
+    if index:
+        try:
+            _check_indexable(bam.refs, regions)
+        except ValueError:
+            bam.close()
+            raise
+        bai = BaiBuilder(len(bam.refs))
 
     def open_out(z):
         # called by the writer thread: the header (and the truncation of a previous output: ~2 ms for a 60 MB file) is written
@@ -636,6 +951,8 @@ def realign_bam(bam_fn, fasta, out_prefix=None, regions=None, max_reads=0, argv=
         else:
             if os.path.dirname(out):
                 os.makedirs(os.path.dirname(out), exist_ok=True)
+            with contextlib.suppress(FileNotFoundError):
+                os.remove(f"{out}.bai")                 # an earlier run's index does not describe this file
             with open(out, "wb") as fh:
                 fh.write(z.compress(bam_header(bam.refs, argv)))
         mark("header written")
@@ -649,7 +966,7 @@ def realign_bam(bam_fn, fasta, out_prefix=None, regions=None, max_reads=0, argv=
         mark("opened")
         if len(devices) > 1:
             written = _realign_sharded(bam, fa, pipes, devices, open_out, regions, max_reads, max_batch_ops, n_threads, n_inflight,
-                                       tm, mark, t0, ext=out_format)
+                                       tm, mark, t0, ext=out_format, bai=bai)
         else:
             def segments():
                 kept = 0
@@ -672,13 +989,18 @@ def realign_bam(bam_fn, fasta, out_prefix=None, regions=None, max_reads=0, argv=
             nt_text = max(1, (n_threads or os.cpu_count() or 1) - int(os.environ.get("NPORE_SPARE_CORES", "3")))
             comp = (lambda: _compressor(devices[0], 0)) if out_format == "bam" else None
             written = _realign_segments(bam, segments(), fa, pipes[0], open_out, tm, n_threads, nt_text, max_batch_ops, n_inflight, mark, t0,
-                                        compressor=comp)
+                                        compressor=comp, bai=bai)
         if out_format == "bam":
             fd = os.open(out, os.O_WRONLY)
             try:
                 _write_all(fd, BGZF_EOF, os.fstat(fd).st_size)
             finally:
                 os.close(fd)
+        if bai is not None:
+            t1 = time.perf_counter()
+            bai.write(f"{out}.bai")
+            tm["index"] += time.perf_counter() - t1
+            mark("index written")
     finally:
         bam.close()
     mark("closed")

@@ -30,6 +30,7 @@
 #include "finish.cuh"
 #include "confusion.cuh"
 #include "bgzf.cuh"
+#include "bai.cuh"
 
 namespace {
 
@@ -135,6 +136,10 @@ struct npore_bgzf {
     cudaStream_t stream = nullptr;
     cudaEvent_t ev[2]{};
     DevBuf d_in, d_tok, d_slots, d_sizes, d_out, d_total;
+    int64_t last_n = 0;                  // input bytes of the last npore_bgzf_compress (still in d_in, its member sizes in d_sizes)
+    // npore_bgzf_index
+    DevBuf d_rec_off, d_moff, d_recs, d_chunks, d_sorted, d_segs, d_out_chunks, d_out_refs, d_win, d_counts;
+    HostBuf h_counts, h_lists;
     ~npore_bgzf()
     {
         for (auto &e : ev) if (e) cudaEventDestroy(e);
@@ -1017,6 +1022,7 @@ int npore_bgzf_compress(npore_bgzf *z, const uint8_t *in, int64_t n, uint8_t *ou
 {
     if (!z || n < 0 || !out_len || (n && (!in || !out))) return NPORE_ERR_BAD_ARG;
     *out_len = 0;
+    z->last_n = 0;
     if (device_ms) *device_ms = 0.0f;
     if (!n) return NPORE_OK;
     const int64_t members = (n + BGZF_BLOCK - 1) / BGZF_BLOCK;
@@ -1053,6 +1059,77 @@ int npore_bgzf_compress(npore_bgzf *z, const uint8_t *in, int64_t n, uint8_t *ou
         return rc;
     if (device_ms && (rc = check(cudaEventElapsedTime(device_ms, z->ev[0], z->ev[1])))) return rc;
     *out_len = total;
+    z->last_n = n;
+    return NPORE_OK;
+}
+
+int npore_bgzf_index(npore_bgzf *z, const int64_t *rec_off, int64_t n_rec, uint64_t base, npore_bai_lists *out, float *device_ms)
+{
+    if (!z || !out || n_rec < 0 || (n_rec && !rec_off)) return NPORE_ERR_BAD_ARG;
+    std::memset(out, 0, sizeof(*out));
+    if (device_ms) *device_ms = 0.0f;
+    if (!n_rec) return NPORE_OK;
+    const int64_t n_in = z->last_n, members = (n_in + BGZF_BLOCK - 1) / BGZF_BLOCK;
+    if (rec_off[0] != 0 || rec_off[n_rec] != n_in) return NPORE_ERR_BAD_ARG;      // not the records of the last compressed input
+    auto check = [&](cudaError_t e) {
+        if (e == cudaSuccess) return NPORE_OK;
+        cudaGetLastError();
+        return e == cudaErrorMemoryAllocation ? NPORE_ERR_OOM : NPORE_ERR_CUDA;
+    };
+    int rc;
+    if ((rc = check(cudaSetDevice(z->device))) ||
+        (rc = check(z->d_rec_off.ensure((size_t)(n_rec + 1) * sizeof(int64_t)))) ||
+        (rc = check(z->d_moff.ensure((size_t)(members + 1) * sizeof(uint64_t)))) ||
+        (rc = check(z->d_recs.ensure((size_t)n_rec * sizeof(bai::Rec)))) ||
+        (rc = check(z->d_chunks.ensure((size_t)n_rec * sizeof(bai::Chunk)))) ||
+        (rc = check(z->d_sorted.ensure((size_t)n_rec * sizeof(bai::Chunk)))) ||
+        (rc = check(z->d_segs.ensure((size_t)n_rec * sizeof(bai::Seg)))) ||
+        (rc = check(z->d_out_chunks.ensure((size_t)n_rec * 4 * sizeof(uint64_t)))) ||
+        (rc = check(z->d_out_refs.ensure((size_t)n_rec * 7 * sizeof(uint64_t)))) ||
+        (rc = check(z->d_counts.ensure(4 * sizeof(uint64_t)))) ||
+        (rc = check(z->h_counts.ensure(4 * sizeof(uint64_t)))))
+        return rc;
+    unsigned long long *counts = z->d_counts.as<unsigned long long>();
+    if ((rc = check(cudaMemcpyAsync(z->d_rec_off.p, rec_off, (size_t)(n_rec + 1) * sizeof(int64_t), cudaMemcpyHostToDevice, z->stream))) ||
+        (rc = check(cudaMemsetAsync(counts, 0, 4 * sizeof(uint64_t), z->stream))) ||
+        (rc = check(cudaEventRecord(z->ev[0], z->stream))))
+        return rc;
+    bai::bai_member_kernel<<<1, BAI_THREADS, 0, z->stream>>>(z->d_sizes.as<int32_t>(), members, base, z->d_moff.as<uint64_t>());
+    bai::bai_record_kernel<<<(unsigned)((n_rec + 255) / 256), 256, 0, z->stream>>>(
+        z->d_in.as<uint8_t>(), n_in, members, z->d_rec_off.as<int64_t>(), n_rec, z->d_moff.as<uint64_t>(), z->d_recs.as<bai::Rec>(), counts + 3);
+    bai::bai_chunk_kernel<<<1, BAI_THREADS, 0, z->stream>>>(z->d_recs.as<bai::Rec>(), n_rec, z->d_chunks.as<bai::Chunk>(),
+        z->d_sorted.as<bai::Chunk>(), z->d_segs.as<bai::Seg>(), z->d_out_chunks.as<uint64_t>(), z->d_out_refs.as<uint64_t>(), counts);
+    uint64_t *hc = static_cast<uint64_t *>(z->h_counts.p);
+    if ((rc = check(cudaGetLastError())) ||
+        (rc = check(cudaMemcpyAsync(hc, counts, 4 * sizeof(uint64_t), cudaMemcpyDeviceToHost, z->stream))) ||
+        (rc = check(cudaStreamSynchronize(z->stream))))
+        return rc;
+    out->error_bits = hc[3];
+    if (hc[3]) return NPORE_ERR_BAD_ARG;
+    const int64_t n_ch = (int64_t)hc[0], n_seg = (int64_t)hc[1], n_win = (int64_t)hc[2];
+    const size_t b_ch = (size_t)n_ch * 4 * sizeof(uint64_t), b_seg = (size_t)n_seg * 7 * sizeof(uint64_t), b_win = (size_t)n_win * sizeof(uint64_t);
+    if ((rc = check(z->d_win.ensure(std::max<size_t>(b_win, 8)))) || (rc = check(z->h_lists.ensure(b_ch + b_seg + b_win))))
+        return rc;
+    if (n_win) {
+        if ((rc = check(cudaMemsetAsync(z->d_win.p, 0xFF, b_win, z->stream)))) return rc;
+        bai::bai_linear_kernel<<<(unsigned)((n_rec + 255) / 256), 256, 0, z->stream>>>(z->d_recs.as<bai::Rec>(), n_rec, z->d_segs.as<bai::Seg>(),
+                                                                                       z->d_win.as<unsigned long long>());
+    }
+    uint8_t *h = static_cast<uint8_t *>(z->h_lists.p);
+    if ((rc = check(cudaGetLastError())) ||
+        (rc = check(cudaEventRecord(z->ev[1], z->stream))) ||
+        (rc = check(cudaMemcpyAsync(h, z->d_out_chunks.p, b_ch, cudaMemcpyDeviceToHost, z->stream))) ||
+        (rc = check(cudaMemcpyAsync(h + b_ch, z->d_out_refs.p, b_seg, cudaMemcpyDeviceToHost, z->stream))) ||
+        (n_win && (rc = check(cudaMemcpyAsync(h + b_ch + b_seg, z->d_win.p, b_win, cudaMemcpyDeviceToHost, z->stream)))) ||
+        (rc = check(cudaStreamSynchronize(z->stream))))
+        return rc;
+    if (device_ms && (rc = check(cudaEventElapsedTime(device_ms, z->ev[0], z->ev[1])))) return rc;
+    out->chunks = reinterpret_cast<const uint64_t *>(h);
+    out->n_chunks = n_ch;
+    out->refs = reinterpret_cast<const uint64_t *>(h + b_ch);
+    out->n_refs = n_seg;
+    out->windows = reinterpret_cast<const uint64_t *>(h + b_ch + b_seg);
+    out->n_windows = n_win;
     return NPORE_OK;
 }
 

@@ -85,9 +85,42 @@ inline uint16_t rd16(const uint8_t *p) { uint16_t v; std::memcpy(&v, p, 2); retu
 
 struct Rec {                // decoded once at open
     int64_t off;            // offset of the record's refID field in `data`
+    uint64_t voff;          // virtual offset of the record's block_size field (file offset of its member << 16 | offset inside)
     int32_t ref_id, pos, end, l_seq, n_cigar, n_cigar_kept, lead, trail, hp, name_len;
     uint16_t flag; uint8_t mapq, has_qual;
 };
+
+struct MSeg { size_t pos, len; uint64_t coff; size_t moff; };   // data[pos, pos + len): bytes moff.. of the member at file offset coff
+
+// virtual offset of data[i]; a position at the end of a member belongs to the next one ("next member, offset 0")
+uint64_t voff_at(const std::vector<MSeg> &segs, size_t i)
+{
+    size_t lo = 0, hi = segs.size();
+    while (lo < hi) { const size_t m = (lo + hi) / 2; if (segs[m].pos + segs[m].len <= i) lo = m + 1; else hi = m; }
+    return lo < segs.size() && segs[lo].pos <= i ? segs[lo].coff << 16 | (uint64_t)(segs[lo].moff + i - segs[lo].pos) : UINT64_MAX;
+}
+
+// data position of virtual offset v if its member is loaded, else SIZE_MAX
+size_t pos_of(const std::vector<MSeg> &segs, uint64_t v)
+{
+    for (const MSeg &g : segs)
+        if (g.coff == v >> 16 && (v & 0xffff) >= g.moff && (v & 0xffff) <= g.moff + g.len) return g.pos + (size_t)(v & 0xffff) - g.moff;
+    return SIZE_MAX;
+}
+
+// the segments of data[from, ...), shifted to start at 0
+std::vector<MSeg> segs_from(const std::vector<MSeg> &segs, size_t from)
+{
+    std::vector<MSeg> out;
+    for (const MSeg &g : segs)
+        if (g.pos + g.len > from) {
+            MSeg h = g;
+            if (h.pos < from) { h.moff += from - h.pos; h.len -= from - h.pos; h.pos = 0; }
+            else h.pos -= from;
+            out.push_back(h);
+        }
+    return out;
+}
 
 }  // namespace
 
@@ -96,7 +129,13 @@ struct npore_bam {
     bool eof = false;
     int n_threads = 0;
     int64_t file_size = 0, c_in = 0, c_out = 0;   // bytes in the file; compressed bytes consumed / inflated bytes produced so far
+    int64_t coff = 0, c_read = 0;         // file offset of the next member to read; member bytes read from the file
     Bytes data;                           // inflated BAM stream of the current window (starts with the bytes carried over)
+    std::vector<MSeg> segs, nsegs;        // the members in data / ndata
+    // npore_bam_restrict: only records whose start lies in one of these chunks of virtual offsets (sorted, disjoint)
+    bool restricted = false;
+    std::vector<uint64_t> rbeg, rend;
+    size_t rk = 0;                        // the chunk being read
     size_t head = 0;                      // first byte of `data` not yet consumed (header / complete records before it)
     std::string text;
     std::vector<std::string> ref_names;
@@ -145,14 +184,16 @@ const char *npore_io_last_error(void) { return g_err.c_str(); }
 
 // Append the next BGZF members of the file to b->data until at least `want` more inflated bytes are there (or EOF).
 // Member layout: 12 fixed bytes, XLEN extra (subfield 'B','C' holds BSIZE = member size - 1), deflate data, CRC32, ISIZE.
-static int load_blocks(npore_bam *b, Bytes &data, size_t want)
+// limit_coff >= 0 (a restriction): members starting after that file offset are read only while nothing has been added yet, i.e.
+// when the caller needs more bytes to complete a record.  Every member's file offset goes to segs.
+static int load_blocks(npore_bam *b, Bytes &data, std::vector<MSeg> &segs, size_t want, int64_t limit_coff = -1)
 {
     struct Blk { size_t coff, clen, uoff, ulen; uint32_t crc; };
     Bytes cbuf;
     std::vector<Blk> blks;
     size_t added = 0;
     const size_t base = data.size();
-    while (!b->eof && added < want) {
+    while (!b->eof && added < want && (limit_coff < 0 || b->coff <= limit_coff || blks.empty())) {
         uint8_t hd[12];
         const size_t got = std::fread(hd, 1, 12, b->fh);
         if (got == 0) { b->eof = true; break; }
@@ -175,6 +216,8 @@ static int load_blocks(npore_bam *b, Bytes &data, size_t want)
         Blk k;
         k.coff = at; k.clen = rest - 8; k.crc = rd32(&cbuf[at + rest - 8]); k.ulen = rd32(&cbuf[at + rest - 4]); k.uoff = base + added;
         if (k.ulen > 65536) return io_fail(NPORE_IO_ERR_FORMAT, "BGZF member claims more than 64 KiB of data (SAM spec 4.1: ISIZE <= 65536)");
+        if (k.ulen) segs.push_back({k.uoff, k.ulen, (uint64_t)b->coff, 0});
+        b->coff += (int64_t)bsize; b->c_read += (int64_t)bsize;
         added += k.ulen;
         blks.push_back(k);
     }
@@ -217,7 +260,7 @@ int npore_bam_open(const char *path, int n_threads, npore_bam **out)
     auto have = [&](size_t n) -> int {        // 1: n bytes available, 0: file ended first, <0: error
         while (bam->data.size() < n) {
             if (bam->eof) return 0;
-            const int rc = load_blocks(bam, bam->data, std::max<size_t>(n - bam->data.size(), 1));
+            const int rc = load_blocks(bam, bam->data, bam->segs, std::max<size_t>(n - bam->data.size(), 1));
             if (rc) return rc;
         }
         return 1;
@@ -247,31 +290,73 @@ int npore_bam_open(const char *path, int n_threads, npore_bam **out)
 
 // Next window of records: drops the previous window, inflates members until at least max_bytes of record data are
 // available (<= 0: the rest of the file) and indexes the complete records.  Returns their number; 0 at end of file.
-static int64_t fill_window(npore_bam *bam, Bytes &data, std::vector<Rec> &recs, size_t &head, int64_t max_bytes)
+static int64_t fill_window(npore_bam *bam, Bytes &data, std::vector<MSeg> &segs, std::vector<Rec> &recs, size_t &head, int64_t max_bytes)
 {
     size_t want = max_bytes > 0 ? (size_t)max_bytes : (size_t)-1;
     if (max_bytes > 0 && bam->file_size > 0) {
         // a short last window is a short last batch, and a short batch costs a full chunk latency on the GPU (12 ms for 74 reads
-        // of the C2 file): when what is left of the file would inflate to less than 1.4 windows, this window takes all of it
-        const int64_t at_c = (int64_t)std::ftell(bam->fh);
+        // of the C2 file): when what is left of the file would inflate to less than 1.4 windows, this window takes all of it.
+        // Under a restriction, what is left is the compressed bytes of the chunks not read yet.
+        double left = (double)(bam->file_size - bam->coff);
+        if (bam->restricted) {
+            left = 0;
+            for (size_t k = bam->rk; k < bam->rbeg.size(); k++)
+                left += (double)(bam->rend[k] >> 16) - (double)std::max<int64_t>((int64_t)(bam->rbeg[k] >> 16), bam->coff) + 65536.0;
+        }
         const double ratio = bam->c_in > (1 << 16) ? (double)bam->c_out / (double)bam->c_in : 3.0;
-        if (at_c >= 0 && (double)data.size() + (double)(bam->file_size - at_c) * ratio < 1.4 * (double)max_bytes) want = (size_t)-1;
+        if ((double)data.size() + std::max(left, 0.0) * ratio < 1.4 * (double)max_bytes) want = (size_t)-1;
     }
     std::vector<int64_t> offs;
-    size_t at = 0;
+    size_t at = 0, skip = 0;
     for (;;) {
         // index the complete records present
-        while (at + 4 <= data.size() && !(at >= want && !offs.empty())) {
+        bool chunks_done = false, seek = false;
+        for (;;) {
+            if (bam->restricted) {
+                // the next record starts at `at` (or in the next member of the file, at offset 0)
+                const uint64_t va = at < data.size() ? voff_at(segs, at) : (uint64_t)bam->coff << 16;
+                while (bam->rk < bam->rbeg.size() && va >= bam->rend[bam->rk]) bam->rk++;
+                if (bam->rk == bam->rbeg.size()) { chunks_done = true; break; }
+                if (va < bam->rbeg[bam->rk]) {                // before the chunk: skip to its start, in the data or by a seek
+                    const size_t p = pos_of(segs, bam->rbeg[bam->rk]);
+                    if (p != SIZE_MAX && p >= at) { at = p; continue; }
+                    seek = true;
+                    break;
+                }
+            }
+            if (!(at + 4 <= data.size() && !(at >= want && !offs.empty()))) break;
             const size_t bs = rd32(&data[at]);
             if (bs < 32) return io_fail(NPORE_IO_ERR_FORMAT, "corrupt BAM record (block_size < 32)");
             if (at + 4 + bs > data.size()) break;
             offs.push_back((int64_t)at + 4);
             at += 4 + bs;
         }
-        if ((at >= want && !offs.empty()) || (bam->eof && (at + 4 > data.size() || at + 4 + rd32(&data[at]) > data.size()))) break;
+        if (chunks_done) {                              // every chunk read: nothing after this record counts
+            data.resize(at);
+            while (!segs.empty() && segs.back().pos >= at) segs.pop_back();
+            bam->eof = true;
+            break;
+        }
+        if (seek) {
+            const uint64_t v = bam->rbeg[bam->rk];
+            data.resize(at);
+            while (!segs.empty() && segs.back().pos >= at) segs.pop_back();
+            if (!segs.empty() && segs.back().pos + segs.back().len > at) segs.back().len = at - segs.back().pos;
+            if (std::fseek(bam->fh, (long)(v >> 16), SEEK_SET) != 0) return io_fail(NPORE_IO_ERR_FORMAT, "seek to an indexed chunk failed");
+            bam->coff = (int64_t)(v >> 16); bam->eof = false;
+            skip = (size_t)(v & 0xffff);
+        }
+        if (!seek && ((at >= want && !offs.empty()) || (bam->eof && (at + 4 > data.size() || at + 4 + rd32(&data[at]) > data.size())))) break;
         const size_t need = std::max<size_t>(want > at ? std::min<size_t>(want - at, (size_t)1 << 30) : 1, 1);
-        const int rc = load_blocks(bam, data, need);
+        const size_t before = data.size();
+        const int64_t limit = bam->restricted && bam->rk < bam->rend.size() ? (int64_t)(bam->rend[bam->rk] >> 16) : -1;
+        const int rc = load_blocks(bam, data, segs, need, limit);
         if (rc) return rc;
+        if (skip) {                                     // the chunk starts inside the member just loaded
+            if (data.size() == before || before + skip > data.size()) return io_fail(NPORE_IO_ERR_FORMAT, "indexed chunk starts past its BGZF member");
+            at = before + skip;
+            skip = 0;
+        }
     }
     if (bam->eof && offs.empty() && at != data.size())
         return io_fail(NPORE_IO_ERR_FORMAT, "truncated BAM record at end of file");
@@ -285,6 +370,7 @@ static int64_t fill_window(npore_bam *bam, Bytes &data, std::vector<Rec> &recs, 
             const size_t bs = rd32(r - 4);
             Rec &o = recs[(size_t)k];
             o.off = offs[(size_t)k];
+            o.voff = voff_at(segs, (size_t)offs[(size_t)k] - 4);
             o.ref_id = (int32_t)rd32(r); o.pos = (int32_t)rd32(r + 4);
             o.name_len = r[8] ? r[8] - 1 : 0; o.mapq = r[9];
             o.n_cigar = rd16(r + 12); o.flag = rd16(r + 14); o.l_seq = (int32_t)rd32(r + 16);
@@ -322,12 +408,12 @@ int64_t npore_bam_advance(npore_bam *bam, int64_t max_bytes)
     if (bam->pf.joinable()) {             // the next window was prefetched: swap it in
         bam->pf.join();
         if (bam->pf_rc < 0) return io_fail((int)bam->pf_rc, bam->pf_err);
-        bam->data.swap(bam->ndata); std::swap(bam->recs, bam->nrecs); bam->head = bam->nhead;
+        bam->data.swap(bam->ndata); std::swap(bam->recs, bam->nrecs); std::swap(bam->segs, bam->nsegs); bam->head = bam->nhead;
         return bam->pf_rc;
     }
     bam->recs.clear();
-    if (bam->head) { bam->data.erase_front(bam->head); bam->head = 0; }
-    return fill_window(bam, bam->data, bam->recs, bam->head, max_bytes);
+    if (bam->head) { bam->segs = segs_from(bam->segs, bam->head); bam->data.erase_front(bam->head); bam->head = 0; }
+    return fill_window(bam, bam->data, bam->segs, bam->recs, bam->head, max_bytes);
 }
 
 // Start inflating + indexing the window AFTER the current one on a background thread; the current window stays valid for
@@ -337,16 +423,37 @@ int npore_bam_prefetch(npore_bam *bam, int64_t max_bytes)
     if (!bam) return io_fail(NPORE_IO_ERR_ARG, "null handle");
     if (bam->pf.joinable()) return NPORE_IO_OK;
     bam->ndata.assign(bam->data.data() + bam->head, bam->data.data() + bam->data.size());      // the bytes carried over (a partial record)
+    bam->nsegs = segs_from(bam->segs, bam->head);
     bam->nrecs.clear(); bam->nhead = 0; bam->pf_rc = 0;
     bam->pf = std::thread([bam, max_bytes]() {
         enter_background();
-        bam->pf_rc = fill_window(bam, bam->ndata, bam->nrecs, bam->nhead, max_bytes);
+        bam->pf_rc = fill_window(bam, bam->ndata, bam->nsegs, bam->nrecs, bam->nhead, max_bytes);
         if (bam->pf_rc < 0) bam->pf_err = g_err;
     });
     return NPORE_IO_OK;
 }
 
 void npore_bam_close(npore_bam *b) { delete b; }
+
+int npore_bam_restrict(npore_bam *b, int64_t n, const uint64_t *vbeg, const uint64_t *vend)
+{
+    if (!b || n < 0 || (n && (!vbeg || !vend))) return io_fail(NPORE_IO_ERR_ARG, "null argument");
+    if (b->pf.joinable() || !b->recs.empty() || b->restricted) return io_fail(NPORE_IO_ERR_ARG, "restrict before the first window, once");
+    for (int64_t k = 0; k < n; k++)
+        if (vbeg[k] >= vend[k] || (k && vbeg[k] < vend[k - 1])) return io_fail(NPORE_IO_ERR_ARG, "chunks must be sorted, disjoint and non-empty");
+    b->rbeg.assign(vbeg, vbeg + n); b->rend.assign(vend, vend + n);
+    b->rk = 0; b->restricted = true;
+    return NPORE_IO_OK;
+}
+
+int npore_bam_voffsets(const npore_bam *b, uint64_t *out)
+{
+    if (!b || !out) return io_fail(NPORE_IO_ERR_ARG, "null argument");
+    for (size_t k = 0; k < b->recs.size(); k++) out[k] = b->recs[k].voff;
+    return NPORE_IO_OK;
+}
+
+int64_t npore_bam_bytes_read(const npore_bam *b) { return b ? b->c_read : NPORE_IO_ERR_ARG; }
 
 int64_t npore_bam_header_text(const npore_bam *b, const char **text)
 {
@@ -600,15 +707,13 @@ int64_t npore_bam_bound(int64_t n, const int64_t *name_off, const int64_t *seq_o
     return (name_off[n] - name_off[0]) + 2 * (seq_off[n] - seq_off[0]) + 4 * (rle_off[n] - rle_off[0]) + n * 48;
 }
 
-int64_t npore_bam_format(int64_t n, int n_threads,
-                         const uint8_t *names, const int64_t *name_off, const int32_t *flag, const int32_t *ref_id,
-                         const uint8_t *ref_names, const int64_t *ref_name_off, int32_t n_refs,
+static int64_t bam_format_impl(int64_t n, int n_threads,
+                         const uint8_t *names, const int64_t *name_off, const int32_t *flag, const int32_t *ref_id, int32_t n_refs,
                          const int32_t *pos, const int32_t *end, const int32_t *mapq,
                          const uint32_t *rle, const int64_t *rle_off,
                          const uint8_t *seq_ascii, const uint8_t *qual_ascii, const int64_t *seq_off, const int32_t *has_qual,
-                         const int32_t *hp, uint8_t *out, int64_t out_capacity)
+                         const int32_t *hp, uint8_t *out, int64_t out_capacity, int64_t *rec_off)
 {
-    (void)ref_names; (void)ref_name_off;
     if (n < 0) return io_fail(NPORE_IO_ERR_ARG, "negative count");
     if (!n) return 0;
     if (!names || !name_off || !flag || !ref_id || !pos || !end || !mapq || !rle_off || !seq_off || !has_qual || !hp || !out)
@@ -670,7 +775,35 @@ int64_t npore_bam_format(int64_t n, int n_threads,
             std::memcpy(o + 3, &v, (size_t)nb);          // little-endian: the low bytes of the value
         }
     });
+    if (rec_off) std::memcpy(rec_off, at.data(), ((size_t)n + 1) * sizeof(int64_t));
     return at[(size_t)n];
+}
+
+int64_t npore_bam_format(int64_t n, int n_threads,
+                         const uint8_t *names, const int64_t *name_off, const int32_t *flag, const int32_t *ref_id,
+                         const uint8_t *ref_names, const int64_t *ref_name_off, int32_t n_refs,
+                         const int32_t *pos, const int32_t *end, const int32_t *mapq,
+                         const uint32_t *rle, const int64_t *rle_off,
+                         const uint8_t *seq_ascii, const uint8_t *qual_ascii, const int64_t *seq_off, const int32_t *has_qual,
+                         const int32_t *hp, uint8_t *out, int64_t out_capacity)
+{
+    (void)ref_names; (void)ref_name_off;
+    return bam_format_impl(n, n_threads, names, name_off, flag, ref_id, n_refs, pos, end, mapq, rle, rle_off, seq_ascii, qual_ascii,
+                           seq_off, has_qual, hp, out, out_capacity, nullptr);
+}
+
+int64_t npore_bam_format_offsets(int64_t n, int n_threads,
+                                 const uint8_t *names, const int64_t *name_off, const int32_t *flag, const int32_t *ref_id,
+                                 const uint8_t *ref_names, const int64_t *ref_name_off, int32_t n_refs,
+                                 const int32_t *pos, const int32_t *end, const int32_t *mapq,
+                                 const uint32_t *rle, const int64_t *rle_off,
+                                 const uint8_t *seq_ascii, const uint8_t *qual_ascii, const int64_t *seq_off, const int32_t *has_qual,
+                                 const int32_t *hp, uint8_t *out, int64_t out_capacity, int64_t *rec_off)
+{
+    (void)ref_names; (void)ref_name_off;
+    if (n > 0 && !rec_off) return io_fail(NPORE_IO_ERR_ARG, "null argument");
+    return bam_format_impl(n, n_threads, names, name_off, flag, ref_id, n_refs, pos, end, mapq, rle, rle_off, seq_ascii, qual_ascii,
+                           seq_off, has_qual, hp, out, out_capacity, rec_off);
 }
 
 }  // extern "C"

@@ -442,7 +442,7 @@ class BgzfCompressor:
             raise NporeError(f"npore_bgzf_create failed: {self._L.npore_strerror(rc).decode()} "
                              "(npore_b200 needs a CUDA device; there is no CPU fallback)")
         self._in = self._out = None
-        self.last_device_ms = 0.0
+        self.last_device_ms = self.last_index_ms = 0.0
 
     def compress(self, buf):
         src = np.frombuffer(buf, dtype=np.uint8) if not isinstance(buf, np.ndarray) else buf.reshape(-1).view(np.uint8)
@@ -460,6 +460,29 @@ class BgzfCompressor:
             raise NporeError(f"npore_bgzf_compress: {self._L.npore_strerror(rc).decode()}")
         self.last_device_ms = float(ms.value)
         return pin_out[:got.value]
+
+    def index(self, rec_off, base):
+        """BAM index lists of the records of the last compress() call (npore_bgzf_index): rec_off[n+1] are the records' offsets
+        in its input, base the file offset its first member is written at.  Returns {"chunks": (n, 4), "refs": (m, 7),
+        "windows": (w,)} uint64 arrays (copies); ValueError when the records cannot be indexed.  last_index_ms: kernel time."""
+        rec_off = np.ascontiguousarray(rec_off, dtype=np.int64)
+        lists, ms = _lib.BaiLists(), C.c_float()
+        rc = self._L.npore_bgzf_index(self._z, rec_off.ctypes.data, len(rec_off) - 1, int(base), C.byref(lists), C.byref(ms))
+        if rc != 0:
+            if lists.error_bits:
+                why = [w for b, w in ((1, "records out of coordinate order"), (2, "inconsistent record bytes"),
+                                      (4, "records without a reference or position")) if lists.error_bits & b]
+                raise ValueError(f"cannot index the BAM output: {', '.join(why)}")
+            raise NporeError(f"npore_bgzf_index: {self._L.npore_strerror(rc).decode()}")
+        self.last_index_ms = float(ms.value)
+
+        def rows(ptr, n, width):
+            if not n:
+                return np.zeros((0, width) if width > 1 else 0, np.uint64)
+            a = np.ctypeslib.as_array(C.cast(ptr, C.POINTER(C.c_uint64)), shape=(n * width,)).copy()
+            return a.reshape(n, width) if width > 1 else a
+        return {"chunks": rows(lists.chunks, lists.n_chunks, 4), "refs": rows(lists.refs, lists.n_refs, 7),
+                "windows": rows(lists.windows, lists.n_windows, 1)}
 
     def close(self):
         if getattr(self, "_z", None) and self._z.value:
